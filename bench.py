@@ -8,6 +8,7 @@ With N GPUs every rank fits its own volume of that size (weak scaling, no data-p
 north-star case — ONE volume over N GPUs, host memory in -> host memory out — is measured beside it (`one_volume`).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]                 our CUDA path
+  python bench.py ... --dump-outputs DIR                              + the outputs of the last timed step, DIR/*.npy
   python bench.py --impl reference [--gpus N] --steps K --warmup W    the reference's CPU algorithm (oracle port, all
                                                                       host cores, bounded sample per step)
 Prints ONE JSON line on rank 0.
@@ -25,6 +26,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the checkout may be read-only: no __pycache__ next to the sources
 
 METRIC = "fitted voxels/s (FA+reg NNLS)"
 UNIT = "voxels/s"
@@ -40,6 +42,9 @@ FP64_PEAK_TFLOPS = 34.16    # own DFMA micro-benchmark on this pool's B200 (prof
 HBM_BYTES_PER_VOXEL_T2 = 32 * 8 + 4 + 60 * 8 + 32 * 8 + 8 + 6 * 8 + 4   # T2 kernel: read signal+index, write outputs
 HBM_BYTES_PER_VOXEL_FA = 16 * 32 * 8 + 15 * 8 + 3 * 8 + 8                # FA kernels: signal per search angle + outputs
 NCU_RECORD = "profiles/r02_kernel_counters.json"   # executed flops / DRAM traffic per voxel of the current kernels (ncu)
+# --dump-outputs: per-voxel outputs at a fixed sample of this many voxels (104 float64 outputs + the voxel's index at
+# the config-2 widths = 55 MB), so that the dump stays under 64 MB
+DUMP_VOXELS = 65536
 
 
 def f_alg():
@@ -60,7 +65,14 @@ def parse_args():
     ap.add_argument("--t2-flags", type=int, default=0, help="extra MET2_T2_FLAG_* bits for every T2 fit (A/B runs only)")
     ap.add_argument("--gram", action="store_true",
                     help="A/B runs only: Gram-domain T2 kernel instead of the default reduced-echo-space kernel")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0) as DIR/<name>.npy, float64: "
+                         "FA and T2 outputs at a fixed, seeded sample of %d voxels (voxel_index.npy), fsol_sum whole"
+                         % DUMP_VOXELS)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------- clocks
@@ -254,7 +266,7 @@ def run_ours(args):
         dist.init_process_group("nccl", device_id=dev)
         host_group = dist.new_group(backend="gloo")     # host-side waits that leave the GPUs idle
     shape = SHAPE if args.shape is None else tuple(int(x) for x in args.shape.split(","))
-    lib = _lib.load()
+    lib = _lib.load(build_if_missing=False)      # the library build() left in the tree; never rebuilt here
 
     ph = make_phantom(shape, n_echoes=N_ECHOES, tau=TAU, TR=TR, seed=2 + rank, fa_mode="b1", backend="gpu")
     sig_host = torch.as_tensor(ph["data"].reshape(-1, N_ECHOES)).pin_memory()
@@ -297,6 +309,8 @@ def run_ours(args):
     fa_ms = float(np.mean([e[0].elapsed_time(e[1]) for e in ev]))
     t2_ms = float(np.mean([e[1].elapsed_time(e[2]) for e in ev]))
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, fa_out, t2_out)
 
     # ---- end to end through the public API with host buffers (H2D + fit + D2H inside the timed region)
     pinned = pipeline.host_buffers(plan, V)
@@ -394,6 +408,24 @@ def run_ours(args):
         dist.barrier()
         dist.destroy_process_group()
     return 0
+
+
+def dump_outputs(out_dir, fa_out, t2_out):
+    """The arrays plan.fa_fit / plan.t2_fit returned in the last timed step, as <out_dir>/<name>.npy in float64 (the
+    int32 outputs fa_index, fa_status and status convert exactly).  Per-voxel arrays are cut to the rows listed in
+    voxel_index.npy: all voxels up to DUMP_VOXELS, else a sorted sample of DUMP_VOXELS drawn with seed 0."""
+    import torch
+    V = fa_out["fa_index"].shape[0]
+    pick = np.arange(V) if V <= DUMP_VOXELS else np.sort(np.random.default_rng(0).choice(V, DUMP_VOXELS, replace=False))
+    rows = torch.as_tensor(pick, device=fa_out["fa_index"].device)
+    arrays = {"voxel_index": pick, "fsol_sum": fa_out["fsol_sum"].cpu().numpy()}
+    for name, t in (("fa_index", fa_out["fa_index"]), ("fa_deg", fa_out["fa_deg"]), ("km", fa_out["km"]),
+                    ("fa_status", fa_out["status"]), ("fsol", t2_out["fsol"]), ("est_signal", t2_out["est_signal"]),
+                    ("reg", t2_out["reg"]), ("maps", t2_out["maps"]), ("status", t2_out["status"])):
+        arrays[name] = t.index_select(0, rows).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def one_volume(args, torch, dist, pipeline, plan, dev, rank, world, host_group, shape, barrier):

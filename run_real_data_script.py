@@ -18,7 +18,7 @@ from multicomponent_t2_toolbox_b200.motor.motor_recon_met2_real_data import moto
 
 # (flag, type, default, choices, required, help) — the reference's flags, types, defaults, choices and `required`
 # settings (run_real_data_script.py:18-62): every flag is required there except --numcores (default -1 = all).
-# tests/test_nifti_cli.py parses the reference's own argparse block and diffs this table against it.
+# tests/test_nifti_cli.py diffs this table against the reference's argparse block (tests/golden/reference_cli_flags.json).
 _FLAGS = [
     ("--path_to_folder", str, None, None, True, "folder that holds the data, mask and the output directory (trailing '/')"),
     ("--input", str, None, None, True, "4-D multi-echo NIfTI file inside the folder"),

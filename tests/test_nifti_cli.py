@@ -93,31 +93,15 @@ def test_nifti_big_endian_qform_and_shapes(tmp_path):
         assert np.array_equal(nifti_io.load(q).get_fdata(), x)
 
 
-def _reference_flags(path):
-    """(flag -> dict(type, default, choices, required)) parsed from the reference script's own argparse block."""
-    import ast
-    tree = ast.parse(open(path).read())
-    out = {}
-    for node in ast.walk(tree):
-        if isinstance(node, ast.Call) and getattr(node.func, "attr", "") == "add_argument":
-            flag = ast.literal_eval(node.args[0])
-            kw = {k.arg: k.value for k in node.keywords}
-            out[flag] = dict(type=kw["type"].id if "type" in kw else None,
-                             default=ast.literal_eval(kw["default"]) if "default" in kw else None,
-                             choices=ast.literal_eval(kw["choices"]) if "choices" in kw else None,
-                             required=ast.literal_eval(kw["required"]) if "required" in kw else False)
-    return out
-
-
 @pytest.mark.parametrize("script,mod", [("run_real_data_script.py", "cli"),
                                         ("run_real_data_script_ROI_based_estimation.py", "cli_roi")])
 def test_cli_flag_table_equals_reference_argparse(script, mod):
     """Flag / type / default / choices / required of every option, diffed against the reference's own argparse block
-    (run_real_data_script.py:18-62, run_real_data_script_ROI_based_estimation.py:18-52)."""
-    path = os.path.join("/root/reference", script)
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present on this box")
-    ref = _reference_flags(path)
+    (run_real_data_script.py:18-62, run_real_data_script_ROI_based_estimation.py:18-52) as recorded in
+    tests/golden/reference_cli_flags.json."""
+    import json
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_cli_flags.json")) as fh:
+        ref = json.load(fh)[script]
     ours = {f: dict(type=t.__name__, default=d, choices=c, required=r)
             for f, t, d, c, r, _ in globals()[mod]._FLAGS}
     assert ours == ref
