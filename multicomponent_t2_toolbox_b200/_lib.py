@@ -69,10 +69,6 @@ def load(build_if_missing=True):
     if _LIB is not None:
         return _LIB
     path = _build.LIB_PATH
-    variant = os.environ.get("MET2_LIB_VARIANT")   # A/B runs of a compile-time switch: libmet2_<variant>.so, prebuilt by
-    if variant:                                    # build.build_library(extra_flags=..., out_path=...); never built here
-        path = os.path.join(_build.PKG_DIR, "libmet2_%s.so" % variant)
-        build_if_missing = False
     if build_if_missing and _build.needs_build():
         try:
             _build.build_library()

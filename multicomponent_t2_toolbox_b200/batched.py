@@ -10,7 +10,6 @@ PyTorch is used only for device buffers and streams.  There is no CPU path: cons
 """
 import ctypes
 import math
-import os
 
 import numpy as np
 import torch
@@ -202,13 +201,11 @@ class Dictionary:
 
     def echo_basis(self, ranks=None):
         """Reduced echo basis the echo-space kernels run on: (basis, coef, R) for the smallest rank R among `ranks`
-        (default: both ranks the library is built for, 16 and 24; MET2_ECHO_RANKS=24 restricts them for A/B runs) whose
-        measured residual is within ECHO_TAIL_MAX[R], or None when none is (then the Gram-domain kernels run)."""
+        (default: both ranks the library is built for, 16 and 24) whose measured residual is within ECHO_TAIL_MAX[R], or
+        None when none is (then the Gram-domain kernels run)."""
         if ranks is None:
             lib = _lib.load()
             ranks = (int(lib.met2_echo_rank(1)), int(lib.met2_echo_rank(0)))
-            if os.environ.get("MET2_ECHO_RANKS"):
-                ranks = [r for r in ranks if str(r) in os.environ["MET2_ECHO_RANKS"].split(",")]
         for R in sorted(ranks):
             basis, coef, tail = self.echo_tables(R)
             if tail <= ECHO_TAIL_MAX[R]:

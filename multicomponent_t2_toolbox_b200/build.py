@@ -38,29 +38,26 @@ def needs_build():
     return any(os.path.getmtime(d) > t for d in _deps())
 
 
-def build_library(force=False, verbose=False, extra_flags=(), out_path=None):
+def build_library(force=False, verbose=False):
     """Compile every .cu under csrc/ for sm_100a into libmet2.so.  Returns the library path.
 
     Safe against concurrent callers (torchrun ranks): the build runs under an exclusive file lock, objects go to a
     private temporary directory and the finished library is moved into place atomically, so a process that is loading
-    libmet2.so never sees a half-written file.  `extra_flags` / `out_path` build a VARIANT (A/B runs of a compile-time
-    switch, e.g. ["-DMET2_FOO=1"] -> libmet2_foo.so) without touching the product library."""
+    libmet2.so never sees a half-written file."""
     import fcntl
     import tempfile
-    out_path = LIB_PATH if out_path is None else out_path
-    variant = out_path != LIB_PATH
-    if not force and not variant and not needs_build():
+    if not force and not needs_build():
         return LIB_PATH
     nvcc = _nvcc()
     from concurrent.futures import ThreadPoolExecutor
     with open(os.path.join(PKG_DIR, ".build.lock"), "w") as lock:
         fcntl.flock(lock, fcntl.LOCK_EX)
-        if not force and not variant and not needs_build():      # another process built it while we waited
+        if not force and not needs_build():      # another process built it while we waited
             return LIB_PATH
         with tempfile.TemporaryDirectory(prefix="met2_build_") as tmp:
             def compile_one(src):
                 obj = os.path.join(tmp, src.replace(".cu", ".o"))
-                cmd = [nvcc] + NVCC_FLAGS + list(extra_flags) + ["-c", os.path.join(CSRC, src), "-o", obj]
+                cmd = [nvcc] + NVCC_FLAGS + ["-c", os.path.join(CSRC, src), "-o", obj]
                 r = subprocess.run(cmd, capture_output=True, text=True)
                 if r.returncode != 0:
                     raise RuntimeError("nvcc failed on %s:\n%s" % (src, r.stderr[-8000:]))
@@ -70,20 +67,19 @@ def build_library(force=False, verbose=False, extra_flags=(), out_path=None):
                 results = list(ex.map(compile_one, SOURCES))
             objs = [o for o, _ in results]
             logs = [l for _, l in results]
-            if not variant:
-                # registers / spills / stack per kernel (compile times dropped: they change every build); written BEFORE
-                # the library so that it is never newer than libmet2.so
-                with open(os.path.join(CSRC, "ptxas.log"), "w") as fh:
-                    fh.write("\n".join(l for log in logs for l in log.split("\n") if "Compile time" not in l))
-            tmp_lib = out_path + ".tmp.%d" % os.getpid()
+            # registers / spills / stack per kernel (compile times dropped: they change every build); written BEFORE the
+            # library so that it is never newer than libmet2.so
+            with open(os.path.join(CSRC, "ptxas.log"), "w") as fh:
+                fh.write("\n".join(l for log in logs for l in log.split("\n") if "Compile time" not in l))
+            tmp_lib = LIB_PATH + ".tmp.%d" % os.getpid()
             cmd = [nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", tmp_lib] + objs
             r = subprocess.run(cmd, capture_output=True, text=True)
             if r.returncode != 0:
                 raise RuntimeError("nvcc link failed:\n%s" % r.stderr[-4000:])
-            os.replace(tmp_lib, out_path)
+            os.replace(tmp_lib, LIB_PATH)
         if verbose:
             print("\n".join(logs))
-    return out_path
+    return LIB_PATH
 
 
 EXAMPLE_SRC = os.path.join(PKG_DIR, "..", "examples", "c_host", "met2_host_demo.cpp")

@@ -1,7 +1,8 @@
-// met2_api.cu — error state, launch accounting and diagnostics of the C ABI (include/met2.h).
+// met2_api.cu — error state, launch accounting, test hooks and diagnostics of the C ABI (include/met2.h).
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
+#include <cstdlib>
 
 #include "met2_host.h"
 
@@ -41,6 +42,23 @@ int sm_count() {
     if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
     if (dev >= 0 && dev < 64) table[dev].store(n, std::memory_order_relaxed);
     return n;
+}
+
+Overrides read_overrides() {
+    Overrides o;
+    const char* ev = getenv("MET2_T2_WARPS");
+    o.t2_warps = ev ? atoi(ev) : 0;
+    ev = getenv("MET2_T2_TILE");
+    o.t2_tile = ev ? atoi(ev) : 0;
+    ev = getenv("MET2_LCURVE_SWITCH");
+    o.lcurve_switch_set = ev != nullptr;
+    o.lcurve_switch = ev ? atof(ev) : 0.0;
+    ev = getenv("MET2_FA_SEARCH");
+    o.fa_search_warp = ev && ev[0] == 'w';
+    ev = getenv("MET2_FA_THREAD_PCAP");
+    o.fa_thread_pcap_set = ev != nullptr;
+    o.fa_thread_pcap = ev ? atoi(ev) : 0;
+    return o;
 }
 
 }  // namespace met2

@@ -168,12 +168,6 @@ __global__ void __launch_bounds__(FA_SEARCH_WARPS * 32, 1) fa_search_kernel(FaAr
 //     warm start from the support and coefficients of the previous angle.
 // A voxel whose positive set would exceed PM columns, that runs into itmax or meets a non-positive pivot is handed to
 // the warp-per-voxel kernel (ovf_list), which redoes all its angles.
-#ifdef MET2_HOST_EMU
-static long long ft_dbg[8];   // emulator-only work statistics: ticks, w passes, solves, trials, rejected, rescues, inner, finished
-#define FT_DBG(i) (++ft_dbg[i])
-#else
-#define FT_DBG(i) ((void)0)
-#endif
 constexpr int FT_MAX_THREADS = 256;
 constexpr int FT_PM = 8;
 
@@ -350,7 +344,6 @@ __global__ void __launch_bounds__(FT_MAX_THREADS, 1) fa_search_thread_kernel(FaA
                         q1 = fma(r[e + 1], r[e + 1], q1);
                     }
                     rho2c = q0 + q1;
-                    FT_DBG(5);
                 }
                 if (!(rho2c > 0.0) || !(rho2c > 1.2e-28 * s1c)) {
                     rejected = true;
@@ -477,7 +470,6 @@ __global__ void __launch_bounds__(FT_MAX_THREADS, 1) fa_search_thread_kernel(FaA
             while (__any_sync(FULL_MASK, active && !fin && state != NEED_W)) {
                 if (active && !fin && state != NEED_W) {
                     const bool trial = (state == TRIAL);
-                    FT_DBG(2);
                     if (!trial) residual();   // TRIAL: x has not moved since the w pass
                     const int rc = solve(trial ? p + 1 : p, trial);
                     if (rc > 0) {
@@ -500,14 +492,12 @@ __global__ void __launch_bounds__(FT_MAX_THREADS, 1) fa_search_thread_kernel(FaA
             }
             // ---- w phase: dual of every column, entering candidate (first maximum over the zero set minus rejected ones)
             if (active && !fin) {
-                FT_DBG(0);
                 residual();
                 if (p >= n || p >= m) {
                     fin = true;
                 } else {
                     double bv = 0.0;
                     int bj = -1;
-                    FT_DBG(1);
                     for (int j0 = 0; j0 < n4; j0 += 4) {
                         double w0 = 0.0, w1 = 0.0, w2 = 0.0, w3 = 0.0, u0 = 0.0, u1 = 0.0, u2 = 0.0, u3 = 0.0;
                         const int row = oD + j0 * LDD;
@@ -543,7 +533,6 @@ __global__ void __launch_bounds__(FT_MAX_THREADS, 1) fa_search_thread_kernel(FaA
             __syncwarp();
             // ---- results of the voxels that are done with this angle
             if (active && fin) {
-                FT_DBG(7);
                 if (ovf) {
                     A.ws_p[v] = -1;
                     const int k = atomicAdd(A.ovf_count, 1);
@@ -789,15 +778,14 @@ struct FaGeom {
 
 // Geometry of the thread-per-voxel search for V voxels: the largest CTA (multiple of 32 threads) whose per-thread columns
 // fit beside the tables, not larger than what gives every SM a batch.  MET2_FA_SEARCH=warp switches the kernel off.
-static void fa_thread_geometry(FaGeom& g, const met2_fa_cfg* cfg, long long V, int sms) {
+static void fa_thread_geometry(FaGeom& g, const met2_fa_cfg* cfg, long long V, int sms, const Overrides& ov) {
     g.mr_thread = 0;
     g.threads_thread = g.grid_thread = 0;
     g.smem_thread = 0;
-    if (const char* ev = getenv("MET2_FA_SEARCH"))
-        if (ev[0] == 'w') return;
+    if (ov.fa_search_warp) return;
     // a few voxels per SM are latency bound either way and the warp kernel stages its tables with more threads
     // (config 1, 1 024 voxels: 2.4 ms with the warp kernel, 19 ms with 32-thread CTAs of this one)
-    if (V < (long long)sms * 64 && !getenv("MET2_FA_THREAD_PCAP")) return;
+    if (V < (long long)sms * 64 && !ov.fa_thread_pcap_set) return;
     const int m = cfg->nTE, n = cfg->nT2;
     const int mr = (m <= 32) ? 32 : ((m <= 48) ? 48 : 64);
     const size_t tables = sizeof(double) * (size_t)(mr == 32 ? ft_table_doubles<32>(n) : (mr == 48 ? ft_table_doubles<48>(n) : ft_table_doubles<64>(n)));
@@ -819,7 +807,7 @@ static void fa_thread_geometry(FaGeom& g, const met2_fa_cfg* cfg, long long V, i
 }
 
 template <int NS>
-static FaGeom fa_geometry(const met2_fa_cfg* cfg, long long V) {
+static FaGeom fa_geometry(const met2_fa_cfg* cfg, long long V, const Overrides& ov) {
     FaGeom g;
     g.pmax = cfg->nT2 < cfg->nTE ? cfg->nT2 : cfg->nTE;
     g.smem = sizeof(double) * (size_t)fa_warp_doubles<NS>(g.pmax) * FA_WARPS;
@@ -840,15 +828,15 @@ static FaGeom fa_geometry(const met2_fa_cfg* cfg, long long V) {
         g.warps_search = w;
         g.smem_search = tables + per_warp * w;
     }
-    fa_thread_geometry(g, cfg, V, sms);
+    fa_thread_geometry(g, cfg, V, sms, ov);
     return g;
 }
 
-static FaGeom fa_geometry_any(const met2_fa_cfg* cfg, long long V) {
+static FaGeom fa_geometry_any(const met2_fa_cfg* cfg, long long V, const Overrides& ov) {
     int ns = (cfg->nT2 + 31) / 32;
-    if (ns <= 2) return fa_geometry<2>(cfg, V);
-    if (ns == 3) return fa_geometry<3>(cfg, V);
-    return fa_geometry<4>(cfg, V);
+    if (ns <= 2) return fa_geometry<2>(cfg, V, ov);
+    if (ns == 3) return fa_geometry<3>(cfg, V, ov);
+    return fa_geometry<4>(cfg, V, ov);
 }
 
 template <int MR>
@@ -884,18 +872,6 @@ static int fa_launch(const FaArgs& A, const FaGeom& g, cudaStream_t st) {
     count_launch();
     rc = check_launch("fa_search_kernel");
     if (rc) return rc;
-    if (g.mr_thread && getenv("MET2_FA_DEBUG")) {   // diagnostic (synchronises): how many voxels took the warp-per-voxel path
-        int cnt = -1;
-        cudaStreamSynchronize(st);
-        cudaMemcpy(&cnt, A.ovf_count, sizeof(int), cudaMemcpyDeviceToHost);
-        fprintf(stderr, "met2_fa_fit: thread-per-voxel search (%d threads x %d CTAs, %zu B), %d of %lld voxels handed to the warp kernel\n",
-                g.threads_thread, g.grid_thread, g.smem_thread, cnt, A.V);
-#ifdef MET2_HOST_EMU
-        fprintf(stderr, "  emulator statistics: ticks %lld, w passes %lld, solves %lld (trials %lld, rejected %lld, D-space %lld, interpolation %lld), voxel-angles %lld\n",
-                ft_dbg[0], ft_dbg[1], ft_dbg[2], ft_dbg[3], ft_dbg[4], ft_dbg[5], ft_dbg[6], ft_dbg[7]);
-        for (int i = 0; i < 8; ++i) ft_dbg[i] = 0;
-#endif
-    }
     if (A.cfg.method == MET2_FA_SPLINE) {
         MET2_LAUNCH(1, 32, 0, st, spline_weights_kernel)(A.knots, A.cfg.nKnots, A.wsp);
         count_launch();
@@ -932,7 +908,7 @@ static int fa_check_cfg(const met2_fa_cfg* cfg) {
 
 extern "C" int64_t met2_fa_workspace_bytes(int64_t V, const met2_fa_cfg* cfg) {
     if (fa_check_cfg(cfg) || V < 0) return -1;
-    FaGeom g = fa_geometry_any(cfg, V);
+    FaGeom g = fa_geometry_any(cfg, V, read_overrides());
     int nS = cfg->method == MET2_FA_SPLINE ? cfg->nKnots : 1;
     size_t b = align256(sizeof(double) * (size_t)V * nS);
     b += align256(sizeof(double) * MET2_MAX_KNOTS * MET2_MAX_KNOTS);
@@ -956,7 +932,8 @@ extern "C" int met2_fa_fit(const double* sig, int64_t V, const met2_fa_cfg* cfg,
         return set_error(MET2_ERR_ARG, "met2_fa_fit: spline method needs the coarse dictionary and knots");
     if (V == 0) return MET2_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    FaGeom g = fa_geometry_any(cfg, V);
+    const Overrides ov = read_overrides();
+    FaGeom g = fa_geometry_any(cfg, V, ov);
     FaArgs A;
     A.sig = sig;
     A.V = V;
@@ -989,10 +966,7 @@ extern "C" int met2_fa_fit(const double* sig, int64_t V, const met2_fa_cfg* cfg,
     A.ovf_count = reinterpret_cast<int*>(w);
     A.vlist = nullptr;
     A.thread_pcap = FT_PM;
-    if (const char* ev = getenv("MET2_FA_THREAD_PCAP")) {   // test hook: smaller sets -> more voxels through the hand-back path
-        const int c = atoi(ev);
-        if (c >= 1 && c < FT_PM) A.thread_pcap = c;
-    }
+    if (ov.fa_thread_pcap >= 1 && ov.fa_thread_pcap < FT_PM) A.thread_pcap = ov.fa_thread_pcap;
     A.pmax = g.pmax;
     cudaError_t e = cudaMemsetAsync(status, 0, sizeof(uint32_t) * (size_t)V, st);
     if (e != cudaSuccess) return set_error(MET2_ERR_CUDA, "memset status: %s", cudaGetErrorString(e));

@@ -748,13 +748,8 @@ __device__ __forceinline__ void remove_position(const Slots<NS>& W, int k, int& 
 // (rho^2 = G_jj - r.r = -1.2e-13 for a column SciPy's QR-based test accepts).  Leaves a in S[W.gs..].
 // Everything is passed and returned BY VALUE: a reference argument would force the caller's Slots / rho^2 / y_new into
 // local memory on the hot path (measured with the first, by-reference version: T2 stage +3.3 %, FA stage +3 %).
-#ifndef MET2_DSPACE_INLINE          // A/B switch (libmet2_inl.so): out of line (default) or inlined into the solver
-#define MET2_DSPACE_FN __noinline__
-#else
-#define MET2_DSPACE_FN __forceinline__
-#endif
 template <int PS>
-__device__ MET2_DSPACE_FN double2 dspace_candidate(int oT, int oGs, int oRs, int oIx, const double* __restrict__ DtR,
+__device__ __noinline__ double2 dspace_candidate(int oT, int oGs, int oRs, int oIx, const double* __restrict__ DtR,
                                                  int oMR, int mrows, int j, int p, int lane) {
     double a[PS];
     tmul<PS>(oT, oRs, p, lane, a);
@@ -846,7 +841,6 @@ __device__ __forceinline__ int nnls_gram(const Slots<NS>& W, int oG, const doubl
         const double cj = S[W.cc + j];
         double rinv = rsqrt_fast(rho2);
         double ynew = (cj - s2) * rinv;
-#ifndef MET2_NO_DSPACE_RESCUE   // A/B timing switch only (libmet2_norescue.so); the product library always has the rescue
         if (!reg && p > 0 && rho2 < 1e-10 * gjj) {
             // rho^2 = G_jj - r.r is below the rounding of its terms (nearly collinear long-T2 columns of the 96/100-bin
             // grids): the Gram form resolves rho^2/G_jj to ~1e-16, nnls.f accepts down to ~5e-27.  Rare, so out of line.
@@ -859,7 +853,6 @@ __device__ __forceinline__ int nnls_gram(const Slots<NS>& W, int oG, const doubl
                 ynew = qd.y * rinv;
             }
         }
-#endif
         // nnls.f: reject if the column is numerically dependent on P (unorm + |a_new|*0.01 == unorm, i.e.
         // rho < ~1e-14 unorm) or if its new coefficient ("ztest") is not positive
         const bool ok = (rho2 > 0.0) && (rho2 > 1.2e-28 * s1) && (!need_positive || ynew > 0.0);

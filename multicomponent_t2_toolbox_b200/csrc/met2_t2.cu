@@ -118,7 +118,7 @@ static int t2_launch_full_factors(const T2Args& A, int ntab, const double* G, co
 
 extern "C" int64_t met2_t2_workspace_bytes(int64_t V, const met2_t2_cfg* cfg) {
     if (t2_check_cfg(cfg) || V < 0) return -1;
-    T2Geom g = t2_geometry_any(V, cfg);
+    T2Geom g = t2_geometry_any(V, cfg, read_overrides());
     size_t b = 0;
     b += align256(sizeof(int) * (size_t)cfg->nA) * 2;
     b += align256(sizeof(int) * (size_t)(cfg->nA + 1));
@@ -146,10 +146,13 @@ static int t2_fit_impl(const double* sig, const int32_t* fa_index, int64_t V, co
     if (cfg->method == MET2_REG_LCURVE && !lambdas) return set_error(MET2_ERR_ARG, "met2_t2_fit: L-curve needs lambdas");
     if (cfg->method == MET2_REG_GCV && (cfg->flags & MET2_T2_FLAG_GCV_GRID) && !lambdas)
         return set_error(MET2_ERR_ARG, "met2_t2_fit: the GCV grid mode needs lambdas");
+    if (t2_echo_eligible(cfg) && (!red_basis || !red_coef))
+        return set_error(MET2_ERR_ARG, "met2_t2_fit: MET2_T2_FLAG_ECHO_SPACE needs the reduced echo basis (met2_echo_basis)");
     if (V == 0) return MET2_OK;
     if (V > 0x7fffffffLL) return set_error(MET2_ERR_ARG, "met2_t2_fit: V too large for one call");
     cudaStream_t st = (cudaStream_t)stream;
-    T2Geom g = t2_geometry_any(V, cfg);
+    const Overrides ov = read_overrides();
+    T2Geom g = t2_geometry_any(V, cfg, ov);
     T2Args A;
     A.sig = sig; A.fa_index = fa_index; A.V = V; A.cfg = *cfg;
     A.dic = dic; A.dicT = dicT; A.G = G; A.kband = kband; A.lambdas = lambdas; A.logT2 = logT2; A.comp = comp;
@@ -170,8 +173,7 @@ static int t2_fit_impl(const double* sig, const int32_t* fa_index, int64_t V, co
     A.lam_tab = nullptr;
     A.ntab = 0;
     A.ntab_use = 0;
-    A.lcurve_switch = T2_LCURVE_SWITCH;
-    if (const char* ev = getenv("MET2_LCURVE_SWITCH")) A.lcurve_switch = atof(ev);   // tuning / A-B runs
+    A.lcurve_switch = ov.lcurve_switch_set ? ov.lcurve_switch : T2_LCURVE_SWITCH;
     if (const int ntab = t2_full_tables(cfg)) {
         double* lam_tab = reinterpret_cast<double*>(w);  w += align256(sizeof(double) * T2_NTAB_MAX);
         double* tfull = reinterpret_cast<double*>(w);
@@ -183,10 +185,6 @@ static int t2_fit_impl(const double* sig, const int32_t* fa_index, int64_t V, co
         A.ntab = ntab;
         // full-set starts of the NNLS solves: X2 only (measured; for BayesReg the tables serve the evidence)
         A.ntab_use = (cfg->method == MET2_REG_X2) ? ntab : 0;
-        if (const char* ev = getenv("MET2_T2_NTAB")) {   // tuning / A-B runs
-            const int t = atoi(ev);
-            if (t >= 0 && t < A.ntab_use) A.ntab_use = t;
-        }
         A.tfull = tfull;
         A.lam_tab = lam_tab;
     }
@@ -207,8 +205,8 @@ static int t2_fit_impl(const double* sig, const int32_t* fa_index, int64_t V, co
     if (t2_echo_eligible(cfg)) {
         const bool small = (cfg->echo_rank == MET2_ECHO_RANK_SMALL);
         if (cfg->method == MET2_REG_LCURVE || cfg->method == MET2_REG_BAYESREG)
-            return small ? t2_launch_echo_reg_r16(A, st) : t2_launch_echo_reg_r24(A, st);
-        return small ? t2_launch_echo_r16(A, st) : t2_launch_echo_r24(A, st);
+            return small ? t2_launch_echo_reg_r16(A, ov, st) : t2_launch_echo_reg_r24(A, ov, st);
+        return small ? t2_launch_echo_r16(A, ov, st) : t2_launch_echo_r24(A, ov, st);
     }
     switch (cfg->method) {
         case MET2_REG_NNLS: return t2_launch_nnls(A, g, st);

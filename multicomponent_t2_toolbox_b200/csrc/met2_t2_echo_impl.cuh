@@ -89,13 +89,9 @@ __host__ __device__ __forceinline__ int echo_table_doubles(int n, int m) {
     return (n * t2_ldg(n) + EC_NCOL * EC_LDD + m * RD + tri(RD) + 3 * 64 + 8 + EC_RC_DOUBLES + 31) & ~31;
 }
 
-// unrolled, compile-time-indexed inner products in the X2 / T2SPARC kernels only (see echo_tmul below)
+// unrolled, compile-time-indexed inner products and factor update in the X2 / T2SPARC kernels only (see echo_tmul
+// below); the unrolled update in the L-curve / BayesReg kernel measured slower (L-curve 296 -> 319 ms, BayesReg 340 -> 350)
 constexpr bool ECHO_UNROLLED_TRI = (MET2_ECHO_PART == 1);
-#ifndef MET2_ECHO_REG_UNROLL_UPD
-#define MET2_ECHO_REG_UNROLL_UPD 0     // A/B switch: the unrolled factor update in the L-curve / BayesReg kernel too —
-                                       // measured slower (GPU call 28: L-curve 296 -> 319 ms, BayesReg 340 -> 350 ms)
-#endif
-constexpr bool ECHO_UNROLLED_UPD = ECHO_UNROLLED_TRI || (MET2_ECHO_REG_UNROLL_UPD != 0);
 
 // g = Ct^T v for v at S[oV .. oV + RD): lane + 32 s = column (NC column slots per lane: nT2 <= 32 NC).
 template <int NC>
@@ -251,7 +247,7 @@ __device__ __forceinline__ bool echo_update_T(const Slots<NS>& W, const EchoOff&
     }
     __syncwarp();
     // ---- T' = T Q, one row of T per lane (row r has entries in columns j >= r)
-    if (ECHO_UNROLLED_UPD) {
+    if (ECHO_UNROLLED_TRI) {
         // compile-time column index: constant triangle offsets, (delta, q, u) of two columns per 128-bit broadcast load
         double acc = 0.0;
 #pragma unroll
@@ -565,27 +561,18 @@ __device__ __forceinline__ void echo_stage_diag(const T2Args& A, int ncol, int n
     }
 }
 
-#ifndef MET2_ECHO_MAX_THREADS
-#define MET2_ECHO_MAX_THREADS 640       // A/B switch: 512 = 16 warps at 128 registers, 640 = 20 warps at 96 registers
-#endif
-constexpr int ECHO_MAX_THREADS = MET2_ECHO_MAX_THREADS;
 // Per-kernel launch bounds, measured on the config-2 volume (profiles/r02_ab_echo_warps.json; 640 / 768 / 896 / 1024
 // threads = 20 / 24 / 28 / 30 warps per SM at 96 / 80 / 72 / 64 registers): X2 136.6 / 146.1 / 142.2 / 141.3 ms and the
 // L-curve 293 / 344 / 363 / 394 ms are best at 640 (more resident warps sit in more phases of the kernel: instruction
 // fetch), T2SPARC 56.8 / 54.6 / 52.3 / 51.4 ms and BayesReg (60 bins) 366 / 353 / 353 / 339 ms at 1024.
-#ifndef MET2_ECHO_TIK_MAX_THREADS
-#define MET2_ECHO_TIK_MAX_THREADS 1024
-#endif
-constexpr int ECHO_TIK_MAX_THREADS = MET2_ECHO_TIK_MAX_THREADS;
+constexpr int ECHO_MAX_THREADS = 640;
+constexpr int ECHO_TIK_MAX_THREADS = 1024;
 
-static int echo_warps(size_t tables, size_t per_warp, int max_threads = ECHO_MAX_THREADS) {
+static int echo_warps(size_t tables, size_t per_warp, const Overrides& ov, int max_threads = ECHO_MAX_THREADS) {
     const size_t budget = 227 * 1024 - 1024;
     int warps = tables < budget ? (int)((budget - tables) / per_warp) : 0;
     if (warps > max_threads / 32) warps = max_threads / 32;
-    if (const char* ev = getenv("MET2_T2_WARPS")) {
-        const int w = atoi(ev);
-        if (w >= 1 && w < warps) warps = w;
-    }
+    if (ov.t2_warps >= 1 && ov.t2_warps < warps) warps = ov.t2_warps;
     return warps;
 }
 
@@ -934,10 +921,10 @@ __global__ void __launch_bounds__(ECHO_TIK_MAX_THREADS, 1) t2_echo_tik_kernel(T2
 }
 
 template <int NC, int ME>
-static int t2_launch_echo_tik(const T2Args& A, cudaStream_t st) {
+static int t2_launch_echo_tik(const T2Args& A, const Overrides& ov, cudaStream_t st) {
     const size_t tables = sizeof(double) * (size_t)echo_tik_table_doubles<NC>(A.cfg.nTE);
     const size_t per_warp = sizeof(double) * (size_t)echo_tik_warp_doubles<NC>();
-    const int warps = echo_warps(tables, per_warp, ECHO_TIK_MAX_THREADS);
+    const int warps = echo_warps(tables, per_warp, ov, ECHO_TIK_MAX_THREADS);
     if (warps < 1) return set_error(MET2_ERR_UNSUPPORTED, "met2_t2_fit (echo space): tables do not fit in shared memory");
     const size_t smem = tables + per_warp * warps;
     int sms = sm_count();
@@ -950,18 +937,18 @@ static int t2_launch_echo_tik(const T2Args& A, cudaStream_t st) {
 }
 
 template <int ME>
-static int t2_launch_echo_me(const T2Args& A, cudaStream_t st) {
+static int t2_launch_echo_me(const T2Args& A, const Overrides& ov, cudaStream_t st) {
     const int n = A.cfg.nT2;
     if (A.cfg.method == MET2_REG_T2SPARC) {
         const int nc = (n + 31) / 32;
-        if (nc <= 1) return t2_launch_echo_tik<1, ME>(A, st);
-        if (nc == 2) return t2_launch_echo_tik<2, ME>(A, st);
-        if (nc == 3) return t2_launch_echo_tik<3, ME>(A, st);
-        return t2_launch_echo_tik<4, ME>(A, st);
+        if (nc <= 1) return t2_launch_echo_tik<1, ME>(A, ov, st);
+        if (nc == 2) return t2_launch_echo_tik<2, ME>(A, ov, st);
+        if (nc == 3) return t2_launch_echo_tik<3, ME>(A, ov, st);
+        return t2_launch_echo_tik<4, ME>(A, ov, st);
     }
     const size_t tables = sizeof(double) * (size_t)echo_table_doubles(n, A.cfg.nTE);
     const size_t per_warp = sizeof(double) * (size_t)echo_warp_doubles();
-    const int warps = echo_warps(tables, per_warp);
+    const int warps = echo_warps(tables, per_warp, ov);
     if (warps < 1) return set_error(MET2_ERR_UNSUPPORTED, "met2_t2_fit (echo space): tables do not fit in shared memory");
     const size_t smem = tables + per_warp * warps;
     int sms = sm_count();
@@ -975,11 +962,9 @@ static int t2_launch_echo_me(const T2Args& A, cudaStream_t st) {
 
 }  // namespace MET2_ECHO_NS
 
-int MET2_ECHO_LAUNCH(const T2Args& A, cudaStream_t st) {
-    if (!A.red_basis || !A.red_coef)
-        return set_error(MET2_ERR_ARG, "met2_t2_fit: MET2_T2_FLAG_ECHO_SPACE needs the reduced echo basis (met2_echo_basis)");
-    if (A.cfg.nTE <= 32) return MET2_ECHO_NS::t2_launch_echo_me<1>(A, st);
-    return MET2_ECHO_NS::t2_launch_echo_me<2>(A, st);
+int MET2_ECHO_LAUNCH(const T2Args& A, const Overrides& ov, cudaStream_t st) {
+    if (A.cfg.nTE <= 32) return MET2_ECHO_NS::t2_launch_echo_me<1>(A, ov, st);
+    return MET2_ECHO_NS::t2_launch_echo_me<2>(A, ov, st);
 }
 
 }  // namespace met2

@@ -41,10 +41,6 @@ namespace MET2_ECHO_NS {
 constexpr int EV_RR = RD / 8;   // rows of the evidence state S_j per lane: rg + 8 a, rg = lane & 7
 constexpr int EV_CC = RD / 4;   // columns per lane: cb EV_CC + b, cb = lane >> 3
 
-#ifndef MET2_LCURVE_GRAM_COLD
-#define MET2_LCURVE_GRAM_COLD 0   // A/B switch: cold-start the Gram-domain grid points (prunes nnls_gram's warm-start code,
-                                  // 9.2 k -> 8.7 k SASS instructions) — measured much slower (GPU call 29: 293 -> 466 ms)
-#endif
 constexpr int EV_LCURVE_PMAX = 32;          // positions of the Gram-domain factor of the L-curve kernel (one slot per lane)
 template <int METHOD>
 struct EchoRegPmax {
@@ -335,10 +331,11 @@ __global__ void __launch_bounds__(EchoRegThreads<METHOD, NC>::value, 1) t2_echo_
                     } else if (phase == PH_PLAIN ||
                                (METHOD == MET2_REG_LCURVE && !in_echo && lam_cur < A.lcurve_switch && p < PMAX)) {
                         // Gram domain: the plain solve from the empty set (<= RD positions), or a Tikhonov solve on
-                        // G + lam K from the carried-over positions (<= PMAX; a full factor sends the point to echo space)
+                        // G + lam K from the carried-over positions (<= PMAX; a full factor sends the point to echo space).
+                        // Cold-starting those points as well measured much slower (L-curve 293 -> 466 ms).
                         const bool plain = (METHOD == MET2_REG_BAYESREG) ? true : (phase == PH_PLAIN);   // BayesReg: compile-time
                         const int pn = nnls_gram<NC, GSH, 1>(W, oG, Gg, ldg, oKb, !plain, lam_cur, n, plain ? RD : PMAX, lane,
-                                                              nst, (MET2_LCURVE_GRAM_COLD || plain) ? 0 : p, false);
+                                                              nst, plain ? 0 : p, false);
                         double a = 0.0;
 #pragma unroll
                         for (int s = 0; s < NC; ++s) {
@@ -474,10 +471,10 @@ __global__ void __launch_bounds__(EchoRegThreads<METHOD, NC>::value, 1) t2_echo_
 }
 
 template <int METHOD, int NC, int ME>
-static int t2_launch_echo_reg_one(const T2Args& A, cudaStream_t st) {
+static int t2_launch_echo_reg_one(const T2Args& A, const Overrides& ov, cudaStream_t st) {
     const size_t tables = sizeof(double) * (size_t)echo_reg_table_doubles<NC>(A.cfg.nT2, A.cfg.nTE);
     const size_t per_warp = sizeof(double) * (size_t)echo_reg_warp_doubles<METHOD, NC>();
-    const int warps = echo_warps(tables, per_warp, EchoRegThreads<METHOD, NC>::value);
+    const int warps = echo_warps(tables, per_warp, ov, EchoRegThreads<METHOD, NC>::value);
     if (warps < 1) return set_error(MET2_ERR_UNSUPPORTED, "met2_t2_fit (echo space): tables do not fit in shared memory");
     const size_t smem = tables + per_warp * warps;
     int sms = sm_count();
@@ -490,21 +487,19 @@ static int t2_launch_echo_reg_one(const T2Args& A, cudaStream_t st) {
 }
 
 template <int METHOD>
-static int t2_launch_echo_reg_method(const T2Args& A, cudaStream_t st) {
+static int t2_launch_echo_reg_method(const T2Args& A, const Overrides& ov, cudaStream_t st) {
     const bool wide = A.cfg.nT2 > 64, me2 = A.cfg.nTE > 32;
-    if (!wide && !me2) return t2_launch_echo_reg_one<METHOD, 2, 1>(A, st);
-    if (!wide && me2) return t2_launch_echo_reg_one<METHOD, 2, 2>(A, st);
-    if (wide && !me2) return t2_launch_echo_reg_one<METHOD, 4, 1>(A, st);
-    return t2_launch_echo_reg_one<METHOD, 4, 2>(A, st);
+    if (!wide && !me2) return t2_launch_echo_reg_one<METHOD, 2, 1>(A, ov, st);
+    if (!wide && me2) return t2_launch_echo_reg_one<METHOD, 2, 2>(A, ov, st);
+    if (wide && !me2) return t2_launch_echo_reg_one<METHOD, 4, 1>(A, ov, st);
+    return t2_launch_echo_reg_one<METHOD, 4, 2>(A, ov, st);
 }
 
 }  // namespace MET2_ECHO_NS
 
-int MET2_ECHO_LAUNCH(const T2Args& A, cudaStream_t st) {
-    if (!A.red_basis || !A.red_coef)
-        return set_error(MET2_ERR_ARG, "met2_t2_fit: MET2_T2_FLAG_ECHO_SPACE needs the reduced echo basis (met2_echo_basis)");
-    if (A.cfg.method == MET2_REG_LCURVE) return MET2_ECHO_NS::t2_launch_echo_reg_method<MET2_REG_LCURVE>(A, st);
-    return MET2_ECHO_NS::t2_launch_echo_reg_method<MET2_REG_BAYESREG>(A, st);
+int MET2_ECHO_LAUNCH(const T2Args& A, const Overrides& ov, cudaStream_t st) {
+    if (A.cfg.method == MET2_REG_LCURVE) return MET2_ECHO_NS::t2_launch_echo_reg_method<MET2_REG_LCURVE>(A, ov, st);
+    return MET2_ECHO_NS::t2_launch_echo_reg_method<MET2_REG_BAYESREG>(A, ov, st);
 }
 
 }  // namespace met2

@@ -45,7 +45,7 @@ struct T2Args {
     int ntab;                // tables built
     int ntab_use;            // how many of them the NNLS full-set starts consult
     double lcurve_switch;    // echo-space L-curve: grid points below this lambda are solved in the Gram domain
-                             // (met2_t2_echo_reg_impl.cuh); MET2_LCURVE_SWITCH overrides it for A/B runs
+                             // (met2_t2_echo_reg_impl.cuh); MET2_LCURVE_SWITCH overrides it (met2_host.h)
 };
 
 constexpr int T2_NTAB_X2 = 3;      // measured on config 2 (T2 stage): no table 444 ms, 2 tables 398, 3 tables 390, 4 tables 390
@@ -890,7 +890,7 @@ struct T2Geom {
 };
 
 template <int NS>
-static inline T2Geom t2_geometry(long long V, const met2_t2_cfg* cfg) {
+static inline T2Geom t2_geometry(long long V, const met2_t2_cfg* cfg, const Overrides& ov) {
     T2Geom g;
     const int n = cfg->nT2, m = cfg->nTE;
     const bool plain = (cfg->method == MET2_REG_NNLS);
@@ -903,10 +903,7 @@ static inline T2Geom t2_geometry(long long V, const met2_t2_cfg* cfg) {
     int warps = (int)((budget - tables) / per_warp);
     if (warps > T2_MAX_THREADS / 32) warps = T2_MAX_THREADS / 32;
     if (warps < 1) warps = 1;
-    if (const char* ev = getenv("MET2_T2_WARPS")) {   // tuning/diagnostic override (never raises the limit)
-        int w = atoi(ev);
-        if (w >= 1 && w < warps) warps = w;
-    }
+    if (ov.t2_warps >= 1 && ov.t2_warps < warps) warps = ov.t2_warps;
     g.warps = warps;
     g.smem = tables + per_warp * warps;
     int per_sm = (int)(budget / (g.smem + 1024));
@@ -915,7 +912,7 @@ static inline T2Geom t2_geometry(long long V, const met2_t2_cfg* cfg) {
     if (sms <= 0) sms = 148;
     g.grid = sms * per_sm;
     // guided self-scheduling of the tile list (t2_tiles_kernel): ~8 large tiles per CTA, then small tiles for the last
-    // ~12 % of the voxels; MET2_T2_TILE=<n> forces a uniform tile size (tuning / A-B runs)
+    // ~12 % of the voxels; MET2_T2_TILE=<n> forces a uniform tile size
     long long big = V / ((long long)g.grid * 8);
     big = (big + 31) & ~31LL;
     if (big < 64) big = 64;
@@ -923,22 +920,19 @@ static inline T2Geom t2_geometry(long long V, const met2_t2_cfg* cfg) {
     g.tile_big = (int)big;
     g.tile_small = T2_TILE_MIN;
     g.switch_off = (int)(V - V / 8);
-    if (const char* ev = getenv("MET2_T2_TILE")) {
-        int t = atoi(ev);
-        if (t >= 1) {
-            g.tile_big = g.tile_small = t;
-            g.switch_off = (int)V;
-        }
+    if (ov.t2_tile >= 1) {
+        g.tile_big = g.tile_small = ov.t2_tile;
+        g.switch_off = (int)V;
     }
     g.max_tiles = (int)(V / g.tile_small) + cfg->nA + 1;
     return g;
 }
 
-static inline T2Geom t2_geometry_any(long long V, const met2_t2_cfg* cfg) {
+static inline T2Geom t2_geometry_any(long long V, const met2_t2_cfg* cfg, const Overrides& ov) {
     int ns = (cfg->nT2 + 31) / 32;
-    if (ns <= 2) return t2_geometry<2>(V, cfg);
-    if (ns == 3) return t2_geometry<3>(V, cfg);
-    return t2_geometry<4>(V, cfg);
+    if (ns <= 2) return t2_geometry<2>(V, cfg, ov);
+    if (ns == 3) return t2_geometry<3>(V, cfg, ov);
+    return t2_geometry<4>(V, cfg, ov);
 }
 
 template <int NS, int ME, int METHOD>
@@ -972,10 +966,10 @@ int t2_launch_bayesreg(const T2Args& A, const T2Geom& g, cudaStream_t st);
 int t2_launch_gcv(const T2Args& A, const T2Geom& g, cudaStream_t st);
 // met2_t2_echo_r16.cu / met2_t2_echo_r24.cu (MET2_T2_FLAG_ECHO_SPACE; rank = cfg.echo_rank)
 bool t2_echo_eligible(const met2_t2_cfg* cfg);
-int t2_launch_echo_r16(const T2Args& A, cudaStream_t st);
-int t2_launch_echo_r24(const T2Args& A, cudaStream_t st);
+int t2_launch_echo_r16(const T2Args& A, const Overrides& ov, cudaStream_t st);
+int t2_launch_echo_r24(const T2Args& A, const Overrides& ov, cudaStream_t st);
 // met2_t2_echo_reg_r16.cu / met2_t2_echo_reg_r24.cu (L-curve and BayesReg in the reduced echo space)
-int t2_launch_echo_reg_r16(const T2Args& A, cudaStream_t st);
-int t2_launch_echo_reg_r24(const T2Args& A, cudaStream_t st);
+int t2_launch_echo_reg_r16(const T2Args& A, const Overrides& ov, cudaStream_t st);
+int t2_launch_echo_reg_r24(const T2Args& A, const Overrides& ov, cudaStream_t st);
 
 }  // namespace met2

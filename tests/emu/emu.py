@@ -51,7 +51,7 @@ def build(force=False):
         return LIB
     os.makedirs(BUILD, exist_ok=True)
     flags = ["-std=c++17", "-O2", "-ffp-contract=off", "-fPIC", "-DMET2_HOST_EMU=1", "-x", "c++", "-I", HERE, "-I", CSRC,
-             "-I", os.path.join(ROOT, "include")] + os.environ.get("EMU_EXTRA_DEFS", "").split()   # experiments only
+             "-I", os.path.join(ROOT, "include")]
 
     def compile_one(src):
         obj = os.path.join(BUILD, os.path.basename(src) + ".o")
@@ -82,6 +82,7 @@ def lib():
         _lib.met2_fa_workspace_bytes.argtypes = [ctypes.c_int64, ctypes.POINTER(FaCfg)]
         _lib.met2_segment_workspace_bytes.restype = ctypes.c_int64
         _lib.met2_segment_workspace_bytes.argtypes = [ctypes.c_int, ctypes.c_int]
+        _lib.met2_launch_count.restype = ctypes.c_int64
     return _lib
 
 

@@ -103,6 +103,17 @@ def test_echo_space_x2_kernel_against_reference(setup):
         assert abs(lam["reg"][i] - reg) < 1e-9 * max(1.0, abs(reg))
 
 
+def test_echo_space_without_tables_rejected_before_any_launch(setup):
+    """MET2_T2_FLAG_ECHO_SPACE with NULL red_basis / red_coef is an argument error, returned before the sort kernels or
+    anything else is enqueued."""
+    g, gr = setup["g"], setup["gr"]
+    _, sig, fa = _pick(g, 4)
+    before = emu.lib().met2_launch_count()
+    with pytest.raises(RuntimeError, match=r"\(-1\): met2_t2_fit: MET2_T2_FLAG_ECHO_SPACE needs the reduced echo basis"):
+        _run("forward", sig, fa, setup["Dic"], gr["L"], gr["T2s"], "X2", flags=64)   # flag set, echo=False: no tables
+    assert emu.lib().met2_launch_count() == before
+
+
 def test_echo_space_invt2_and_rejects_non_diagonal(setup):
     g = setup["g"]
     gi = O._grids("X2", "InvT2", "spline", 40.0, 32, 10.0, 1000.0)
