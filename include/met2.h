@@ -201,6 +201,24 @@ int met2_segment_means(const double* sig, const int32_t* fa_index, const int32_t
 int met2_nesma_filter(const double* vol, const int32_t* mask, int nx, int ny, int nz, int nt, int half_window,
                       double threshold_percent, double* out, double* tmp, void* stream);
 
+/* Optional Step-1 preprocessing, --denoise TV (motor/motor_recon_met2_real_data.py:293-303): per echo volume
+ * vol[..., t] with its axes of size 1 dropped (np.squeeze), scikit-image's noise estimate and Chambolle TV filter.
+ * vol/out [nx][ny][nz][nt] C-order; out must not alias vol.  At least one spatial axis must be longer than 1.
+ *
+ * met2_noise_sigma: sigma[t] = median(|c| over the nonzero c) / norm.ppf(0.75), c = the single-level db2 detail band
+ * (PyWavelets 'symmetric' mode, the high-pass along every remaining axis); NaN if a coefficient is NaN or none is
+ * nonzero (skimage.restoration.estimate_sigma(vol, channel_axis=None)).  sigma [nt], device.
+ *
+ * met2_tv_chambolle: skimage.restoration.denoise_tv_chambolle(vol, weight[t], eps, max_iter) per echo (the nd-Chambolle
+ * iteration with tau = 1 / (2 ndim), stopping when |E_prev - E| < eps * E_init).  weight [nt] is a device array, so that
+ * 2 * sigma can be passed without a round trip; iterations [nt] int32 receives the number of iterations run per echo.
+ * Both are bitwise equal to the NumPy restatement in tests/tv_oracle.py (energy sums in NumPy's pairwise order). */
+int64_t met2_noise_sigma_workspace_bytes(int nx, int ny, int nz, int nt);
+int met2_noise_sigma(const double* vol, int nx, int ny, int nz, int nt, double* sigma, void* workspace, void* stream);
+int64_t met2_tv_workspace_bytes(int nx, int ny, int nz, int nt);
+int met2_tv_chambolle(const double* vol, int nx, int ny, int nz, int nt, const double* weight, double eps, int max_iter,
+                      double* out, int32_t* iterations, void* workspace, void* stream);
+
 /* Diagnostics */
 const char* met2_last_error(void);
 int met2_version(void);

@@ -99,6 +99,63 @@ def nesma_filter(data, mask, half_window=6, threshold=2.5, device=None):
     return out
 
 
+def _volume(data, dev):
+    if isinstance(data, np.ndarray):
+        data = torch.as_tensor(np.ascontiguousarray(data, dtype=np.float64))
+    vol = data.to(device=dev, dtype=torch.float64).contiguous()
+    if vol.dim() != 4:
+        raise ValueError("data must be [nx, ny, nz, nt]")
+    return vol
+
+
+def noise_sigma(data, device=None):
+    """Per-echo noise estimate of Step 1 with --denoise TV (motor...:296) on the GPU (met2_noise_sigma): for every echo
+    t, skimage.restoration.estimate_sigma(np.squeeze(data[..., t]), channel_axis=None), the median absolute db2 detail
+    coefficient over 0.6745.  data[nx, ny, nz, nt]; returns a CUDA float64 tensor [nt]."""
+    dev = _require_cuda(device)
+    lib = _lib.load()
+    vol = _volume(data, dev)
+    nx, ny, nz, nt = vol.shape
+    sigma = torch.empty(nt, dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
+        nbytes = lib.met2_noise_sigma_workspace_bytes(nx, ny, nz, nt)
+        if nbytes < 0:
+            _lib.check(int(nbytes), "met2_noise_sigma_workspace_bytes")
+        ws = torch.empty(int(nbytes), dtype=torch.uint8, device=dev)
+        _lib.check(lib.met2_noise_sigma(_ptr(vol), nx, ny, nz, nt, _ptr(sigma), _ptr(ws), _stream()), "met2_noise_sigma")
+    return sigma
+
+
+def tv_denoise(data, weight=None, eps=2e-4, max_num_iter=200, device=None):
+    """Chambolle total-variation denoising of every echo volume on the GPU (met2_tv_chambolle):
+    skimage.restoration.denoise_tv_chambolle(np.squeeze(data[..., t]), weight[t], eps, max_num_iter) for every t.
+    weight=None uses 2 * noise_sigma(data), Step 1 of the reference with --denoise TV (motor...:293-303); otherwise a
+    scalar or one weight per echo.  Returns (denoised CUDA tensor like data, iterations run per echo, int32 [nt])."""
+    dev = _require_cuda(device)
+    lib = _lib.load()
+    vol = _volume(data, dev)
+    nx, ny, nz, nt = vol.shape
+    if weight is None:
+        w = 2.0 * noise_sigma(vol, dev)
+    else:
+        w = torch.as_tensor(weight, dtype=torch.float64).to(dev).reshape(-1)
+        if w.numel() == 1:
+            w = w.expand(nt)
+        if w.numel() != nt:
+            raise ValueError("weight must be a scalar or have one value per echo (%d)" % nt)
+        w = w.contiguous()
+    out = torch.empty_like(vol)
+    iterations = torch.empty(nt, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        nbytes = lib.met2_tv_workspace_bytes(nx, ny, nz, nt)
+        if nbytes < 0:
+            _lib.check(int(nbytes), "met2_tv_workspace_bytes")
+        ws = torch.empty(int(nbytes), dtype=torch.uint8, device=dev)
+        _lib.check(lib.met2_tv_chambolle(_ptr(vol), nx, ny, nz, nt, _ptr(w), float(eps), int(max_num_iter), _ptr(out),
+                                         _ptr(iterations), _ptr(ws), _stream()), "met2_tv_chambolle")
+    return out, iterations
+
+
 def segment_means(sig, fa_index, labels, n_seg, dictionary):
     """Per-segment mean signal and mean kernel (met2_segment_means; motor...:377-392 and
     motor_recon_met2_real_data_ROI.py:408-423).  sig[V, nTE], fa_index[V], labels[V] in [0, n_seg) (else: no segment).
