@@ -219,6 +219,26 @@ int64_t met2_tv_workspace_bytes(int nx, int ny, int nz, int nt);
 int met2_tv_chambolle(const double* vol, int nx, int ny, int nz, int nt, const double* weight, double eps, int max_iter,
                       double* out, int32_t* iterations, void* workspace, void* stream);
 
+/* Per-voxel bootstrap uncertainty of the six maps (no counterpart in the reference).  Definition in
+ * csrc/met2_boot.cu; both calls are bitwise equal to the NumPy restatement in tests/boot_oracle.py.
+ *
+ * met2_boot_resample: wild-bootstrap replicates with Rademacher signs, rows r = v*B + b of rep_sig [V*B][nTE]:
+ * s*_e = est_e +/- (sig_e - est_e), the sign from bit e of splitmix64(seed, (voxel_offset + v)*B + b), so that a voxel's
+ * replicates depend only on its position in the whole voxel list.  sig [V][nTE] is the signal the point fit used,
+ * est_signal [V][nTE] its fitted signal, fa_index [V] its flip-angle index; rep_fa_index [V*B] repeats it (the FA is
+ * held at the point estimate).  1 <= B <= 1024, 1 <= nTE <= MET2_MAX_NTE.
+ *
+ * met2_boot_summary: over the replicates b of voxel v whose rep_status lacks MET2_ST_SKIPPED (n_valid [V] of them), per
+ * map (columns of rep_maps [V*B][6], the `maps` of met2_t2_fit): stats [V][6][4] = mean, sd (ddof 1), 2.5th and 97.5th
+ * percentile (numpy's 'linear' method).  n_valid = 0: zeros; a NaN among a map's values: that map's four numbers NaN.
+ *
+ * Both: V = 0 is a no-op; bad arguments return MET2_ERR_ARG before anything is enqueued. */
+int met2_boot_resample(const double* sig, const double* est_signal, const int32_t* fa_index, int64_t V, int nTE,
+                       int B, uint64_t seed, int64_t voxel_offset, double* rep_sig, int32_t* rep_fa_index,
+                       void* stream);
+int met2_boot_summary(const double* rep_maps, const uint32_t* rep_status, int64_t V, int B, double* stats,
+                      int32_t* n_valid, void* stream);
+
 /* Diagnostics */
 const char* met2_last_error(void);
 int met2_version(void);

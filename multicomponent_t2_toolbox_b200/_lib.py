@@ -53,6 +53,10 @@ SIGNATURES = {
     "met2_tv_workspace_bytes": (ctypes.c_int64, [ctypes.c_int] * 4),
     "met2_tv_chambolle": (ctypes.c_int, [c_void_p] + [ctypes.c_int] * 4 + [c_void_p, ctypes.c_double, ctypes.c_int,
                                                                           c_void_p, c_void_p, c_void_p, c_void_p]),
+    "met2_boot_resample": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_int,
+                                          ctypes.c_uint64, ctypes.c_int64, c_void_p, c_void_p, c_void_p]),
+    "met2_boot_summary": (ctypes.c_int, [c_void_p, c_void_p, ctypes.c_int64, ctypes.c_int, c_void_p, c_void_p,
+                                         c_void_p]),
     "met2_last_error": (ctypes.c_char_p, []),
     "met2_version": (ctypes.c_int, []),
     "met2_echo_rank": (ctypes.c_int, [ctypes.c_int]),

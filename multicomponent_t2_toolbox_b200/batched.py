@@ -486,3 +486,53 @@ class Met2Plan:
         fa = self.fa_fit(sig if sig_fa is None else sig_fa)
         t2 = self.t2_fit(sig, fa["fa_index"])
         return fa, t2
+
+    # ------------------------------------------------------------------ bootstrap uncertainty of the maps
+    def bootstrap(self, sig, fa_index, est_signal, B=100, seed=0, voxel_offset=0, max_replicates=1 << 21):
+        """Per-voxel wild-bootstrap uncertainty of the six maps (definition in csrc/met2_boot.cu).
+
+        sig[V, nTE] is the signal the point fit used, fa_index[V] and est_signal[V, nTE] are that fit's results.  Each
+        voxel gets B replicates (1 <= B <= 1024), refitted by this plan's `t2_fit` at the point fit's flip angle, with
+        lambda re-selected.  voxel_offset is the position of voxel 0 in the whole voxel list: a voxel's replicates
+        depend only on that position and `seed`, so any split of the list gives the same result.  Voxels are processed
+        in chunks of max_replicates // B (replicate buffers of about 1 KB per replicate at 32 echoes and 60 bins).
+        Returns CUDA tensors stats[V, 6, 4] (mean, sd, p2.5, p97.5 of MWF, IEWF, FWF, T2_M, T2_IE, TWC) and n_valid[V]
+        (int32, the replicates whose fit was not skipped).  All work is enqueued on the current stream."""
+        B = int(B)
+        if not 1 <= B <= 1024:
+            raise ValueError("B must be in [1, 1024], got %d" % B)
+        seed, voxel_offset = int(seed), int(voxel_offset)
+        if not 0 <= seed < 1 << 64:
+            raise ValueError("seed must be an unsigned 64-bit integer")
+        if voxel_offset < 0:
+            raise ValueError("voxel_offset must be >= 0")
+        if int(max_replicates) < B:
+            raise ValueError("max_replicates must be at least B")
+        sig = self._signals(sig)
+        est = self._signals(est_signal)
+        V = sig.shape[0]
+        dev = self.dev
+        fa_index = torch.as_tensor(fa_index).to(device=dev, dtype=torch.int32).contiguous()
+        if fa_index.shape != (V,) or est.shape[0] != V:
+            raise ValueError("sig, fa_index and est_signal must describe the same V voxels")
+        stats = torch.zeros((V, 6, 4), dtype=torch.float64, device=dev)
+        n_valid = torch.zeros(V, dtype=torch.int32, device=dev)
+        if V == 0:
+            return stats, n_valid
+        chunk = min(V, int(max_replicates) // B)
+        with torch.cuda.device(dev):
+            rep_sig = torch.empty((chunk * B, self.nTE), dtype=torch.float64, device=dev)
+            rep_fa = torch.empty(chunk * B, dtype=torch.int32, device=dev)
+            bufs = None       # the refits' outputs, allocated by the first chunk and reused by the others
+            for lo in range(0, V, chunk):
+                n = min(chunk, V - lo)
+                R = n * B
+                _lib.check(self.lib.met2_boot_resample(_ptr(sig[lo:]), _ptr(est[lo:]), _ptr(fa_index[lo:]), n, self.nTE,
+                                                       B, seed, voxel_offset + lo, _ptr(rep_sig), _ptr(rep_fa),
+                                                       _stream()), "met2_boot_resample")
+                fits = self.t2_fit(rep_sig[:R], rep_fa[:R],
+                                   out=None if bufs is None else {k: v[:R] for k, v in bufs.items()})
+                bufs = bufs if bufs is not None else fits
+                _lib.check(self.lib.met2_boot_summary(_ptr(fits["maps"]), _ptr(fits["status"]), n, B, _ptr(stats[lo:]),
+                                                      _ptr(n_valid[lo:]), _stream()), "met2_boot_summary")
+        return stats, n_valid

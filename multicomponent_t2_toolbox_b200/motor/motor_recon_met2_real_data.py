@@ -19,6 +19,7 @@ from .. import _lib, batched, nifti_io, pipeline
 from ..reference_api import create_Laplacian_matrix, fitting_slice_T2  # noqa: F401
 
 OUTPUTS = ("MWF", "IEWF", "FWF", "T2_M", "T2_IE", "TWC", "FA", "fsol_4D", "Est_Signal", "reg_param")
+BOOTSTRAP_OUTPUTS = tuple(name + "_bootstrap" for name in pipeline.MAP_NAMES) + ("bootstrap_n_valid",)
 
 
 def tv_denoise(data):
@@ -61,9 +62,13 @@ def _warm_gpus(n_gpus):
 
 
 def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR, reg_method, reg_matrix, denoise,
-                     FA_method, FA_smooth, myelin_T2, num_cores):
+                     FA_method, FA_smooth, myelin_T2, num_cores, n_bootstrap=0, bootstrap_seed=0):
     """Same arguments as the reference.  `num_cores` selects the number of GPUs (-1 = all visible; see
-    n_gpus_from_num_cores): the masked voxels of the volume are spread over them by pipeline.MultiGpuFit."""
+    n_gpus_from_num_cores): the masked voxels of the volume are spread over them by pipeline.MultiGpuFit.
+
+    n_bootstrap > 0 (not in the reference): also the per-voxel bootstrap uncertainty of the six maps with that many
+    wild-bootstrap replicates per voxel (pipeline.recon_arrays), written as <MAP>_bootstrap.nii.gz (4 frames: mean,
+    sd, 2.5th and 97.5th percentile) and bootstrap_n_valid.nii.gz beside the ten outputs."""
     n_gpus = n_gpus_from_num_cores(num_cores)
     warm = threading.Thread(target=_warm_gpus, args=(n_gpus,), daemon=True)   # CUDA contexts + libmet2.so while the files load
     warm.start()
@@ -98,11 +103,12 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
     print('Step #3: Estimation of T2 spectra:')
     vol = pipeline.recon_arrays(data, mask, np.asarray(TE_array, dtype=np.float64), TR, reg_method, reg_matrix,
                                 FA_method, myelin_T2=myelin_T2, data_fa=data_fa, diagnostics=True, premasked=True,
-                                n_gpus=n_gpus)
+                                n_gpus=n_gpus, n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed)
     print('Step #4: Estimation of quantitative metrics')
     # the ten volumes (motor...:474-503) are written concurrently, largest first: every writer deflates with all cores
     # (nifti_io), but the eight 3-D maps are too small to keep them busy one at a time (2.2 s -> 1.2 s on 8 cores)
-    order = sorted(OUTPUTS, key=lambda name: -vol[name].size)
+    names = OUTPUTS + (BOOTSTRAP_OUTPUTS if n_bootstrap > 0 else ())
+    order = sorted(names, key=lambda name: -vol[name].size)
     with ThreadPoolExecutor(max_workers=4) as pool:
         list(pool.map(lambda name: nifti_io.save(vol[name], join(name + '.nii.gz'), affine=img.affine), order))
     dg = vol.get("diagnostics")

@@ -73,6 +73,19 @@ def chunk_deal(n_voxels, n_parts, chunks_per_part=4, align=64):
 
 
 OUT_KEYS = ("fa_index", "fa_deg", "km", "fa_status", "fsol", "est_signal", "reg", "maps", "status")
+BOOT_KEYS = ("boot_stats", "boot_n_valid")
+
+
+def bootstrap_fitted(plan, sig, fa_index, t2, n_bootstrap, seed, voxel_offset):
+    """`Met2Plan.bootstrap` of the voxels of one point fit (`t2`: the `t2_fit` result on sig[V, nTE] at fa_index[V]),
+    with voxel_offset = the position of sig[0] in the whole voxel list.  Voxels the point fit skipped get zeros, like
+    their maps.  Returns dict(boot_stats[V, 6, 4], boot_n_valid[V]) of CUDA tensors, enqueued on the current stream."""
+    stats, n_valid = plan.bootstrap(sig, fa_index, t2["est_signal"], B=n_bootstrap, seed=seed,
+                                    voxel_offset=voxel_offset)
+    skipped = (t2["status"] & batched.ST_SKIPPED) != 0
+    stats.masked_fill_(skipped[:, None, None], 0.0)
+    n_valid.masked_fill_(skipped, 0)
+    return dict(boot_stats=stats, boot_n_valid=n_valid)
 
 
 def host_buffers(plan, V, pinned=True):
@@ -116,9 +129,11 @@ class MultiGpuFit:
                                 range(n)))
         return cls(plans, chunks_per_device)
 
-    def fit(self, sig, sig_fa=None, out=None):
+    def fit(self, sig, sig_fa=None, out=None, n_bootstrap=0, bootstrap_seed=0):
         """sig[V, nTE] (+ sig_fa for the FA stage): host tensors / arrays, pinned for full-speed DMA.  `out`: dict of
         host tensors as from `host_buffers` (allocated if None).  Returns dict of numpy views of `out`.
+        n_bootstrap > 0: also the per-voxel bootstrap of the maps (`bootstrap_fitted`, keys BOOT_KEYS), each device
+        over its own chunks with voxel_offset = the chunk's start, so the result does not depend on the device count.
 
         Everything is ENQUEUED from this one thread, phase by phase over the devices (copies in, FA stage, T2 stage,
         copies out: ~0.1 ms of host time per device and phase, all asynchronous), then the streams are drained.  A
@@ -130,6 +145,10 @@ class MultiGpuFit:
         V = sig.shape[0]
         if out is None:
             out = host_buffers(self.plans[0], V)
+        if n_bootstrap > 0 and "boot_stats" not in out:
+            pin = torch.cuda.is_available()
+            out["boot_stats"] = torch.empty((V, 6, 4), dtype=torch.float64, pin_memory=pin)
+            out["boot_n_valid"] = torch.empty(V, dtype=torch.int32, pin_memory=pin)
         nd = len(self.plans)
         parts = chunk_deal(V, nd, self.chunks_per_device)
         trace = [dict() for _ in self.plans] if os.environ.get("MET2_MULTI_TRACE") else None
@@ -170,6 +189,19 @@ class MultiGpuFit:
             with torch.cuda.device(plan.dev), torch.cuda.stream(self.streams[d]):
                 b["t2"] = plan.t2_fit(b["sig"], b["fa"]["fa_index"], out=b["t2"])
             mark(d, "t2_enqueued")
+        boot = {}
+        if n_bootstrap > 0:
+            for d in live:                               # ---- phase 3b: bootstrap, chunk by chunk
+                plan, b = self.plans[d], bufs[d]
+                with torch.cuda.device(plan.dev), torch.cuda.stream(self.streams[d]):
+                    o, boot[d] = 0, []
+                    for lo, hi in parts[d]:
+                        rows = slice(o, o + hi - lo)
+                        t2 = {k: b["t2"][k][rows] for k in ("est_signal", "status")}
+                        boot[d].append(bootstrap_fitted(plan, b["sig"][rows], b["fa"]["fa_index"][rows], t2,
+                                                        n_bootstrap, bootstrap_seed, lo))
+                        o += hi - lo
+                mark(d, "bootstrap_enqueued")
         for d in live:                                   # ---- phase 4: device -> its rows of the host arrays
             plan, b = self.plans[d], bufs[d]
             fa, t2 = b["fa"], b["t2"]
@@ -178,9 +210,11 @@ class MultiGpuFit:
                            status=t2["status"])
             with torch.cuda.device(plan.dev), torch.cuda.stream(self.streams[d]):
                 o = 0
-                for lo, hi in parts[d]:
+                for i, (lo, hi) in enumerate(parts[d]):
                     for k in OUT_KEYS:
                         out[k][lo:hi].copy_(dev_out[k][o:o + hi - lo], non_blocking=True)
+                    for k in (BOOT_KEYS if n_bootstrap > 0 else ()):
+                        out[k][lo:hi].copy_(boot[d][i][k], non_blocking=True)
                     o += hi - lo
             mark(d, "d2h_enqueued")
         fs = torch.zeros(self.plans[0].npc, dtype=torch.float64)
@@ -194,11 +228,14 @@ class MultiGpuFit:
         return {k: (v.numpy() if k == "fsol_sum" else v[:V].numpy()) for k, v in out.items()}
 
 
-def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, fa_only=False):
+def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, fa_only=False, n_bootstrap=0,
+               bootstrap_seed=0, voxel_offset=0):
     """Steps 2-4 on a list of voxels given as host array sig[V, nTE]; returns host arrays (dict).
     in_mask[V] (optional): also return the mean-spectrum diagnostics of motor...:375-403 over the voxels with
     in_mask == 1 (key "diagnostics").  roi = (labels[V], values) (optional): also the ROI-based estimates of
-    motor_recon_met2_real_data_ROI.py:405-445 (key "roi")."""
+    motor_recon_met2_real_data_ROI.py:405-445 (key "roi").  n_bootstrap > 0: also the per-voxel bootstrap of the maps
+    with that many replicates (`bootstrap_fitted`, keys BOOT_KEYS); voxel_offset: the position of sig[0] in the whole
+    voxel list (a torchrun rank's slab start)."""
     dev = plan.dev
     V = sig.shape[0]
     with torch.cuda.device(dev):
@@ -215,6 +252,8 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
         if not fa_only:
             t2 = plan.t2_fit(d_sig, fa["fa_index"])
             out.update(fsol=t2["fsol"], est_signal=t2["est_signal"], reg=t2["reg"], maps=t2["maps"], status=t2["status"])
+            if n_bootstrap > 0:
+                out.update(bootstrap_fitted(plan, d_sig, fa["fa_index"], t2, n_bootstrap, bootstrap_seed, voxel_offset))
         extra = {}
         if in_mask is not None and V > 0:
             extra["diagnostics"] = mean_spectrum_diagnostics(plan, d_sig, fa["fa_index"], in_mask, fa["fsol_sum"])
@@ -235,8 +274,14 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
 
 def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, myelin_T2=40.0, data_fa=None, plan=None,
                  npc=None, n_alphas=None, device=None, rank=0, world_size=1, diagnostics=False, rois=None,
-                 premasked=False, fa_only=False, n_gpus=1):
+                 premasked=False, fa_only=False, n_gpus=1, n_bootstrap=0, bootstrap_seed=0):
     """Steps 2-4 of motor_recon_met2 on in-memory arrays.  Returns the ten output volumes (plus FA_index) as numpy.
+
+    n_bootstrap > 0: also the per-voxel bootstrap uncertainty of the six maps with that many replicates per voxel
+    (`batched.Met2Plan.bootstrap`): volumes "<MAP>_bootstrap" [nx, ny, nz, 4] (mean, sd, p2.5, p97.5) and
+    "bootstrap_n_valid" [nx, ny, nz]; voxels outside the mask or skipped by the fit are zero.  Replicates are keyed on
+    the voxel's position in the masked-voxel list and on bootstrap_seed, so the volumes are the same for any number of
+    GPUs or ranks.
 
     n_gpus != 1 (None / -1 = all visible GPUs): the voxel list of this ONE volume is spread over the GPUs of the node by
     `MultiGpuFit` (host in -> host out, no collective).  With world_size > 1 (one process per GPU under torchrun) only
@@ -289,7 +334,7 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
         if sig_fa is not None:
             pin_fa = torch.empty((V, nt), dtype=torch.float64).pin_memory()
             pin_fa.copy_(sig_fa if isinstance(sig_fa, torch.Tensor) else torch.as_tensor(sig_fa))
-        res = multi.fit(pin, pin_fa)
+        res = multi.fit(pin, pin_fa, n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed)
         if (in_mask is not None or roi is not None) and V > 0:
             # whole-volume reductions (a few ms): on the first device, from the gathered FA indices
             with torch.cuda.device(plan.dev):
@@ -300,7 +345,8 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
                 if roi is not None:
                     res["roi"] = roi_estimates(plan, d_sig, d_idx, roi[0], roi[1])
     else:
-        res = fit_voxels(plan, sig[lo:hi], sig_fa, in_mask=in_mask, roi=roi, fa_only=fa_only)
+        res = fit_voxels(plan, sig[lo:hi], sig_fa, in_mask=in_mask, roi=roi, fa_only=fa_only,
+                         n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed, voxel_offset=lo)
     sel = flat[lo:hi]
     nvox = nx * ny * nz
     vol = {}
@@ -331,6 +377,14 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
     vol["status"] = np.zeros(nvox, dtype=np.int32)
     vol["status"][sel] = res["status"]
     vol["status"] = vol["status"].reshape(nx, ny, nz)
+    if n_bootstrap > 0:
+        for i, name in enumerate(MAP_NAMES):
+            a = np.zeros((nvox, 4))
+            a[sel] = res["boot_stats"][:, i, :]
+            vol[name + "_bootstrap"] = a.reshape(nx, ny, nz, 4)
+        a = np.zeros(nvox, dtype=np.int32)
+        a[sel] = res["boot_n_valid"]
+        vol["bootstrap_n_valid"] = a.reshape(nx, ny, nz)
     return vol
 
 
