@@ -239,6 +239,28 @@ int met2_boot_resample(const double* sig, const double* est_signal, const int32_
 int met2_boot_summary(const double* rep_maps, const uint32_t* rep_status, int64_t V, int B, double* stats,
                       int32_t* n_valid, void* stream);
 
+/* Spatially regularised spectrum fitting (no counterpart in the reference; the reference's unused prior-spectrum
+ * argument points the same way).  Definition in csrc/met2_spatial.cu; the NumPy restatement is tests/spatial_oracle.py.
+ * Normalised units: x [V][nT2] holds fsol / sig[0] of the point fit (met2_t2_fit) and is updated in place.
+ *
+ * met2_spatial_sweep: one half-sweep of red-black block updates, for the voxels vox [Vc] (positions in 0..V-1, all of
+ * one colour): x_v <- argmin_{x >= 0} ||D_a x - y_v||^2 + lam_v ||L x||^2 + mu n_v ||x - p_v||^2, with y_v = sig_v /
+ * sig_v[0], a = fa_index[v], p_v the mean of the rows x_q of its n_v neighbours q = nbr[v][0..6) (int32, -1 = none).
+ * lam [V] is the point fit's lambda (reg under MET2_T2_FLAG_REG_IS_LAMBDA); G, dicT, kband as for met2_t2_fit.
+ * status [V]: voxels with MET2_ST_SKIPPED are left alone; a solve that hits itmax ORs MET2_ST_ITMAX.
+ *
+ * met2_spatial_finish: fsol = x sig[0], est_signal = D_a x sig[0] and maps [V][6] as met2_t2_fit computes them; voxels
+ * with MET2_ST_SKIPPED in status get met2_t2_fit's outputs for a skipped voxel.
+ *
+ * Both: gram-domain sizes of met2_t2_fit (nT2 <= 128, nTE <= 64), V < 2^31; mu must be finite and >= 0; V (or Vc) = 0
+ * is a no-op; bad arguments return MET2_ERR_ARG before anything is enqueued. */
+int met2_spatial_sweep(const double* sig, const int32_t* fa_index, const double* lam, const int32_t* nbr,
+                       const int32_t* vox, int64_t Vc, int64_t V, int nTE, int nT2, int nA, const double* G,
+                       const double* dicT, const double* kband, double mu, double* x, uint32_t* status, void* stream);
+int met2_spatial_finish(const double* sig, const int32_t* fa_index, const uint32_t* status, const double* x,
+                        int64_t V, int nTE, int nT2, int nA, const double* dicT, const double* logT2,
+                        const uint8_t* comp, double* fsol, double* est_signal, double* maps, void* stream);
+
 /* Diagnostics */
 const char* met2_last_error(void);
 int met2_version(void);

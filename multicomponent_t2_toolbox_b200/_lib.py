@@ -57,6 +57,11 @@ SIGNATURES = {
                                           ctypes.c_uint64, ctypes.c_int64, c_void_p, c_void_p, c_void_p]),
     "met2_boot_summary": (ctypes.c_int, [c_void_p, c_void_p, ctypes.c_int64, ctypes.c_int, c_void_p, c_void_p,
                                          c_void_p]),
+    "met2_spatial_sweep": (ctypes.c_int, [c_void_p] * 5 + [ctypes.c_int64, ctypes.c_int64, ctypes.c_int, ctypes.c_int,
+                                                          ctypes.c_int, c_void_p, c_void_p, c_void_p, ctypes.c_double,
+                                                          c_void_p, c_void_p, c_void_p]),
+    "met2_spatial_finish": (ctypes.c_int, [c_void_p] * 4 + [ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int]
+                            + [c_void_p] * 7),
     "met2_last_error": (ctypes.c_char_p, []),
     "met2_version": (ctypes.c_int, []),
     "met2_echo_rank": (ctypes.c_int, [ctypes.c_int]),

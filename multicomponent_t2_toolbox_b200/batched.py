@@ -487,6 +487,80 @@ class Met2Plan:
         t2 = self.t2_fit(sig, fa["fa_index"])
         return fa, t2
 
+    # ------------------------------------------------------------------ spatially regularised fit
+    def spatial_half_sweep(self, sig, fa_index, lam, x, nbr, vox, mu, status):
+        """One half-sweep of met2_spatial_sweep: block updates of the voxels `vox` (all of one colour) of the
+        normalised spectra x[V, nT2] (CUDA float64, updated in place); status[V] (CUDA int32) gets MET2_ST_ITMAX where a
+        solve hit itmax.  sig[V, nTE], fa_index[V], lam[V] and nbr[V, 6] as for `spatial_fit`, already on this device."""
+        V = sig.shape[0]
+        hr = self.dict_hr
+        with torch.cuda.device(self.dev):
+            _lib.check(self.lib.met2_spatial_sweep(
+                _ptr(sig), _ptr(fa_index), _ptr(lam), _ptr(nbr), _ptr(vox), vox.numel(), V, self.nTE, self.npc, hr.nA,
+                _ptr(hr.G), _ptr(hr.dicT), _ptr(self.kband), float(mu), _ptr(x), _ptr(status), _stream()),
+                "met2_spatial_sweep")
+
+    def spatial_fit(self, sig, fa_index, lam, fsol, nbr, colours, mu, n_sweeps=10, status=None):
+        """Spatially regularised spectra (definition in csrc/met2_spatial.cu): n_sweeps red-black sweeps of
+        neighbour-coupled block updates with coupling weight mu >= 0, started from a point fit of this plan.
+
+        sig[V, nTE] is the signal the point fit used, fa_index[V] its flip-angle indices, lam[V] the lambda it selected
+        (`t2_fit(..., flags=REG_IS_LAMBDA)["reg"]`), fsol[V, nT2] its spectra and status[V] its status (None: the
+        voxels in neither colour list count as skipped).  nbr[V, 6] and colours come from
+        `pipeline.spatial_neighbours`.  The sweeps solve in the Gram domain, whichever kernels the point fit ran.
+        Returns CUDA tensors fsol[V, nT2], est_signal[V, nTE], maps[V, 6], status[V] (the point fit's, with
+        MET2_ST_ITMAX added where a sweep solve hit itmax) and x[V, nT2] = fsol / sig[0].  All work is enqueued on the
+        current stream."""
+        mu, n_sweeps = float(mu), int(n_sweeps)
+        if not (math.isfinite(mu) and mu >= 0.0):
+            raise ValueError("mu must be finite and >= 0, got %r" % mu)
+        if n_sweeps < 0:
+            raise ValueError("n_sweeps must be >= 0")
+        sig = self._signals(sig)
+        V = sig.shape[0]
+        dev = self.dev
+        i32 = lambda a: torch.as_tensor(a).to(device=dev, dtype=torch.int32).contiguous()
+        fa_index, nbr = i32(fa_index), i32(nbr)
+        colours = [i32(c).reshape(-1) for c in colours]
+        lam = torch.as_tensor(lam).to(device=dev, dtype=torch.float64).contiguous()
+        fsol = torch.as_tensor(fsol).to(device=dev, dtype=torch.float64)
+        if (fa_index.shape != (V,) or lam.shape != (V,) or tuple(fsol.shape) != (V, self.npc)
+                or tuple(nbr.shape) != (V, 6) or len(colours) != 2):
+            raise ValueError("spatial_fit: sig[V, nTE], fa_index[V], lam[V], fsol[V, nT2], nbr[V, 6] and two colour "
+                             "lists expected")
+        for c in colours:
+            if c.numel() and (int(c.min()) < 0 or int(c.max()) >= V):
+                raise ValueError("spatial_fit: colour lists hold positions in [0, V)")
+        if nbr.numel() and (int(nbr.min()) < -1 or int(nbr.max()) >= V):
+            raise ValueError("spatial_fit: nbr holds positions in [0, V) or -1")
+        if status is None:
+            status = torch.full((V,), ST_SKIPPED, dtype=torch.int32, device=dev)
+            for c in colours:
+                status[c.long()] = 0
+        else:
+            status = i32(status).clone()
+            if status.shape != (V,):
+                raise ValueError("status must be [V]")
+        out = dict(fsol=torch.empty((V, self.npc), dtype=torch.float64, device=dev),
+                   est_signal=torch.empty((V, self.nTE), dtype=torch.float64, device=dev),
+                   maps=torch.empty((V, 6), dtype=torch.float64, device=dev), status=status)
+        if V == 0:
+            out["x"] = torch.empty((0, self.npc), dtype=torch.float64, device=dev)
+            return out
+        with torch.cuda.device(dev):
+            fitted = (status & ST_SKIPPED) == 0
+            x = torch.where(fitted[:, None], fsol / sig[:, :1], 0.0).contiguous()
+            for _ in range(n_sweeps):
+                for vox in colours:
+                    self.spatial_half_sweep(sig, fa_index, lam, x, nbr, vox, mu, status)
+            hr = self.dict_hr
+            _lib.check(self.lib.met2_spatial_finish(
+                _ptr(sig), _ptr(fa_index), _ptr(status), _ptr(x), V, self.nTE, self.npc, hr.nA, _ptr(hr.dicT),
+                _ptr(self.logT2), _ptr(self.comp), _ptr(out["fsol"]), _ptr(out["est_signal"]), _ptr(out["maps"]),
+                _stream()), "met2_spatial_finish")
+        out["x"] = x
+        return out
+
     # ------------------------------------------------------------------ bootstrap uncertainty of the maps
     def bootstrap(self, sig, fa_index, est_signal, B=100, seed=0, voxel_offset=0, max_replicates=1 << 21):
         """Per-voxel wild-bootstrap uncertainty of the six maps (definition in csrc/met2_boot.cu).

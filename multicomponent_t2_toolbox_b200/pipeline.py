@@ -76,6 +76,43 @@ OUT_KEYS = ("fa_index", "fa_deg", "km", "fa_status", "fsol", "est_signal", "reg"
 BOOT_KEYS = ("boot_stats", "boot_n_valid")
 
 
+def spatial_neighbours(flat, shape, fitted):
+    """Neighbour table and red-black colours of the spatially regularised fit (`batched.Met2Plan.spatial_fit`).
+    flat[V]: C-order indices of the masked voxels in a volume of `shape` (nx, ny, nz), as `masked_voxel_list` returns
+    them; fitted[V]: the voxels the point fit did not skip.  Returns nbr int32 [V, 6] (positions in 0..V-1 of the
+    fitted face neighbours in the order -x, +x, -y, +y, -z, +z; -1 = none, and all -1 for a voxel that is not fitted)
+    and the two colour lists (positions of the fitted voxels with (i + j + k) % 2 == 0 and == 1, ascending)."""
+    nx, ny, nz = (int(s) for s in shape)
+    flat = np.asarray(flat, dtype=np.int64)
+    fitted = np.asarray(fitted, dtype=bool)
+    where = np.full(nx * ny * nz, -1, dtype=np.int64)
+    where[flat[fitted]] = np.nonzero(fitted)[0]
+    i, j, k = np.unravel_index(flat, (nx, ny, nz))
+    nbr = np.full((len(flat), 6), -1, dtype=np.int32)
+    for f, (di, dj, dk) in enumerate(((-1, 0, 0), (1, 0, 0), (0, -1, 0), (0, 1, 0), (0, 0, -1), (0, 0, 1))):
+        a, b, c = i + di, j + dj, k + dk
+        inside = fitted & (a >= 0) & (a < nx) & (b >= 0) & (b < ny) & (c >= 0) & (c < nz)
+        nbr[inside, f] = where[(a[inside] * ny + b[inside]) * nz + c[inside]]
+    colour = (i + j + k) % 2
+    colours = tuple(np.nonzero(fitted & (colour == c))[0].astype(np.int32) for c in (0, 1))
+    return nbr, colours
+
+
+SPATIAL_KEYS = ("fsol", "est_signal", "maps", "status")
+
+
+def spatial_fitted(plan, sig, fa_index, t2, flat, shape, mu, n_sweeps):
+    """`Met2Plan.spatial_fit` after the point fit `t2` (the `t2_fit` result on sig[V, nTE] at fa_index[V], CUDA) of the
+    masked voxels flat[V] of a volume of `shape`: lambda_v from a second `t2_fit` with MET2_T2_FLAG_REG_IS_LAMBDA, the
+    neighbour table of the fitted voxels (`spatial_neighbours`; reads the point fit's status back to the host), then the
+    sweeps.  Returns dict(fsol, est_signal, maps, status) of CUDA tensors; reg stays the point fit's."""
+    lam = plan.t2_fit(sig, fa_index, flags=batched.REG_IS_LAMBDA)["reg"]
+    fitted = ((t2["status"] & batched.ST_SKIPPED) == 0).cpu().numpy()
+    nbr, colours = spatial_neighbours(flat, shape, fitted)
+    sp = plan.spatial_fit(sig, fa_index, lam, t2["fsol"], nbr, colours, mu, n_sweeps, status=t2["status"])
+    return {k: sp[k] for k in SPATIAL_KEYS}
+
+
 def bootstrap_fitted(plan, sig, fa_index, t2, n_bootstrap, seed, voxel_offset):
     """`Met2Plan.bootstrap` of the voxels of one point fit (`t2`: the `t2_fit` result on sig[V, nTE] at fa_index[V]),
     with voxel_offset = the position of sig[0] in the whole voxel list.  Voxels the point fit skipped get zeros, like
@@ -229,13 +266,15 @@ class MultiGpuFit:
 
 
 def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, fa_only=False, n_bootstrap=0,
-               bootstrap_seed=0, voxel_offset=0):
+               bootstrap_seed=0, voxel_offset=0, spatial=None):
     """Steps 2-4 on a list of voxels given as host array sig[V, nTE]; returns host arrays (dict).
     in_mask[V] (optional): also return the mean-spectrum diagnostics of motor...:375-403 over the voxels with
     in_mask == 1 (key "diagnostics").  roi = (labels[V], values) (optional): also the ROI-based estimates of
     motor_recon_met2_real_data_ROI.py:405-445 (key "roi").  n_bootstrap > 0: also the per-voxel bootstrap of the maps
     with that many replicates (`bootstrap_fitted`, keys BOOT_KEYS); voxel_offset: the position of sig[0] in the whole
-    voxel list (a torchrun rank's slab start)."""
+    voxel list (a torchrun rank's slab start).  spatial = (flat, shape, mu, n_sweeps) (optional): the voxels are the
+    masked voxels flat[V] of a volume of `shape`, and fsol / est_signal / maps / status are those of the spatially
+    regularised fit with coupling weight mu (`spatial_fitted`)."""
     dev = plan.dev
     V = sig.shape[0]
     with torch.cuda.device(dev):
@@ -252,6 +291,8 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
         if not fa_only:
             t2 = plan.t2_fit(d_sig, fa["fa_index"])
             out.update(fsol=t2["fsol"], est_signal=t2["est_signal"], reg=t2["reg"], maps=t2["maps"], status=t2["status"])
+            if spatial is not None:
+                out.update(spatial_fitted(plan, d_sig, fa["fa_index"], t2, *spatial))
             if n_bootstrap > 0:
                 out.update(bootstrap_fitted(plan, d_sig, fa["fa_index"], t2, n_bootstrap, bootstrap_seed, voxel_offset))
         extra = {}
@@ -274,7 +315,8 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
 
 def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, myelin_T2=40.0, data_fa=None, plan=None,
                  npc=None, n_alphas=None, device=None, rank=0, world_size=1, diagnostics=False, rois=None,
-                 premasked=False, fa_only=False, n_gpus=1, n_bootstrap=0, bootstrap_seed=0):
+                 premasked=False, fa_only=False, n_gpus=1, n_bootstrap=0, bootstrap_seed=0, spatial_mu=0.0,
+                 spatial_sweeps=10):
     """Steps 2-4 of motor_recon_met2 on in-memory arrays.  Returns the ten output volumes (plus FA_index) as numpy.
 
     n_bootstrap > 0: also the per-voxel bootstrap uncertainty of the six maps with that many replicates per voxel
@@ -283,12 +325,25 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
     the voxel's position in the masked-voxel list and on bootstrap_seed, so the volumes are the same for any number of
     GPUs or ranks.
 
+    spatial_mu > 0: the maps, fsol_4D, Est_Signal and status are those of the spatially regularised fit
+    (`batched.Met2Plan.spatial_fit`, definition in csrc/met2_spatial.cu): spatial_sweeps red-black sweeps that couple
+    each fitted voxel's spectrum to its fitted face neighbours with weight spatial_mu, started from the point fit; FA
+    and reg_param stay the point fit's.  With several GPUs the point fit is spread over them and the sweeps run on the
+    first.  It needs the whole volume in one process (world_size 1) and cannot be combined with n_bootstrap.
+
     n_gpus != 1 (None / -1 = all visible GPUs): the voxel list of this ONE volume is spread over the GPUs of the node by
     `MultiGpuFit` (host in -> host out, no collective).  With world_size > 1 (one process per GPU under torchrun) only
     this rank's slab of the masked voxels is fitted and the other voxels are left zero; the caller combines the ranks
     (`gather_slabs`).  fa_only: stop after the flip-angle stage (the ROI-based estimator never fits voxel spectra,
     motor_recon_met2_real_data_ROI.py:349-445): the spectrum volumes are not produced.
     """
+    spatial_mu = float(spatial_mu)
+    if not (np.isfinite(spatial_mu) and spatial_mu >= 0.0):
+        raise ValueError("spatial_mu must be finite and >= 0")
+    if spatial_mu > 0 and world_size != 1:
+        raise ValueError("the spatially regularised fit couples neighbouring voxels: run it unsharded")
+    if spatial_mu > 0 and n_bootstrap > 0:
+        raise ValueError("spatial_mu > 0 cannot be combined with n_bootstrap")
     data = np.asarray(data, dtype=np.float64)
     nx, ny, nz, nt = data.shape
     TE_array = np.asarray(TE_array, dtype=np.float64)
@@ -344,9 +399,19 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
                     res["diagnostics"] = mean_spectrum_diagnostics(plan, d_sig, d_idx, in_mask, res["fsol_sum"])
                 if roi is not None:
                     res["roi"] = roi_estimates(plan, d_sig, d_idx, roi[0], roi[1])
+        if spatial_mu > 0 and V > 0:
+            # the sweeps couple voxels of every device's chunks: on the first device, from the gathered point fit
+            with torch.cuda.device(plan.dev):
+                d_sig = pin.to(plan.dev, non_blocking=True)
+                d_idx = torch.as_tensor(res["fa_index"]).to(plan.dev)
+                t2 = dict(fsol=torch.as_tensor(res["fsol"]).to(plan.dev),
+                          status=torch.as_tensor(res["status"]).to(plan.dev))
+                sp = spatial_fitted(plan, d_sig, d_idx, t2, flat, (nx, ny, nz), spatial_mu, spatial_sweeps)
+                res.update({k: v.cpu().numpy() for k, v in sp.items()})
     else:
+        spatial = (flat, (nx, ny, nz), spatial_mu, spatial_sweeps) if spatial_mu > 0 and not fa_only else None
         res = fit_voxels(plan, sig[lo:hi], sig_fa, in_mask=in_mask, roi=roi, fa_only=fa_only,
-                         n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed, voxel_offset=lo)
+                         n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed, voxel_offset=lo, spatial=spatial)
     sel = flat[lo:hi]
     nvox = nx * ny * nz
     vol = {}
