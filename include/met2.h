@@ -51,6 +51,7 @@ extern "C" {
 #define MET2_ST_SSE_ZERO 8u     /* X2: plain-NNLS residual is exactly 0 -> NaN objective (algorithms.py:231) */
 #define MET2_ST_ECHO_BAD_L 32u  /* MET2_T2_FLAG_ECHO_SPACE given with a non-diagonal L: voxel skipped */
 #define MET2_ST_NOT_PD 16u      /* BayesReg: beta*B + beta*x*K not positive definite (reference: LinAlgError) */
+#define MET2_ST_AT_BOUND 64u    /* met2_param_fit: a fitted T2 or the flip angle ends on its box (informational) */
 
 /* flip-angle search methods: run_real_data_script.py --FA_method */
 #define MET2_FA_BRUTE_FORCE 0
@@ -260,6 +261,30 @@ int met2_spatial_sweep(const double* sig, const int32_t* fa_index, const double*
 int met2_spatial_finish(const double* sig, const int32_t* fa_index, const uint32_t* status, const double* x,
                         int64_t V, int nTE, int nT2, int nA, const double* dicT, const double* logT2,
                         const uint8_t* comp, double* fsol, double* est_signal, double* maps, void* stream);
+
+/* Three-pool parametric T2 fit (no counterpart in the reference): bounded Levenberg-Marquardt over the amplitudes and
+ * continuous T2s of a myelin, an intra/extra-cellular and a free-water pool, each an EPG decay curve of the dictionary's
+ * recurrence, sharing one continuous refocusing angle.  Definition and defaults in csrc/met2_param.cu; the NumPy
+ * restatement is tests/param_oracle.py.
+ * Inputs are the point fit's: sig [V][nTE] raw signals, fa_deg [V] (met2_fa_fit), fsol [V][nT2] and status [V]
+ * (met2_t2_fit); logT2 [nT2] and comp [nT2] as for met2_t2_fit.  Voxels with MET2_ST_SKIPPED or MET2_ST_NONFINITE get
+ * all-zero outputs.  Outputs: params [V][7] = the three amplitudes (raw units), the three T2s (ms) and the flip angle
+ * (deg); maps [V][6] as met2_t2_fit's columns; est_signal [V][nTE]; sse [V]; iters [V] int32; status [V].
+ * V = 0 is a no-op; bad arguments (sizes, NULL pointers, an empty box, V >= 2^31) return MET2_ERR_ARG before anything
+ * is enqueued. */
+typedef struct met2_param_cfg {
+    int32_t nTE, nT2;
+    int32_t max_iter;         /* Levenberg-Marquardt iterations (2000); MET2_ST_ITMAX when reached */
+    int32_t reserved;
+    double tau, TR, T1;       /* ms: echo spacing, repetition time, T1 of the dictionary */
+    double t2_lo[3], t2_hi[3];/* ms: T2 box of the myelin, intra/extra-cellular and free-water pools */
+    double fa_lo, fa_hi;      /* deg: flip-angle box (90, 180) */
+    double mu0, mu_max;       /* initial damping (1e-3) and the cap that stops the iteration (1e16) */
+    double ftol, xtol;        /* relative decrease of the cost (1e-12), scaled step (1e-10) */
+} met2_param_cfg;
+int met2_param_fit(const double* sig, const double* fa_deg, const double* fsol, const uint32_t* status_in, int64_t V,
+                   const met2_param_cfg* cfg, const double* logT2, const uint8_t* comp, double* params, double* maps,
+                   double* est_signal, double* sse, int32_t* iters, uint32_t* status, void* stream);
 
 /* Diagnostics */
 const char* met2_last_error(void);

@@ -25,6 +25,14 @@ class T2Cfg(ctypes.Structure):
                 ("log_det_L", ctypes.c_double), ("flags", ctypes.c_int32), ("echo_rank", ctypes.c_int32)]
 
 
+class ParamCfg(ctypes.Structure):
+    _fields_ = [("nTE", ctypes.c_int32), ("nT2", ctypes.c_int32), ("max_iter", ctypes.c_int32),
+                ("reserved", ctypes.c_int32), ("tau", ctypes.c_double), ("TR", ctypes.c_double), ("T1", ctypes.c_double),
+                ("t2_lo", ctypes.c_double * 3), ("t2_hi", ctypes.c_double * 3), ("fa_lo", ctypes.c_double),
+                ("fa_hi", ctypes.c_double), ("mu0", ctypes.c_double), ("mu_max", ctypes.c_double),
+                ("ftol", ctypes.c_double), ("xtol", ctypes.c_double)]
+
+
 # every symbol include/met2.h declares, with its ctypes signature
 SIGNATURES = {
     "met2_epg_dictionary": (ctypes.c_int, [c_void_p, ctypes.c_int, c_void_p, c_void_p, ctypes.c_int, ctypes.c_int,
@@ -62,6 +70,7 @@ SIGNATURES = {
                                                           c_void_p, c_void_p, c_void_p]),
     "met2_spatial_finish": (ctypes.c_int, [c_void_p] * 4 + [ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int]
                             + [c_void_p] * 7),
+    "met2_param_fit": (ctypes.c_int, [c_void_p] * 4 + [ctypes.c_int64, ctypes.POINTER(ParamCfg)] + [c_void_p] * 9),
     "met2_last_error": (ctypes.c_char_p, []),
     "met2_version": (ctypes.c_int, []),
     "met2_echo_rank": (ctypes.c_int, [ctypes.c_int]),

@@ -20,6 +20,9 @@ FA_METHOD_CODE = {"brute-force": 0, "spline": 1}
 REG_METHOD_CODE = {"NNLS": 0, "T2SPARC": 1, "X2": 2, "L_curve": 3, "GCV": 4, "BayesReg": 5}
 
 ST_SKIPPED, ST_NONFINITE, ST_ITMAX, ST_SSE_ZERO, ST_NOT_PD = 1, 2, 4, 8, 16
+ST_AT_BOUND = 64
+# Levenberg-Marquardt settings of the three-pool parametric fit (csrc/met2_param.cu)
+PARAM_DEFAULTS = dict(mu0=1e-3, mu_max=1e16, ftol=1e-12, xtol=1e-10, max_iter=2000)
 REG_IS_LAMBDA, NO_NORMALISE, COLD_START, GCV_EVAL, FULL_START, GCV_GRID, ECHO_SPACE = 1, 2, 4, 8, 16, 32, 64   # MET2_T2_FLAG_*
 # Largest residual of the reduction (max_j |d_j - U C_j| / max_j |d_j| over the flip angles, measured by
 # met2_echo_basis) for which a rank of the reduced echo space is used.  24 (MET2_ECHO_RANK): the rounding of the
@@ -307,6 +310,7 @@ class Met2Plan:
         self.npc = grids.default_npc(reg_method) if npc is None else int(npc)
         self.T2s = grids.t2_grid(self.npc) if T2s is None else np.asarray(T2s, dtype=np.float64)
         self.T1s = float(T1) * np.ones_like(self.T2s)
+        self.myelin_T2 = float(myelin_T2)
         self.ind_m, self.ind_t, self.ind_csf = grids.compartment_masks(self.T2s, myelin_T2)
         self.alpha_values, self.alpha_spline = grids.fa_grids(FA_method, n_alphas)
         if Dic_3D is not None:
@@ -559,6 +563,52 @@ class Met2Plan:
                 _ptr(self.logT2), _ptr(self.comp), _ptr(out["fsol"]), _ptr(out["est_signal"]), _ptr(out["maps"]),
                 _stream()), "met2_spatial_finish")
         out["x"] = x
+        return out
+
+    # ------------------------------------------------------------------ three-pool parametric fit
+    def param_cfg(self, **overrides):
+        """met2_param_cfg of this plan: T2 boxes T2s[0]..myelin_T2, myelin_T2..200, 200..T2s[-1] (motor...:215-220),
+        flip angle 90..180, the plan's tau / TR / T1, and PARAM_DEFAULTS unless overridden."""
+        unknown = set(overrides) - set(PARAM_DEFAULTS)
+        if unknown:
+            raise ValueError("unknown param_fit settings %s" % sorted(unknown))
+        o = {**PARAM_DEFAULTS, **overrides}
+        T2s = self.T2s
+        return _lib.ParamCfg(nTE=self.nTE, nT2=self.npc, max_iter=int(o["max_iter"]), reserved=0, tau=self.tau,
+                             TR=self.TR, T1=float(self.T1s[0]),
+                             t2_lo=(ctypes.c_double * 3)(T2s[0], self.myelin_T2, 200.0),
+                             t2_hi=(ctypes.c_double * 3)(self.myelin_T2, 200.0, T2s[-1]), fa_lo=90.0, fa_hi=180.0,
+                             mu0=float(o["mu0"]), mu_max=float(o["mu_max"]), ftol=float(o["ftol"]),
+                             xtol=float(o["xtol"]))
+
+    def param_fit(self, sig, fa_deg, fsol, status, **cfg):
+        """Three-pool parametric fit (definition in csrc/met2_param.cu): bounded Levenberg-Marquardt over the
+        amplitudes and continuous T2s of a myelin, an intra/extra-cellular and a free-water EPG pool with one shared
+        continuous flip angle, started from a point fit of this plan.  sig[V, nTE] is the signal the point fit used,
+        fa_deg[V] the FA stage's angles, fsol[V, nT2] and status[V] the `t2_fit` results; cfg overrides
+        PARAM_DEFAULTS.  Returns CUDA tensors params[V, 7] (amplitudes in signal units, T2_m, T2_ie, T2_fw in ms,
+        flip angle in deg), maps[V, 6] (met2_t2_fit's columns), est_signal[V, nTE], sse[V], iters[V] (int32) and
+        status[V] (int32).  Voxels the point fit skipped get zeros.  All work is enqueued on the current stream."""
+        c = self.param_cfg(**cfg)
+        sig = self._signals(sig)
+        V = sig.shape[0]
+        dev = self.dev
+        fa_deg = torch.as_tensor(fa_deg).to(device=dev, dtype=torch.float64).contiguous()
+        fsol = torch.as_tensor(fsol).to(device=dev, dtype=torch.float64).contiguous()
+        status = torch.as_tensor(status).to(device=dev, dtype=torch.int32).contiguous()
+        if fa_deg.shape != (V,) or tuple(fsol.shape) != (V, self.npc) or status.shape != (V,):
+            raise ValueError("param_fit: sig[V, nTE], fa_deg[V], fsol[V, nT2] and status[V] expected")
+        out = dict(params=torch.empty((V, 7), dtype=torch.float64, device=dev),
+                   maps=torch.empty((V, 6), dtype=torch.float64, device=dev),
+                   est_signal=torch.empty((V, self.nTE), dtype=torch.float64, device=dev),
+                   sse=torch.empty(V, dtype=torch.float64, device=dev),
+                   iters=torch.empty(V, dtype=torch.int32, device=dev),
+                   status=torch.empty(V, dtype=torch.int32, device=dev))
+        with torch.cuda.device(dev):
+            _lib.check(self.lib.met2_param_fit(
+                _ptr(sig), _ptr(fa_deg), _ptr(fsol), _ptr(status), V, ctypes.byref(c), _ptr(self.logT2),
+                _ptr(self.comp), _ptr(out["params"]), _ptr(out["maps"]), _ptr(out["est_signal"]), _ptr(out["sse"]),
+                _ptr(out["iters"]), _ptr(out["status"]), _stream()), "met2_param_fit")
         return out
 
     # ------------------------------------------------------------------ bootstrap uncertainty of the maps

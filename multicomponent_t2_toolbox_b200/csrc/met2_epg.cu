@@ -4,24 +4,19 @@
 // dense (3n+1)^2 matrices S (shift), R (relaxation over tau/2), T (RF) and iterates x <- (R S) T (R S) x per echo
 // (epg.py:89-91,143-153).  Here one thread owns one (flip angle, T2) pair and applies the same operator sequence
 // directly to the banded state (F0; F+k, F-k, Zk, k = 1..n): shift, relax, RF, shift, relax; O(n^2) instead of O(n^3).
+// The coefficients and block operators are those of met2_epg.cuh, shared with the parametric fit (met2_param.cu).
 #include "met2_host.h"
+#include "met2_epg.cuh"
 
 namespace met2 {
 
 __device__ __forceinline__ void epg_decay(double alpha_deg, double T2, double T1, int n, double tau, double scale,
                                           double* out, int out_stride) {
-    const double rad = 3.14159265358979323846 / 180.0;
-    const double a = alpha_deg * rad;
-    const double a_exc = (alpha_deg / 2.0) * rad;   // epg.py:57: excitation = alpha/2
-    const double half = tau / 2.0;
-    const double e2 = exp(-half * (1.0 / T2));
-    const double e1 = exp(-half * (1.0 / T1));
-    const double ch = cos(a / 2.0), sh = sin(a / 2.0);
-    const double c2 = ch * ch, s2 = sh * sh, sa = sin(a), ca = cos(a);
+    const EpgCoef<double> c = epg_coef(alpha_deg, T2, T1, tau);
     double Fp[MET2_MAX_NTE + 2], Fm[MET2_MAX_NTE + 2], Z[MET2_MAX_NTE + 2];
     for (int k = 0; k < n + 2; ++k) Fp[k] = Fm[k] = Z[k] = 0.0;
-    double F0 = sin(a_exc);      // epg.py:145
-    Fm[1] = cos(a_exc);          // epg.py:147 (index 2 of the state vector is the F-1 slot)
+    double F0 = c.f0;
+    Fm[1] = c.fm1;
     for (int echo = 0; echo < n; ++echo) {
         for (int half_step = 0; half_step < 2; ++half_step) {
             // shift (epg.py:97-116): F0 <- F-1, F+1 <- F0, F+k <- F+(k-1), F-k <- F-(k+1), F-n <- 0
@@ -30,22 +25,10 @@ __device__ __forceinline__ void epg_decay(double alpha_deg, double T2, double T1
             Fp[1] = F0;
             for (int k = 1; k < n; ++k) Fm[k] = Fm[k + 1];
             Fm[n] = 0.0;
-            // relaxation over tau/2 (epg.py:82-85,133-141)
-            F0 = newF0 * e2;
-            for (int k = 1; k <= n; ++k) {
-                Fp[k] *= e2;
-                Fm[k] *= e2;
-                Z[k] *= e1;
-            }
-            if (half_step == 0) {
-                // RF mixing of every (F+k, F-k, Zk) block; F0 is not mixed (epg.py:118-131)
-                for (int k = 1; k <= n; ++k) {
-                    double fp = Fp[k], fm = Fm[k], z = Z[k];
-                    Fp[k] = c2 * fp + s2 * fm + sa * z;
-                    Fm[k] = s2 * fp + c2 * fm - sa * z;
-                    Z[k] = -0.5 * sa * fp + 0.5 * sa * fm + ca * z;
-                }
-            }
+            F0 = newF0 * c.e2;
+            for (int k = 1; k <= n; ++k) epg_relax(Fp[k], Fm[k], Z[k], c);
+            if (half_step == 0)
+                for (int k = 1; k <= n; ++k) epg_rf(Fp[k], Fm[k], Z[k], c);
         }
         out[(size_t)echo * out_stride] = scale * F0;
     }

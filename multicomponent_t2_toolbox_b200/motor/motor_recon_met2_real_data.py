@@ -63,7 +63,7 @@ def _warm_gpus(n_gpus):
 
 def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR, reg_method, reg_matrix, denoise,
                      FA_method, FA_smooth, myelin_T2, num_cores, n_bootstrap=0, bootstrap_seed=0, spatial_mu=0.0,
-                     spatial_sweeps=10):
+                     spatial_sweeps=10, parametric=False):
     """Same arguments as the reference.  `num_cores` selects the number of GPUs (-1 = all visible; see
     n_gpus_from_num_cores): the masked voxels of the volume are spread over them by pipeline.MultiGpuFit.
 
@@ -73,7 +73,11 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
 
     spatial_mu > 0 (not in the reference): the six maps, fsol_4D and Est_Signal are those of the spatially regularised
     fit, spatial_sweeps red-black sweeps that couple each voxel's spectrum to its face neighbours' with weight
-    spatial_mu (pipeline.recon_arrays); FA and reg_param stay the point fit's.  The same ten files are written."""
+    spatial_mu (pipeline.recon_arrays); FA and reg_param stay the point fit's.  The same ten files are written.
+
+    parametric=True (not in the reference): also the three-pool parametric fit started from each voxel's point fit
+    (pipeline.recon_arrays), written as MWF_3pool, IEWF_3pool, FWF_3pool, T2_M_3pool, T2_IE_3pool, T2_FW_3pool,
+    FA_3pool, TWC_3pool, SSE_3pool and Est_Signal_3pool (.nii.gz) beside the unchanged ten outputs."""
     n_gpus = n_gpus_from_num_cores(num_cores)
     warm = threading.Thread(target=_warm_gpus, args=(n_gpus,), daemon=True)   # CUDA contexts + libmet2.so while the files load
     warm.start()
@@ -109,11 +113,12 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
     vol = pipeline.recon_arrays(data, mask, np.asarray(TE_array, dtype=np.float64), TR, reg_method, reg_matrix,
                                 FA_method, myelin_T2=myelin_T2, data_fa=data_fa, diagnostics=True, premasked=True,
                                 n_gpus=n_gpus, n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed,
-                                spatial_mu=spatial_mu, spatial_sweeps=spatial_sweeps)
+                                spatial_mu=spatial_mu, spatial_sweeps=spatial_sweeps, parametric=parametric)
     print('Step #4: Estimation of quantitative metrics')
     # the ten volumes (motor...:474-503) are written concurrently, largest first: every writer deflates with all cores
     # (nifti_io), but the eight 3-D maps are too small to keep them busy one at a time (2.2 s -> 1.2 s on 8 cores)
-    names = OUTPUTS + (BOOTSTRAP_OUTPUTS if n_bootstrap > 0 else ())
+    names = OUTPUTS + (BOOTSTRAP_OUTPUTS if n_bootstrap > 0 else ()) + \
+        (tuple(pipeline.PARAM_VOLUMES) if parametric else ())
     order = sorted(names, key=lambda name: -vol[name].size)
     with ThreadPoolExecutor(max_workers=4) as pool:
         list(pool.map(lambda name: nifti_io.save(vol[name], join(name + '.nii.gz'), affine=img.affine), order))

@@ -125,6 +125,23 @@ def bootstrap_fitted(plan, sig, fa_index, t2, n_bootstrap, seed, voxel_offset):
     return dict(boot_stats=stats, boot_n_valid=n_valid)
 
 
+PARAM_KEYS = ("param_params", "param_maps", "param_est_signal", "param_sse", "param_iters", "param_status")
+# the volumes of the three-pool parametric fit: name -> (output, column)
+PARAM_VOLUMES = {"MWF_3pool": ("param_maps", 0), "IEWF_3pool": ("param_maps", 1), "FWF_3pool": ("param_maps", 2),
+                 "T2_M_3pool": ("param_maps", 3), "T2_IE_3pool": ("param_maps", 4), "T2_FW_3pool": ("param_params", 5),
+                 "FA_3pool": ("param_params", 6), "TWC_3pool": ("param_maps", 5), "SSE_3pool": ("param_sse", None),
+                 "Est_Signal_3pool": ("param_est_signal", None)}
+
+
+def param_fitted(plan, sig, fa_deg, t2):
+    """`Met2Plan.param_fit` started from one point fit (`t2`: the `t2_fit` result on sig[V, nTE]; fa_deg[V] the FA
+    stage's angles).  Returns the PARAM_KEYS of CUDA tensors, enqueued on the current stream; T2_FW (params column 5)
+    is zeroed where the free-water amplitude is 0, like T2_M and T2_IE in the maps."""
+    pf = plan.param_fit(sig, fa_deg, t2["fsol"], t2["status"])
+    pf["params"][:, 5].masked_fill_(pf["params"][:, 2] <= 0.0, 0.0)
+    return {"param_" + k: pf[k] for k in ("params", "maps", "est_signal", "sse", "iters", "status")}
+
+
 def host_buffers(plan, V, pinned=True):
     """Host (pinned) arrays for the per-voxel outputs of `fit_voxels` / `MultiGpuFit.fit` of V voxels."""
     def mk(shape, dtype):
@@ -166,11 +183,12 @@ class MultiGpuFit:
                                 range(n)))
         return cls(plans, chunks_per_device)
 
-    def fit(self, sig, sig_fa=None, out=None, n_bootstrap=0, bootstrap_seed=0):
+    def fit(self, sig, sig_fa=None, out=None, n_bootstrap=0, bootstrap_seed=0, parametric=False):
         """sig[V, nTE] (+ sig_fa for the FA stage): host tensors / arrays, pinned for full-speed DMA.  `out`: dict of
         host tensors as from `host_buffers` (allocated if None).  Returns dict of numpy views of `out`.
         n_bootstrap > 0: also the per-voxel bootstrap of the maps (`bootstrap_fitted`, keys BOOT_KEYS), each device
         over its own chunks with voxel_offset = the chunk's start, so the result does not depend on the device count.
+        parametric: also the three-pool parametric fit (`param_fitted`, keys PARAM_KEYS), chunk by chunk on each device.
 
         Everything is ENQUEUED from this one thread, phase by phase over the devices (copies in, FA stage, T2 stage,
         copies out: ~0.1 ms of host time per device and phase, all asynchronous), then the streams are drained.  A
@@ -186,6 +204,13 @@ class MultiGpuFit:
             pin = torch.cuda.is_available()
             out["boot_stats"] = torch.empty((V, 6, 4), dtype=torch.float64, pin_memory=pin)
             out["boot_n_valid"] = torch.empty(V, dtype=torch.int32, pin_memory=pin)
+        if parametric and "param_params" not in out:
+            pin = torch.cuda.is_available()
+            nTE = self.plans[0].nTE
+            for k, shape, dt in (("param_params", (V, 7), torch.float64), ("param_maps", (V, 6), torch.float64),
+                                 ("param_est_signal", (V, nTE), torch.float64), ("param_sse", (V,), torch.float64),
+                                 ("param_iters", (V,), torch.int32), ("param_status", (V,), torch.int32)):
+                out[k] = torch.empty(shape, dtype=dt, pin_memory=pin)
         nd = len(self.plans)
         parts = chunk_deal(V, nd, self.chunks_per_device)
         trace = [dict() for _ in self.plans] if os.environ.get("MET2_MULTI_TRACE") else None
@@ -239,6 +264,18 @@ class MultiGpuFit:
                                                         n_bootstrap, bootstrap_seed, lo))
                         o += hi - lo
                 mark(d, "bootstrap_enqueued")
+        par = {}
+        if parametric:
+            for d in live:                               # ---- phase 3c: parametric fit, chunk by chunk
+                plan, b = self.plans[d], bufs[d]
+                with torch.cuda.device(plan.dev), torch.cuda.stream(self.streams[d]):
+                    o, par[d] = 0, []
+                    for lo, hi in parts[d]:
+                        rows = slice(o, o + hi - lo)
+                        t2 = {k: b["t2"][k][rows] for k in ("fsol", "status")}
+                        par[d].append(param_fitted(plan, b["sig"][rows], b["fa"]["fa_deg"][rows], t2))
+                        o += hi - lo
+                mark(d, "parametric_enqueued")
         for d in live:                                   # ---- phase 4: device -> its rows of the host arrays
             plan, b = self.plans[d], bufs[d]
             fa, t2 = b["fa"], b["t2"]
@@ -252,6 +289,8 @@ class MultiGpuFit:
                         out[k][lo:hi].copy_(dev_out[k][o:o + hi - lo], non_blocking=True)
                     for k in (BOOT_KEYS if n_bootstrap > 0 else ()):
                         out[k][lo:hi].copy_(boot[d][i][k], non_blocking=True)
+                    for k in (PARAM_KEYS if parametric else ()):
+                        out[k][lo:hi].copy_(par[d][i][k], non_blocking=True)
                     o += hi - lo
             mark(d, "d2h_enqueued")
         fs = torch.zeros(self.plans[0].npc, dtype=torch.float64)
@@ -266,7 +305,7 @@ class MultiGpuFit:
 
 
 def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, fa_only=False, n_bootstrap=0,
-               bootstrap_seed=0, voxel_offset=0, spatial=None):
+               bootstrap_seed=0, voxel_offset=0, spatial=None, parametric=False):
     """Steps 2-4 on a list of voxels given as host array sig[V, nTE]; returns host arrays (dict).
     in_mask[V] (optional): also return the mean-spectrum diagnostics of motor...:375-403 over the voxels with
     in_mask == 1 (key "diagnostics").  roi = (labels[V], values) (optional): also the ROI-based estimates of
@@ -274,7 +313,8 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
     with that many replicates (`bootstrap_fitted`, keys BOOT_KEYS); voxel_offset: the position of sig[0] in the whole
     voxel list (a torchrun rank's slab start).  spatial = (flat, shape, mu, n_sweeps) (optional): the voxels are the
     masked voxels flat[V] of a volume of `shape`, and fsol / est_signal / maps / status are those of the spatially
-    regularised fit with coupling weight mu (`spatial_fitted`)."""
+    regularised fit with coupling weight mu (`spatial_fitted`).  parametric: also the three-pool parametric fit started
+    from the point fit (`param_fitted`, keys PARAM_KEYS)."""
     dev = plan.dev
     V = sig.shape[0]
     with torch.cuda.device(dev):
@@ -295,6 +335,8 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
                 out.update(spatial_fitted(plan, d_sig, fa["fa_index"], t2, *spatial))
             if n_bootstrap > 0:
                 out.update(bootstrap_fitted(plan, d_sig, fa["fa_index"], t2, n_bootstrap, bootstrap_seed, voxel_offset))
+            if parametric:
+                out.update(param_fitted(plan, d_sig, fa["fa_deg"], t2))
         extra = {}
         if in_mask is not None and V > 0:
             extra["diagnostics"] = mean_spectrum_diagnostics(plan, d_sig, fa["fa_index"], in_mask, fa["fsol_sum"])
@@ -316,7 +358,7 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
 def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, myelin_T2=40.0, data_fa=None, plan=None,
                  npc=None, n_alphas=None, device=None, rank=0, world_size=1, diagnostics=False, rois=None,
                  premasked=False, fa_only=False, n_gpus=1, n_bootstrap=0, bootstrap_seed=0, spatial_mu=0.0,
-                 spatial_sweeps=10):
+                 spatial_sweeps=10, parametric=False):
     """Steps 2-4 of motor_recon_met2 on in-memory arrays.  Returns the ten output volumes (plus FA_index) as numpy.
 
     n_bootstrap > 0: also the per-voxel bootstrap uncertainty of the six maps with that many replicates per voxel
@@ -331,6 +373,13 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
     and reg_param stay the point fit's.  With several GPUs the point fit is spread over them and the sweeps run on the
     first.  It needs the whole volume in one process (world_size 1) and cannot be combined with n_bootstrap.
 
+    parametric: also the three-pool parametric fit (`batched.Met2Plan.param_fit`, definition in csrc/met2_param.cu)
+    started from each voxel's point fit: volumes MWF_3pool, IEWF_3pool, FWF_3pool, T2_M_3pool, T2_IE_3pool, T2_FW_3pool
+    (each T2 is 0 where its pool's amplitude is 0), FA_3pool, TWC_3pool, SSE_3pool [nx, ny, nz] and Est_Signal_3pool
+    [nx, ny, nz, nt]; zero outside the mask and where the point fit skipped the voxel.  The ten standard volumes are
+    unchanged.  Per voxel, so it runs on every GPU and rank like the point fit; it cannot be combined with spatial_mu,
+    since either spectrum could then start it.
+
     n_gpus != 1 (None / -1 = all visible GPUs): the voxel list of this ONE volume is spread over the GPUs of the node by
     `MultiGpuFit` (host in -> host out, no collective).  With world_size > 1 (one process per GPU under torchrun) only
     this rank's slab of the masked voxels is fitted and the other voxels are left zero; the caller combines the ranks
@@ -344,6 +393,9 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
         raise ValueError("the spatially regularised fit couples neighbouring voxels: run it unsharded")
     if spatial_mu > 0 and n_bootstrap > 0:
         raise ValueError("spatial_mu > 0 cannot be combined with n_bootstrap")
+    if spatial_mu > 0 and parametric:
+        raise ValueError("spatial_mu > 0 cannot be combined with parametric: it is ambiguous which spectrum starts the "
+                         "parametric fit")
     data = np.asarray(data, dtype=np.float64)
     nx, ny, nz, nt = data.shape
     TE_array = np.asarray(TE_array, dtype=np.float64)
@@ -389,7 +441,7 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
         if sig_fa is not None:
             pin_fa = torch.empty((V, nt), dtype=torch.float64).pin_memory()
             pin_fa.copy_(sig_fa if isinstance(sig_fa, torch.Tensor) else torch.as_tensor(sig_fa))
-        res = multi.fit(pin, pin_fa, n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed)
+        res = multi.fit(pin, pin_fa, n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed, parametric=parametric)
         if (in_mask is not None or roi is not None) and V > 0:
             # whole-volume reductions (a few ms): on the first device, from the gathered FA indices
             with torch.cuda.device(plan.dev):
@@ -411,7 +463,8 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
     else:
         spatial = (flat, (nx, ny, nz), spatial_mu, spatial_sweeps) if spatial_mu > 0 and not fa_only else None
         res = fit_voxels(plan, sig[lo:hi], sig_fa, in_mask=in_mask, roi=roi, fa_only=fa_only,
-                         n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed, voxel_offset=lo, spatial=spatial)
+                         n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed, voxel_offset=lo, spatial=spatial,
+                         parametric=parametric)
     sel = flat[lo:hi]
     nvox = nx * ny * nz
     vol = {}
@@ -450,6 +503,12 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
         a = np.zeros(nvox, dtype=np.int32)
         a[sel] = res["boot_n_valid"]
         vol["bootstrap_n_valid"] = a.reshape(nx, ny, nz)
+    if parametric:
+        for name, (key, col) in PARAM_VOLUMES.items():
+            src = res[key] if col is None else res[key][:, col]
+            a = np.zeros((nvox,) + src.shape[1:])
+            a[sel] = src
+            vol[name] = a.reshape((nx, ny, nz) + src.shape[1:])
     return vol
 
 
