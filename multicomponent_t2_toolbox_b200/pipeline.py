@@ -72,10 +72,6 @@ def chunk_deal(n_voxels, n_parts, chunks_per_part=4, align=64):
     return parts
 
 
-OUT_KEYS = ("fa_index", "fa_deg", "km", "fa_status", "fsol", "est_signal", "reg", "maps", "status")
-BOOT_KEYS = ("boot_stats", "boot_n_valid")
-
-
 def spatial_neighbours(flat, shape, fitted):
     """Neighbour table and red-black colours of the spatially regularised fit (`batched.Met2Plan.spatial_fit`).
     flat[V]: C-order indices of the masked voxels in a volume of `shape` (nx, ny, nz), as `masked_voxel_list` returns
@@ -98,69 +94,133 @@ def spatial_neighbours(flat, shape, fitted):
     return nbr, colours
 
 
-SPATIAL_KEYS = ("fsol", "est_signal", "maps", "status")
+# The per-voxel outputs of the stages: name, trailing shape (ints and Met2Plan attributes), dtype, and the stage that
+# produces it.  "fa" always runs, "t2" unless fa_only, "bootstrap" when n_bootstrap > 0, "parametric" when parametric.
+VOXEL_OUTPUTS = (
+    ("fa_index", (), torch.int32, "fa"), ("fa_deg", (), torch.float64, "fa"), ("km", (), torch.float64, "fa"),
+    ("fa_status", (), torch.int32, "fa"),
+    ("fsol", ("npc",), torch.float64, "t2"), ("est_signal", ("nTE",), torch.float64, "t2"),
+    ("reg", (), torch.float64, "t2"), ("maps", (6,), torch.float64, "t2"), ("status", (), torch.int32, "t2"),
+    ("boot_stats", (6, 4), torch.float64, "bootstrap"), ("boot_n_valid", (), torch.int32, "bootstrap"),
+    ("param_params", (7,), torch.float64, "parametric"), ("param_maps", (6,), torch.float64, "parametric"),
+    ("param_est_signal", ("nTE",), torch.float64, "parametric"), ("param_sse", (), torch.float64, "parametric"),
+    ("param_iters", (), torch.int32, "parametric"), ("param_status", (), torch.int32, "parametric"))
 
-
-def spatial_fitted(plan, sig, fa_index, t2, flat, shape, mu, n_sweeps):
-    """`Met2Plan.spatial_fit` after the point fit `t2` (the `t2_fit` result on sig[V, nTE] at fa_index[V], CUDA) of the
-    masked voxels flat[V] of a volume of `shape`: lambda_v from a second `t2_fit` with MET2_T2_FLAG_REG_IS_LAMBDA, the
-    neighbour table of the fitted voxels (`spatial_neighbours`; reads the point fit's status back to the host), then the
-    sweeps.  Returns dict(fsol, est_signal, maps, status) of CUDA tensors; reg stays the point fit's."""
-    lam = plan.t2_fit(sig, fa_index, flags=batched.REG_IS_LAMBDA)["reg"]
-    fitted = ((t2["status"] & batched.ST_SKIPPED) == 0).cpu().numpy()
-    nbr, colours = spatial_neighbours(flat, shape, fitted)
-    sp = plan.spatial_fit(sig, fa_index, lam, t2["fsol"], nbr, colours, mu, n_sweeps, status=t2["status"])
-    return {k: sp[k] for k in SPATIAL_KEYS}
-
-
-def bootstrap_fitted(plan, sig, fa_index, t2, n_bootstrap, seed, voxel_offset):
-    """`Met2Plan.bootstrap` of the voxels of one point fit (`t2`: the `t2_fit` result on sig[V, nTE] at fa_index[V]),
-    with voxel_offset = the position of sig[0] in the whole voxel list.  Voxels the point fit skipped get zeros, like
-    their maps.  Returns dict(boot_stats[V, 6, 4], boot_n_valid[V]) of CUDA tensors, enqueued on the current stream."""
-    stats, n_valid = plan.bootstrap(sig, fa_index, t2["est_signal"], B=n_bootstrap, seed=seed,
-                                    voxel_offset=voxel_offset)
-    skipped = (t2["status"] & batched.ST_SKIPPED) != 0
-    stats.masked_fill_(skipped[:, None, None], 0.0)
-    n_valid.masked_fill_(skipped, 0)
-    return dict(boot_stats=stats, boot_n_valid=n_valid)
-
-
-PARAM_KEYS = ("param_params", "param_maps", "param_est_signal", "param_sse", "param_iters", "param_status")
 # the volumes of the three-pool parametric fit: name -> (output, column)
 PARAM_VOLUMES = {"MWF_3pool": ("param_maps", 0), "IEWF_3pool": ("param_maps", 1), "FWF_3pool": ("param_maps", 2),
                  "T2_M_3pool": ("param_maps", 3), "T2_IE_3pool": ("param_maps", 4), "T2_FW_3pool": ("param_params", 5),
                  "FA_3pool": ("param_params", 6), "TWC_3pool": ("param_maps", 5), "SSE_3pool": ("param_sse", None),
                  "Est_Signal_3pool": ("param_est_signal", None)}
 
+# The volumes of `recon_arrays`: name, per-voxel output, column (None: all of it) and dtype.  A volume is returned when
+# its per-voxel output was computed.
+VOLUMES = (("FA", "fa_deg", None, np.float64), ("FA_index", "fa_index", None, np.float64),
+           *((name, "maps", i, np.float64) for i, name in enumerate(MAP_NAMES)),
+           ("reg_param", "reg", None, np.float64), ("fsol_4D", "fsol", None, np.float64),
+           ("Est_Signal", "est_signal", None, np.float64), ("status", "status", None, np.int32),
+           *((name + "_bootstrap", "boot_stats", i, np.float64) for i, name in enumerate(MAP_NAMES)),
+           ("bootstrap_n_valid", "boot_n_valid", None, np.int32),
+           *((name, key, col, np.float64) for name, (key, col) in PARAM_VOLUMES.items()))
 
-def param_fitted(plan, sig, fa_deg, t2):
-    """`Met2Plan.param_fit` started from one point fit (`t2`: the `t2_fit` result on sig[V, nTE]; fa_deg[V] the FA
-    stage's angles).  Returns the PARAM_KEYS of CUDA tensors, enqueued on the current stream; T2_FW (params column 5)
-    is zeroed where the free-water amplitude is 0, like T2_M and T2_IE in the maps."""
-    pf = plan.param_fit(sig, fa_deg, t2["fsol"], t2["status"])
+
+def _fa_stage(plan, s):
+    fa = s["fa"] = plan.fa_fit(s["sig_fa"], out=s["fa"])
+    return dict(fa_index=fa["fa_index"], fa_deg=fa["fa_deg"], km=fa["km"], fa_status=fa["status"])
+
+
+def _t2_stage(plan, s):
+    s["t2"] = plan.t2_fit(s["sig"], s["fa"]["fa_index"], out=s["t2"])
+    return dict(s["t2"])
+
+
+def _bootstrap_stage(plan, s, n_bootstrap, seed):
+    """`Met2Plan.bootstrap` from the point fit, one call per contiguous range of s["ranges"] with voxel_offset = the
+    range's start in the whole voxel list (a voxel's replicates depend on that position).  Voxels the point fit skipped
+    get zeros, like their maps."""
+    t2, fa_index = s["t2"], s["fa"]["fa_index"]
+    parts, o = [], 0
+    for lo, hi in s["ranges"]:
+        rows = slice(o, o + hi - lo)
+        parts.append(plan.bootstrap(s["sig"][rows], fa_index[rows], t2["est_signal"][rows], B=n_bootstrap, seed=seed,
+                                    voxel_offset=lo))
+        o += hi - lo
+    stats, n_valid = (torch.cat(p) for p in zip(*parts))
+    skipped = (t2["status"] & batched.ST_SKIPPED) != 0
+    stats.masked_fill_(skipped[:, None, None], 0.0)
+    n_valid.masked_fill_(skipped, 0)
+    return dict(boot_stats=stats, boot_n_valid=n_valid)
+
+
+def _param_stage(plan, s):
+    """`Met2Plan.param_fit` started from the point fit; T2_FW (params column 5) is zeroed where the free-water
+    amplitude is 0, like T2_M and T2_IE in the maps."""
+    pf = plan.param_fit(s["sig"], s["fa"]["fa_deg"], s["t2"]["fsol"], s["t2"]["status"])
     pf["params"][:, 5].masked_fill_(pf["params"][:, 2] <= 0.0, 0.0)
-    return {"param_" + k: pf[k] for k in ("params", "maps", "est_signal", "sse", "iters", "status")}
+    return {"param_" + k: v for k, v in pf.items()}
 
 
-def host_buffers(plan, V, pinned=True):
-    """Host (pinned) arrays for the per-voxel outputs of `fit_voxels` / `MultiGpuFit.fit` of V voxels."""
-    def mk(shape, dtype):
-        t = torch.empty(shape, dtype=dtype)
-        return t.pin_memory() if pinned and torch.cuda.is_available() else t
-    return {"fsol": mk((V, plan.npc), torch.float64), "est_signal": mk((V, plan.nTE), torch.float64),
-            "maps": mk((V, 6), torch.float64), "reg": mk((V,), torch.float64), "fa_deg": mk((V,), torch.float64),
-            "fa_index": mk((V,), torch.int32), "km": mk((V,), torch.float64), "status": mk((V,), torch.int32),
-            "fa_status": mk((V,), torch.int32), "fsol_sum": mk((plan.npc,), torch.float64)}
+def _stages(fa_only=False, n_bootstrap=0, bootstrap_seed=0, parametric=False):
+    """The per-voxel stages in order, as (name, stage).  A stage takes (plan, s), s: the device state of one set of
+    voxels (sig, sig_fa, ranges: their (lo, hi) in the whole voxel list, and the fa / t2 results, reused as `out=`), and
+    returns its VOXEL_OUTPUTS as CUDA tensors, enqueued on the current stream.  Bootstrap and the parametric fit start
+    from the point fit."""
+    stages = [("fa", _fa_stage)]
+    if not fa_only:
+        stages.append(("t2", _t2_stage))
+        if n_bootstrap > 0:
+            stages.append(("bootstrap", lambda plan, s: _bootstrap_stage(plan, s, n_bootstrap, bootstrap_seed)))
+        if parametric:
+            stages.append(("parametric", _param_stage))
+    return stages
+
+
+def _outputs(stages):
+    """The entries of VOXEL_OUTPUTS that `stages` produce."""
+    ran = {name for name, _ in stages}
+    return [o for o in VOXEL_OUTPUTS if o[3] in ran]
+
+
+def host_buffers(plan, V, pinned=True, n_bootstrap=0, parametric=False):
+    """Host (pinned) arrays for the outputs of `fit_voxels` / `MultiGpuFit.fit` of V voxels: the per-voxel outputs of
+    the point fit, plus those of the bootstrap (n_bootstrap > 0) and of the parametric fit, and fsol_sum[npc]."""
+    pin = pinned and torch.cuda.is_available()
+    bufs = {name: torch.empty((V,) + tuple(getattr(plan, n) if isinstance(n, str) else n for n in shape), dtype=dtype,
+                              pin_memory=pin)
+            for name, shape, dtype, _ in _outputs(_stages(n_bootstrap=n_bootstrap, parametric=parametric))}
+    bufs["fsol_sum"] = torch.empty(plan.npc, dtype=torch.float64, pin_memory=pin)
+    return bufs
+
+
+def _whole_volume(plan, sig, fa_index, fsol_sum, in_mask=None, roi=None, spatial=None, fsol=None, status=None):
+    """The steps that need every voxel on one device (plan.dev), from sig[V, nTE] and fa_index[V] (CUDA): the
+    mean-spectrum diagnostics over in_mask, the ROI estimates of roi = (labels[V], values), and the spatially
+    regularised fit of spatial = (flat, shape, mu, n_sweeps) started from the point fit's fsol / status (host or CUDA):
+    lambda_v from a second `t2_fit` with MET2_T2_FLAG_REG_IS_LAMBDA, the neighbour table of the fitted voxels, then the
+    sweeps.  Returns ({"diagnostics", "roi"} as requested, the spatial fit's fsol / est_signal / maps / status as CUDA
+    tensors); reg stays the point fit's."""
+    extra, sp = {}, {}
+    if in_mask is not None:
+        extra["diagnostics"] = mean_spectrum_diagnostics(plan, sig, fa_index, in_mask, fsol_sum)
+    if roi is not None:
+        extra["roi"] = roi_estimates(plan, sig, fa_index, roi[0], roi[1])
+    if spatial is not None:
+        flat, shape, mu, n_sweeps = spatial
+        lam = plan.t2_fit(sig, fa_index, flags=batched.REG_IS_LAMBDA)["reg"]
+        status = torch.as_tensor(status).to(plan.dev)
+        nbr, colours = spatial_neighbours(flat, shape, ((status & batched.ST_SKIPPED) == 0).cpu().numpy())
+        sp = plan.spatial_fit(sig, fa_index, lam, fsol, nbr, colours, mu, n_sweeps, status=status)
+        sp = {k: sp[k] for k in ("fsol", "est_signal", "maps", "status")}
+    return extra, sp
 
 
 class MultiGpuFit:
     """Steps 2-4 of ONE volume on several GPUs of one node, host memory in -> host memory out (the reference's only
     parallel knob, `num_cores` of motor_recon_met2 — joblib workers over image rows, motor...:165,357,365,435 — becomes
     the number of GPUs).  Voxels are independent, so there is no collective: the voxel list is dealt to the devices in
-    a few large contiguous chunks (`chunk_deal`), one host thread per device copies its chunks from the (pinned) input
-    array, runs the two batched kernels on its own stream and copies every output straight into its rows of ONE set of
-    pinned host arrays — disjoint ranges, written by DMA, nothing to gather afterwards.  Per-voxel results are
-    byte-identical to the single-GPU run (tests/test_gpu_multi.py)."""
+    a few large contiguous chunks (`chunk_deal`), each device copies its chunks from the (pinned) input array, runs the
+    stages on its own stream and copies every output straight into its rows of ONE set of pinned host arrays —
+    disjoint ranges, written by DMA, nothing to gather afterwards.  Per-voxel results are byte-identical to the
+    single-GPU run (tests/test_gpu_multi.py, tests/test_gpu_pipeline.py)."""
 
     def __init__(self, plans, chunks_per_device=4):
         if not plans:
@@ -185,32 +245,24 @@ class MultiGpuFit:
 
     def fit(self, sig, sig_fa=None, out=None, n_bootstrap=0, bootstrap_seed=0, parametric=False):
         """sig[V, nTE] (+ sig_fa for the FA stage): host tensors / arrays, pinned for full-speed DMA.  `out`: dict of
-        host tensors as from `host_buffers` (allocated if None).  Returns dict of numpy views of `out`.
-        n_bootstrap > 0: also the per-voxel bootstrap of the maps (`bootstrap_fitted`, keys BOOT_KEYS), each device
-        over its own chunks with voxel_offset = the chunk's start, so the result does not depend on the device count.
-        parametric: also the three-pool parametric fit (`param_fitted`, keys PARAM_KEYS), chunk by chunk on each device.
+        host tensors as from `host_buffers` (what it lacks is allocated).  Returns dict of numpy views of `out`.
+        n_bootstrap > 0: also the per-voxel bootstrap of the maps (keys boot_*), each device over its own chunks with
+        voxel_offset = the chunk's start, so the result does not depend on the device count.  parametric: also the
+        three-pool parametric fit (keys param_*).
 
-        Everything is ENQUEUED from this one thread, phase by phase over the devices (copies in, FA stage, T2 stage,
-        copies out: ~0.1 ms of host time per device and phase, all asynchronous), then the streams are drained.  A
-        thread per device was measured slower: two threads inside the CUDA runtime stalled each other for ~36 ms per
-        call (profiles/r02_multi_gpu.json), a serial enqueue staggers the devices by well under a millisecond."""
+        Everything is ENQUEUED from this one thread, phase by phase over the devices (copies in, then each stage of
+        `_stages`, then copies out: ~0.1 ms of host time per device and phase, all asynchronous), then the streams are
+        drained.  A thread per device was measured slower: two threads inside the CUDA runtime stalled each other for
+        ~36 ms per call (profiles/r02_multi_gpu.json), a serial enqueue staggers the devices by well under a
+        millisecond."""
         sig = torch.as_tensor(sig)
         if sig_fa is not None:
             sig_fa = torch.as_tensor(sig_fa)
         V = sig.shape[0]
-        if out is None:
-            out = host_buffers(self.plans[0], V)
-        if n_bootstrap > 0 and "boot_stats" not in out:
-            pin = torch.cuda.is_available()
-            out["boot_stats"] = torch.empty((V, 6, 4), dtype=torch.float64, pin_memory=pin)
-            out["boot_n_valid"] = torch.empty(V, dtype=torch.int32, pin_memory=pin)
-        if parametric and "param_params" not in out:
-            pin = torch.cuda.is_available()
-            nTE = self.plans[0].nTE
-            for k, shape, dt in (("param_params", (V, 7), torch.float64), ("param_maps", (V, 6), torch.float64),
-                                 ("param_est_signal", (V, nTE), torch.float64), ("param_sse", (V,), torch.float64),
-                                 ("param_iters", (V,), torch.int32), ("param_status", (V,), torch.int32)):
-                out[k] = torch.empty(shape, dtype=dt, pin_memory=pin)
+        stages = _stages(False, n_bootstrap, bootstrap_seed, parametric)
+        names = [name for name, *_ in _outputs(stages)]
+        if out is None or not all(k in out for k in names):
+            out = {**host_buffers(self.plans[0], V, n_bootstrap=n_bootstrap, parametric=parametric), **(out or {})}
         nd = len(self.plans)
         parts = chunk_deal(V, nd, self.chunks_per_device)
         trace = [dict() for _ in self.plans] if os.environ.get("MET2_MULTI_TRACE") else None
@@ -228,11 +280,11 @@ class MultiGpuFit:
             b = self._bufs.get(key)
             with torch.cuda.device(plan.dev), torch.cuda.stream(self.streams[d]):
                 if b is None:
-                    b = dict(sig=torch.empty((Vd, plan.nTE), dtype=torch.float64, device=plan.dev),
-                             sig_fa=(torch.empty((Vd, plan.nTE), dtype=torch.float64, device=plan.dev)
-                                     if sig_fa is not None else None), fa=None, t2=None)
+                    d_sig = torch.empty((Vd, plan.nTE), dtype=torch.float64, device=plan.dev)
+                    b = dict(sig=d_sig, sig_fa=d_sig if sig_fa is None else torch.empty_like(d_sig), fa=None, t2=None)
                     self._bufs = {k: v for k, v in self._bufs.items() if k[0] != d}
                     self._bufs[key] = b
+                b["ranges"] = parts[d]
                 o = 0
                 for lo, hi in parts[d]:
                     b["sig"][o:o + hi - lo].copy_(sig[lo:hi], non_blocking=True)
@@ -241,56 +293,18 @@ class MultiGpuFit:
                     o += hi - lo
             bufs[d] = b
             mark(d, "h2d_enqueued")
-        for d in live:                                   # ---- phase 2: flip-angle stage
-            plan, b = self.plans[d], bufs[d]
-            with torch.cuda.device(plan.dev), torch.cuda.stream(self.streams[d]):
-                b["fa"] = plan.fa_fit(b["sig"] if sig_fa is None else b["sig_fa"], out=b["fa"])
-            mark(d, "fa_enqueued")
-        for d in live:                                   # ---- phase 3: spectrum fit + maps
-            plan, b = self.plans[d], bufs[d]
-            with torch.cuda.device(plan.dev), torch.cuda.stream(self.streams[d]):
-                b["t2"] = plan.t2_fit(b["sig"], b["fa"]["fa_index"], out=b["t2"])
-            mark(d, "t2_enqueued")
-        boot = {}
-        if n_bootstrap > 0:
-            for d in live:                               # ---- phase 3b: bootstrap, chunk by chunk
-                plan, b = self.plans[d], bufs[d]
-                with torch.cuda.device(plan.dev), torch.cuda.stream(self.streams[d]):
-                    o, boot[d] = 0, []
-                    for lo, hi in parts[d]:
-                        rows = slice(o, o + hi - lo)
-                        t2 = {k: b["t2"][k][rows] for k in ("est_signal", "status")}
-                        boot[d].append(bootstrap_fitted(plan, b["sig"][rows], b["fa"]["fa_index"][rows], t2,
-                                                        n_bootstrap, bootstrap_seed, lo))
-                        o += hi - lo
-                mark(d, "bootstrap_enqueued")
-        par = {}
-        if parametric:
-            for d in live:                               # ---- phase 3c: parametric fit, chunk by chunk
-                plan, b = self.plans[d], bufs[d]
-                with torch.cuda.device(plan.dev), torch.cuda.stream(self.streams[d]):
-                    o, par[d] = 0, []
-                    for lo, hi in parts[d]:
-                        rows = slice(o, o + hi - lo)
-                        t2 = {k: b["t2"][k][rows] for k in ("fsol", "status")}
-                        par[d].append(param_fitted(plan, b["sig"][rows], b["fa"]["fa_deg"][rows], t2))
-                        o += hi - lo
-                mark(d, "parametric_enqueued")
+        res = {d: {} for d in live}
+        for name, stage in stages:                       # ---- phases 2-3: each stage on every device
+            for d in live:
+                with torch.cuda.device(self.plans[d].dev), torch.cuda.stream(self.streams[d]):
+                    res[d].update(stage(self.plans[d], bufs[d]))
+                mark(d, name + "_enqueued")
         for d in live:                                   # ---- phase 4: device -> its rows of the host arrays
-            plan, b = self.plans[d], bufs[d]
-            fa, t2 = b["fa"], b["t2"]
-            dev_out = dict(fa_index=fa["fa_index"], fa_deg=fa["fa_deg"], km=fa["km"], fa_status=fa["status"],
-                           fsol=t2["fsol"], est_signal=t2["est_signal"], reg=t2["reg"], maps=t2["maps"],
-                           status=t2["status"])
-            with torch.cuda.device(plan.dev), torch.cuda.stream(self.streams[d]):
+            with torch.cuda.device(self.plans[d].dev), torch.cuda.stream(self.streams[d]):
                 o = 0
-                for i, (lo, hi) in enumerate(parts[d]):
-                    for k in OUT_KEYS:
-                        out[k][lo:hi].copy_(dev_out[k][o:o + hi - lo], non_blocking=True)
-                    for k in (BOOT_KEYS if n_bootstrap > 0 else ()):
-                        out[k][lo:hi].copy_(boot[d][i][k], non_blocking=True)
-                    for k in (PARAM_KEYS if parametric else ()):
-                        out[k][lo:hi].copy_(par[d][i][k], non_blocking=True)
+                for lo, hi in parts[d]:
+                    for k in names:
+                        out[k][lo:hi].copy_(res[d][k][o:o + hi - lo], non_blocking=True)
                     o += hi - lo
             mark(d, "d2h_enqueued")
         fs = torch.zeros(self.plans[0].npc, dtype=torch.float64)
@@ -310,11 +324,11 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
     in_mask[V] (optional): also return the mean-spectrum diagnostics of motor...:375-403 over the voxels with
     in_mask == 1 (key "diagnostics").  roi = (labels[V], values) (optional): also the ROI-based estimates of
     motor_recon_met2_real_data_ROI.py:405-445 (key "roi").  n_bootstrap > 0: also the per-voxel bootstrap of the maps
-    with that many replicates (`bootstrap_fitted`, keys BOOT_KEYS); voxel_offset: the position of sig[0] in the whole
-    voxel list (a torchrun rank's slab start).  spatial = (flat, shape, mu, n_sweeps) (optional): the voxels are the
-    masked voxels flat[V] of a volume of `shape`, and fsol / est_signal / maps / status are those of the spatially
-    regularised fit with coupling weight mu (`spatial_fitted`).  parametric: also the three-pool parametric fit started
-    from the point fit (`param_fitted`, keys PARAM_KEYS)."""
+    with that many replicates (keys boot_*); voxel_offset: the position of sig[0] in the whole voxel list (a torchrun
+    rank's slab start).  spatial = (flat, shape, mu, n_sweeps) (optional): the voxels are the masked voxels flat[V] of
+    a volume of `shape`, and fsol / est_signal / maps / status are those of the spatially regularised fit with coupling
+    weight mu.  parametric: also the three-pool parametric fit started from the point fit (keys param_*).  fa_only:
+    only the FA stage's outputs."""
     dev = plan.dev
     V = sig.shape[0]
     with torch.cuda.device(dev):
@@ -325,25 +339,20 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
             d_sig_fa = sig_fa.to(dev)
         else:
             d_sig_fa = torch.as_tensor(sig_fa).to(dev, non_blocking=True)
-        fa = plan.fa_fit(d_sig_fa)
-        out = dict(fa_index=fa["fa_index"], fa_deg=fa["fa_deg"], km=fa["km"], fsol_sum=fa["fsol_sum"],
-                   fa_status=fa["status"])
-        if not fa_only:
-            t2 = plan.t2_fit(d_sig, fa["fa_index"])
-            out.update(fsol=t2["fsol"], est_signal=t2["est_signal"], reg=t2["reg"], maps=t2["maps"], status=t2["status"])
-            if spatial is not None:
-                out.update(spatial_fitted(plan, d_sig, fa["fa_index"], t2, *spatial))
-            if n_bootstrap > 0:
-                out.update(bootstrap_fitted(plan, d_sig, fa["fa_index"], t2, n_bootstrap, bootstrap_seed, voxel_offset))
-            if parametric:
-                out.update(param_fitted(plan, d_sig, fa["fa_deg"], t2))
+        s = dict(sig=d_sig, sig_fa=d_sig_fa, ranges=[(voxel_offset, voxel_offset + V)], fa=None, t2=None)
+        stages = _stages(fa_only, n_bootstrap, bootstrap_seed, parametric)
+        out = {}
+        for _, stage in stages:
+            out.update(stage(plan, s))
+        out["fsol_sum"] = s["fa"]["fsol_sum"]
         extra = {}
-        if in_mask is not None and V > 0:
-            extra["diagnostics"] = mean_spectrum_diagnostics(plan, d_sig, fa["fa_index"], in_mask, fa["fsol_sum"])
-        if roi is not None and V > 0:
-            extra["roi"] = roi_estimates(plan, d_sig, fa["fa_index"], roi[0], roi[1])
+        if V > 0:
+            extra, sp = _whole_volume(plan, d_sig, out["fa_index"], out["fsol_sum"], in_mask, roi,
+                                      None if fa_only else spatial, out.get("fsol"), out.get("status"))
+            out.update(sp)
         host = {}
-        for k, t in out.items():
+        for k in [name for name, *_ in _outputs(stages)] + ["fsol_sum"]:
+            t = out[k]
             if pinned_out is not None and k in pinned_out:
                 pinned_out[k][:t.shape[0]].copy_(t, non_blocking=True)
                 host[k] = pinned_out[k][:t.shape[0]]
@@ -433,6 +442,7 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
         vals = np.unique(np.asarray(rois).astype(np.int64))
         roi = (rl[flat], vals[vals != 0])
     in_mask = np.asarray(mask).reshape(-1)[flat] if diagnostics else None
+    spatial = (flat, (nx, ny, nz), spatial_mu, spatial_sweeps) if spatial_mu > 0 and not fa_only else None
     if multi is not None:
         V = hi - lo
         pin = torch.empty((V, nt), dtype=torch.float64).pin_memory()
@@ -442,73 +452,29 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
             pin_fa = torch.empty((V, nt), dtype=torch.float64).pin_memory()
             pin_fa.copy_(sig_fa if isinstance(sig_fa, torch.Tensor) else torch.as_tensor(sig_fa))
         res = multi.fit(pin, pin_fa, n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed, parametric=parametric)
-        if (in_mask is not None or roi is not None) and V > 0:
-            # whole-volume reductions (a few ms): on the first device, from the gathered FA indices
+        if V > 0 and (in_mask is not None or roi is not None or spatial is not None):
+            # these couple the voxels of every device's chunks: on the first device, from the gathered point fit
             with torch.cuda.device(plan.dev):
                 d_sig = pin.to(plan.dev, non_blocking=True)
                 d_idx = torch.as_tensor(res["fa_index"]).to(plan.dev)
-                if in_mask is not None:
-                    res["diagnostics"] = mean_spectrum_diagnostics(plan, d_sig, d_idx, in_mask, res["fsol_sum"])
-                if roi is not None:
-                    res["roi"] = roi_estimates(plan, d_sig, d_idx, roi[0], roi[1])
-        if spatial_mu > 0 and V > 0:
-            # the sweeps couple voxels of every device's chunks: on the first device, from the gathered point fit
-            with torch.cuda.device(plan.dev):
-                d_sig = pin.to(plan.dev, non_blocking=True)
-                d_idx = torch.as_tensor(res["fa_index"]).to(plan.dev)
-                t2 = dict(fsol=torch.as_tensor(res["fsol"]).to(plan.dev),
-                          status=torch.as_tensor(res["status"]).to(plan.dev))
-                sp = spatial_fitted(plan, d_sig, d_idx, t2, flat, (nx, ny, nz), spatial_mu, spatial_sweeps)
-                res.update({k: v.cpu().numpy() for k, v in sp.items()})
+                extra, sp = _whole_volume(plan, d_sig, d_idx, res["fsol_sum"], in_mask, roi, spatial, res["fsol"],
+                                          res["status"])
+                res.update(extra, **{k: v.cpu().numpy() for k, v in sp.items()})
     else:
-        spatial = (flat, (nx, ny, nz), spatial_mu, spatial_sweeps) if spatial_mu > 0 and not fa_only else None
         res = fit_voxels(plan, sig[lo:hi], sig_fa, in_mask=in_mask, roi=roi, fa_only=fa_only,
                          n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed, voxel_offset=lo, spatial=spatial,
                          parametric=parametric)
     sel = flat[lo:hi]
-    nvox = nx * ny * nz
     vol = {}
-    for name, key in (("FA", "fa_deg"), ("FA_index", "fa_index")):
-        a = np.zeros(nvox)
-        a[sel] = res[key]
-        vol[name] = a.reshape(nx, ny, nz)
-    vol["mean_T2_dist"] = res["fsol_sum"]
-    vol["T2s"] = plan.T2s
-    for k in ("diagnostics", "roi"):
-        if k in res:
-            vol[k] = res[k]
-    if fa_only:
-        return vol
-    for i, name in enumerate(MAP_NAMES):
-        a = np.zeros(nvox)
-        a[sel] = res["maps"][:, i]
-        vol[name] = a.reshape(nx, ny, nz)
-    a = np.zeros(nvox)
-    a[sel] = res["reg"]
-    vol["reg_param"] = a.reshape(nx, ny, nz)
-    f4 = np.zeros((nvox, plan.npc))
-    f4[sel] = res["fsol"]
-    vol["fsol_4D"] = f4.reshape(nx, ny, nz, plan.npc)
-    s4 = np.zeros((nvox, nt))
-    s4[sel] = res["est_signal"]
-    vol["Est_Signal"] = s4.reshape(nx, ny, nz, nt)
-    vol["status"] = np.zeros(nvox, dtype=np.int32)
-    vol["status"][sel] = res["status"]
-    vol["status"] = vol["status"].reshape(nx, ny, nz)
-    if n_bootstrap > 0:
-        for i, name in enumerate(MAP_NAMES):
-            a = np.zeros((nvox, 4))
-            a[sel] = res["boot_stats"][:, i, :]
-            vol[name + "_bootstrap"] = a.reshape(nx, ny, nz, 4)
-        a = np.zeros(nvox, dtype=np.int32)
-        a[sel] = res["boot_n_valid"]
-        vol["bootstrap_n_valid"] = a.reshape(nx, ny, nz)
-    if parametric:
-        for name, (key, col) in PARAM_VOLUMES.items():
+    for name, key, col, dtype in VOLUMES:
+        if key in res:
             src = res[key] if col is None else res[key][:, col]
-            a = np.zeros((nvox,) + src.shape[1:])
+            a = np.zeros((nx * ny * nz,) + src.shape[1:], dtype=dtype)
             a[sel] = src
             vol[name] = a.reshape((nx, ny, nz) + src.shape[1:])
+    vol["mean_T2_dist"] = res["fsol_sum"]
+    vol["T2s"] = plan.T2s
+    vol.update({k: res[k] for k in ("diagnostics", "roi") if k in res})
     return vol
 
 
