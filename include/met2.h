@@ -220,6 +220,19 @@ int64_t met2_tv_workspace_bytes(int nx, int ny, int nz, int nt);
 int met2_tv_chambolle(const double* vol, int nx, int ny, int nz, int nt, const double* weight, double eps, int max_iter,
                       double* out, int32_t* iterations, void* workspace, void* stream);
 
+/* Optional Step-1 preprocessing (no counterpart in the reference): Marchenko-Pastur PCA denoising (Veraart et al. 2016,
+ * MRtrix3's dwidenoise) with a per-voxel noise map.  Definition in csrc/met2_mppca.cu; bitwise equal to the NumPy
+ * restatement in tests/mppca_oracle.py.  For every voxel with mask == 1: PCA of the (2r + 1)^3 window (shifted, not
+ * shrunk, at the volume's edges), Marchenko-Pastur split of the eigenvalues into noise and signal, and the centre voxel
+ * rebuilt from the signal components.  vol/out [nx][ny][nz][nt] C-order (out must not alias vol), mask [nx][ny][nz]
+ * int32; outputs out, sigma [nx][ny][nz] (the noise standard deviation) and n_signal [nx][ny][nz] int32.  Voxels with
+ * mask != 1 get zeros; a window holding a non-finite sample gives out = the input, sigma = NaN, n_signal = -1.
+ * nt <= MET2_MAX_NTE, r >= 1 and at least 2 samples per window, else MET2_ERR_ARG before anything is enqueued; a mask
+ * with no voxel set is not an error (all outputs zero). */
+int64_t met2_mppca_workspace_bytes(int nx, int ny, int nz, int nt, int r);
+int met2_mppca(const double* vol, const int32_t* mask, int nx, int ny, int nz, int nt, int r, double* out, double* sigma,
+               int32_t* n_signal, void* workspace, void* stream);
+
 /* Per-voxel bootstrap uncertainty of the six maps (no counterpart in the reference).  Definition in
  * csrc/met2_boot.cu; both calls are bitwise equal to the NumPy restatement in tests/boot_oracle.py.
  *

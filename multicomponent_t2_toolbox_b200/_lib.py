@@ -61,6 +61,8 @@ SIGNATURES = {
     "met2_tv_workspace_bytes": (ctypes.c_int64, [ctypes.c_int] * 4),
     "met2_tv_chambolle": (ctypes.c_int, [c_void_p] + [ctypes.c_int] * 4 + [c_void_p, ctypes.c_double, ctypes.c_int,
                                                                           c_void_p, c_void_p, c_void_p, c_void_p]),
+    "met2_mppca_workspace_bytes": (ctypes.c_int64, [ctypes.c_int] * 5),
+    "met2_mppca": (ctypes.c_int, [c_void_p, c_void_p] + [ctypes.c_int] * 5 + [c_void_p] * 5),
     "met2_boot_resample": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_int,
                                           ctypes.c_uint64, ctypes.c_int64, c_void_p, c_void_p, c_void_p]),
     "met2_boot_summary": (ctypes.c_int, [c_void_p, c_void_p, ctypes.c_int64, ctypes.c_int, c_void_p, c_void_p,

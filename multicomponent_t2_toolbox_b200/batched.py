@@ -159,6 +159,33 @@ def tv_denoise(data, weight=None, eps=2e-4, max_num_iter=200, device=None):
     return out, iterations
 
 
+def mppca_denoise(data, mask, patch_radius=2, device=None):
+    """Marchenko-Pastur PCA denoising on the GPU (met2_mppca; definition in csrc/met2_mppca.cu): every voxel with
+    mask == 1 is rebuilt from the signal components of the PCA of its (2 patch_radius + 1)^3 window.  data[nx, ny, nz,
+    nt], mask[nx, ny, nz].  Returns CUDA tensors (denoised like data, noise sigma [nx, ny, nz], number of signal
+    components [nx, ny, nz] int32; 0 outside the mask, -1 where the window holds a non-finite sample)."""
+    dev = _require_cuda(device)
+    lib = _lib.load()
+    vol = _volume(data, dev)
+    if isinstance(mask, np.ndarray):
+        mask = torch.as_tensor(np.ascontiguousarray(mask))
+    msk = mask.to(device=dev, dtype=torch.int32).contiguous()
+    if tuple(msk.shape) != tuple(vol.shape[:3]):
+        raise ValueError("mask must be [nx, ny, nz] like data[..., 0]")
+    nx, ny, nz, nt = vol.shape
+    out = torch.empty_like(vol)
+    sigma = torch.empty((nx, ny, nz), dtype=torch.float64, device=dev)
+    n_signal = torch.empty((nx, ny, nz), dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        nbytes = lib.met2_mppca_workspace_bytes(nx, ny, nz, nt, int(patch_radius))
+        if nbytes < 0:
+            _lib.check(int(nbytes), "met2_mppca_workspace_bytes")
+        ws = torch.empty(int(nbytes), dtype=torch.uint8, device=dev)
+        _lib.check(lib.met2_mppca(_ptr(vol), _ptr(msk), nx, ny, nz, nt, int(patch_radius), _ptr(out), _ptr(sigma),
+                                  _ptr(n_signal), _ptr(ws), _stream()), "met2_mppca")
+    return out, sigma, n_signal
+
+
 def segment_means(sig, fa_index, labels, n_seg, dictionary):
     """Per-segment mean signal and mean kernel (met2_segment_means; motor...:377-392 and
     motor_recon_met2_real_data_ROI.py:408-423).  sig[V, nTE], fa_index[V], labels[V] in [0, n_seg) (else: no segment).

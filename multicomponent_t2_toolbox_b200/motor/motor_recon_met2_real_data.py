@@ -77,7 +77,11 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
 
     parametric=True (not in the reference): also the three-pool parametric fit started from each voxel's point fit
     (pipeline.recon_arrays), written as MWF_3pool, IEWF_3pool, FWF_3pool, T2_M_3pool, T2_IE_3pool, T2_FW_3pool,
-    FA_3pool, TWC_3pool, SSE_3pool and Est_Signal_3pool (.nii.gz) beside the unchanged ten outputs."""
+    FA_3pool, TWC_3pool, SSE_3pool and Est_Signal_3pool (.nii.gz) beside the unchanged ten outputs.
+
+    denoise='MPPCA' (not in the reference, reached from Python only): Step 1 is Marchenko-Pastur PCA denoising on the
+    GPU (batched.mppca_denoise, patch radius 2), and its per-voxel noise sigma is written as MPPCA_sigma.nii.gz beside
+    the ten outputs."""
     n_gpus = n_gpus_from_num_cores(num_cores)
     warm = threading.Thread(target=_warm_gpus, args=(n_gpus,), daemon=True)   # CUDA contexts + libmet2.so while the files load
     warm.start()
@@ -104,6 +108,11 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
     if denoise == 'NESMA':
         print('Step #1: Denoising using the NESMA filter:')
         data = batched.nesma_filter(data, mask).cpu().numpy()
+    mppca_sigma = None
+    if denoise == 'MPPCA':
+        print('Step #1: Denoising using MP-PCA:')
+        den, mppca_sigma, _ = batched.mppca_denoise(data, mask)
+        data, mppca_sigma = den.cpu().numpy(), mppca_sigma.cpu().numpy()
     print('Step #2: Estimation of flip angles:')
     data_fa = None
     if FA_smooth == 'yes':
@@ -122,6 +131,8 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
     order = sorted(names, key=lambda name: -vol[name].size)
     with ThreadPoolExecutor(max_workers=4) as pool:
         list(pool.map(lambda name: nifti_io.save(vol[name], join(name + '.nii.gz'), affine=img.affine), order))
+    if mppca_sigma is not None:
+        nifti_io.save(mppca_sigma, join('MPPCA_sigma.nii.gz'), affine=img.affine)
     dg = vol.get("diagnostics")
     if dg is not None:
         np.savetxt(join('Mean_spectrum_from_all_voxels.txt'),

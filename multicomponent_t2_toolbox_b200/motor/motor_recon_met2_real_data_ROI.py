@@ -31,6 +31,8 @@ def motor_recon_met2_ROIs(TE_array, path_to_data, path_to_mask, path_to_ROIs, pa
         data = tv_denoise(data)
     if denoise == 'NESMA':
         data = batched.nesma_filter(data, mask).cpu().numpy()
+    if denoise == 'MPPCA':      # not in the reference: MP-PCA on the GPU (batched.mppca_denoise), reached from Python
+        data = batched.mppca_denoise(data, mask)[0].cpu().numpy()
     data_fa = batched.gaussian_smooth(data, sigma=2.0) if FA_smooth == 'yes' else None
     vol = pipeline.recon_arrays(data, mask, np.asarray(TE_array, dtype=np.float64), TR, "X2", reg_matrix, FA_method,
                                 myelin_T2=myelin_T2, data_fa=data_fa, diagnostics=True, rois=ROIs, premasked=True,
