@@ -233,6 +233,21 @@ int64_t met2_mppca_workspace_bytes(int nx, int ny, int nz, int nt, int r);
 int met2_mppca(const double* vol, const int32_t* mask, int nx, int ny, int nz, int nt, int r, double* out, double* sigma,
                int32_t* n_signal, void* workspace, void* stream);
 
+/* Optional preprocessing after Step 1 (no counterpart in the reference): Gibbs-ringing removal by local subvoxel shifts
+ * (Kellner et al. 2016, MRtrix3's mrdegibbs, basic 2-D mode; partial-Fourier data are out of scope) on every in-plane
+ * slice vol[:, :, z, t].  Definition in csrc/met2_degibbs.cu; bitwise equal to the NumPy restatement in
+ * tests/degibbs_oracle.py.  vol/out [nx][ny][nz][nt] C-order float64 (out must not alias vol).  nsh shifts per half
+ * pixel (MRtrix: 20), TV window minW..maxW (MRtrix: 1..3).  1 <= nx, ny <= 256, nsh >= 1, 0 <= minW <= maxW,
+ * 2 maxW < nx and ny, and (2 nsh + 33) * 8 * max(nx, ny) bytes <= 227 KB (nsh <= 40 at 256), else MET2_ERR_ARG before
+ * anything is enqueued.
+ * met2_degibbs_tables writes the n * (2 nsh + 4) doubles of the tables of in-plane size n (cos[n], sin[n],
+ * 1 + cos(2 pi fftfreq)[n], the interpolation kernels h[2 nsh + 1][n]) to host_out unless it is NULL, and returns that
+ * count (MET2_ERR_ARG for n outside 1..256 or nsh outside 1..1024).  The kernels build the same bits on the device. */
+int64_t met2_degibbs_tables(int n, int nsh, double* host_out);
+int64_t met2_degibbs_workspace_bytes(int nx, int ny, int nz, int nt, int nsh, int minW, int maxW);
+int met2_degibbs(const double* vol, int nx, int ny, int nz, int nt, int nsh, int minW, int maxW, double* out,
+                 void* workspace, void* stream);
+
 /* Per-voxel bootstrap uncertainty of the six maps (no counterpart in the reference).  Definition in
  * csrc/met2_boot.cu; both calls are bitwise equal to the NumPy restatement in tests/boot_oracle.py.
  *

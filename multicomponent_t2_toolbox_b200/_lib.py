@@ -63,6 +63,9 @@ SIGNATURES = {
                                                                           c_void_p, c_void_p, c_void_p, c_void_p]),
     "met2_mppca_workspace_bytes": (ctypes.c_int64, [ctypes.c_int] * 5),
     "met2_mppca": (ctypes.c_int, [c_void_p, c_void_p] + [ctypes.c_int] * 5 + [c_void_p] * 5),
+    "met2_degibbs_tables": (ctypes.c_int64, [ctypes.c_int, ctypes.c_int, c_void_p]),
+    "met2_degibbs_workspace_bytes": (ctypes.c_int64, [ctypes.c_int] * 7),
+    "met2_degibbs": (ctypes.c_int, [c_void_p] + [ctypes.c_int] * 7 + [c_void_p] * 3),
     "met2_boot_resample": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_int,
                                           ctypes.c_uint64, ctypes.c_int64, c_void_p, c_void_p, c_void_p]),
     "met2_boot_summary": (ctypes.c_int, [c_void_p, c_void_p, ctypes.c_int64, ctypes.c_int, c_void_p, c_void_p,

@@ -186,6 +186,32 @@ def mppca_denoise(data, mask, patch_radius=2, device=None):
     return out, sigma, n_signal
 
 
+def degibbs(data, nsh=20, minW=1, maxW=3, axes=(0, 1), device=None):
+    """Gibbs-ringing removal by local subvoxel shifts on the GPU (met2_degibbs; definition in csrc/met2_degibbs.cu), the
+    method of MRtrix3's mrdegibbs (Kellner et al. 2016), applied to every 2-D slice spanned by `axes` of data[nx, ny, nz,
+    nt] (axes=(0, 2) or (1, 2) for sagittal or coronal slices).  Partial-Fourier data are out of scope.  Returns a CUDA
+    tensor like data."""
+    dev = _require_cuda(device)
+    lib = _lib.load()
+    vol = _volume(data, dev)
+    a0, a1 = (int(a) % 4 for a in axes)
+    if a0 == a1 or 3 in (a0, a1):
+        raise ValueError("axes must be two distinct spatial axes of [nx, ny, nz, nt]")
+    perm = [a0, a1] + [a for a in range(4) if a not in (a0, a1)]
+    vol = vol.permute(perm).contiguous()
+    n0, n1, n2, n3 = vol.shape
+    out = torch.empty_like(vol)
+    with torch.cuda.device(dev):
+        nbytes = lib.met2_degibbs_workspace_bytes(n0, n1, n2, n3, int(nsh), int(minW), int(maxW))
+        if nbytes < 0:
+            _lib.check(int(nbytes), "met2_degibbs_workspace_bytes")
+        ws = torch.empty(int(nbytes), dtype=torch.uint8, device=dev)
+        _lib.check(lib.met2_degibbs(_ptr(vol), n0, n1, n2, n3, int(nsh), int(minW), int(maxW), _ptr(out), _ptr(ws),
+                                    _stream()), "met2_degibbs")
+    inv = [perm.index(a) for a in range(4)]
+    return out.permute(inv).contiguous()
+
+
 def segment_means(sig, fa_index, labels, n_seg, dictionary):
     """Per-segment mean signal and mean kernel (met2_segment_means; motor...:377-392 and
     motor_recon_met2_real_data_ROI.py:408-423).  sig[V, nTE], fa_index[V], labels[V] in [0, n_seg) (else: no segment).

@@ -61,9 +61,19 @@ def _warm_gpus(n_gpus):
         pass
 
 
+def degibbs_step1(data, mask):
+    """Gibbs-ringing removal of the Step-1 output data[nx, ny, nz, nt] (batched.degibbs, in-plane axes 0 and 1, MRtrix's
+    defaults), masked again with negatives clipped to 0 like Step 1's input: the state recon_arrays(premasked=True)
+    expects."""
+    out = batched.degibbs(data).cpu().numpy()
+    np.multiply(out, mask[..., None], out=out)
+    out[out < 0.0] = 0.0
+    return out
+
+
 def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR, reg_method, reg_matrix, denoise,
                      FA_method, FA_smooth, myelin_T2, num_cores, n_bootstrap=0, bootstrap_seed=0, spatial_mu=0.0,
-                     spatial_sweeps=10, parametric=False):
+                     spatial_sweeps=10, parametric=False, degibbs=False):
     """Same arguments as the reference.  `num_cores` selects the number of GPUs (-1 = all visible; see
     n_gpus_from_num_cores): the masked voxels of the volume are spread over them by pipeline.MultiGpuFit.
 
@@ -81,7 +91,11 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
 
     denoise='MPPCA' (not in the reference, reached from Python only): Step 1 is Marchenko-Pastur PCA denoising on the
     GPU (batched.mppca_denoise, patch radius 2), and its per-voxel noise sigma is written as MPPCA_sigma.nii.gz beside
-    the ten outputs."""
+    the ten outputs.
+
+    degibbs=True (not in the reference, reached from Python only): after Step 1 (denoising first, as MRtrix advises:
+    unringing correlates the noise), every axial slice of every echo is unrung on the GPU (degibbs_step1, the local
+    subvoxel-shift method of MRtrix3's mrdegibbs), then masked again with negatives clipped to 0.  No file is added."""
     n_gpus = n_gpus_from_num_cores(num_cores)
     warm = threading.Thread(target=_warm_gpus, args=(n_gpus,), daemon=True)   # CUDA contexts + libmet2.so while the files load
     warm.start()
@@ -113,6 +127,9 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
         print('Step #1: Denoising using MP-PCA:')
         den, mppca_sigma, _ = batched.mppca_denoise(data, mask)
         data, mppca_sigma = den.cpu().numpy(), mppca_sigma.cpu().numpy()
+    if degibbs:
+        print('Step #1b: Gibbs-ringing removal:')
+        data = degibbs_step1(data, mask)
     print('Step #2: Estimation of flip angles:')
     data_fa = None
     if FA_smooth == 'yes':

@@ -12,11 +12,11 @@ import numpy as np
 from tabulate import tabulate
 
 from .. import batched, nifti_io, pipeline
-from .motor_recon_met2_real_data import tv_denoise
+from .motor_recon_met2_real_data import degibbs_step1, tv_denoise
 
 
 def motor_recon_met2_ROIs(TE_array, path_to_data, path_to_mask, path_to_ROIs, path_to_save_data, TR, reg_matrix, denoise,
-                          FA_method, FA_smooth, myelin_T2, num_cores):
+                          FA_method, FA_smooth, myelin_T2, num_cores, degibbs=False):
     img = nifti_io.load(path_to_data)
     data = img.get_fdata().astype(np.float64, copy=False)
     mask = nifti_io.load(path_to_mask).get_fdata().astype(np.int64, copy=False)
@@ -33,6 +33,8 @@ def motor_recon_met2_ROIs(TE_array, path_to_data, path_to_mask, path_to_ROIs, pa
         data = batched.nesma_filter(data, mask).cpu().numpy()
     if denoise == 'MPPCA':      # not in the reference: MP-PCA on the GPU (batched.mppca_denoise), reached from Python
         data = batched.mppca_denoise(data, mask)[0].cpu().numpy()
+    if degibbs:                 # not in the reference: Gibbs-ringing removal after Step 1, as motor_recon_met2(degibbs=True)
+        data = degibbs_step1(data, mask)
     data_fa = batched.gaussian_smooth(data, sigma=2.0) if FA_smooth == 'yes' else None
     vol = pipeline.recon_arrays(data, mask, np.asarray(TE_array, dtype=np.float64), TR, "X2", reg_matrix, FA_method,
                                 myelin_T2=myelin_T2, data_fa=data_fa, diagnostics=True, rois=ROIs, premasked=True,
