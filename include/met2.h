@@ -52,6 +52,8 @@ extern "C" {
 #define MET2_ST_ECHO_BAD_L 32u  /* MET2_T2_FLAG_ECHO_SPACE given with a non-diagonal L: voxel skipped */
 #define MET2_ST_NOT_PD 16u      /* BayesReg: beta*B + beta*x*K not positive definite (reference: LinAlgError) */
 #define MET2_ST_AT_BOUND 64u    /* met2_param_fit: a fitted T2 or the flip angle ends on its box (informational) */
+#define MET2_ST_MM_CAP 128u     /* met2_rician_fit: the MM iteration ran max_iter solves without meeting tol */
+#define MET2_ST_BAD_SIGMA 256u  /* met2_rician_fit: the noise sigma is NaN, +-Inf or negative (voxel skipped) */
 
 /* flip-angle search methods: run_real_data_script.py --FA_method */
 #define MET2_FA_BRUTE_FORCE 0
@@ -313,6 +315,24 @@ typedef struct met2_param_cfg {
 int met2_param_fit(const double* sig, const double* fa_deg, const double* fsol, const uint32_t* status_in, int64_t V,
                    const met2_param_cfg* cfg, const double* logT2, const uint8_t* comp, double* params, double* maps,
                    double* est_signal, double* sse, int32_t* iters, uint32_t* status, void* stream);
+
+/* Rician-likelihood spectrum fitting (no counterpart in the reference): majorize-minimize iterations of warm-started
+ * Tikhonov NNLS solves with modified data yt = y * I1/I0(y f / sn^2), started from the point fit.  Definition in
+ * csrc/met2_rician.cu; the NumPy restatement is tests/rician_oracle.py.
+ * Inputs are the point fit's: sig [V][nTE] raw signals, fa_index [V], lam [V] (any lam >= 0; the pipeline passes reg
+ * under MET2_T2_FLAG_REG_IS_LAMBDA), x0 [V][nT2] = fsol / sig[0] and status_in [V]; sigma [V] is the noise SD in raw
+ * signal units.  G, dicT, kband as for met2_t2_fit.  Outputs: x [V][nT2] (normalised spectra; met2_spatial_finish turns
+ * them into fsol / est_signal / maps), iters [V] int32 (MM solves run), status [V] = status_in plus MET2_ST_MM_CAP,
+ * MET2_ST_ITMAX and MET2_ST_BAD_SIGMA | MET2_ST_SKIPPED.  sigma = 0 reproduces the point fit (iters 0, x = x0).
+ * Gram-domain sizes (nT2 <= 128, nTE <= 64), V < 2^31, max_iter >= 1, tol finite and >= 0; V = 0 is a no-op; bad
+ * arguments return MET2_ERR_ARG before anything is enqueued.
+ * met2_bessel_ratio writes A(z) = I1(z) / I0(z) of the kernel's routine for n HOST values z to out (host memory) and
+ * returns n (MET2_ERR_ARG for n < 0 or a NULL pointer with n > 0). */
+int met2_rician_fit(const double* sig, const int32_t* fa_index, const double* lam, const double* sigma,
+                    const double* x0, const uint32_t* status_in, int64_t V, int nTE, int nT2, int nA, const double* G,
+                    const double* dicT, const double* kband, int max_iter, double tol, double* x, int32_t* iters,
+                    uint32_t* status, void* stream);
+int64_t met2_bessel_ratio(const double* z, int64_t n, double* out);
 
 /* Diagnostics */
 const char* met2_last_error(void);

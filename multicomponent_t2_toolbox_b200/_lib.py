@@ -76,6 +76,9 @@ SIGNATURES = {
     "met2_spatial_finish": (ctypes.c_int, [c_void_p] * 4 + [ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int]
                             + [c_void_p] * 7),
     "met2_param_fit": (ctypes.c_int, [c_void_p] * 4 + [ctypes.c_int64, ctypes.POINTER(ParamCfg)] + [c_void_p] * 9),
+    "met2_rician_fit": (ctypes.c_int, [c_void_p] * 6 + [ctypes.c_int64, ctypes.c_int, ctypes.c_int, ctypes.c_int]
+                        + [c_void_p] * 3 + [ctypes.c_int, ctypes.c_double] + [c_void_p] * 4),
+    "met2_bessel_ratio": (ctypes.c_int64, [c_void_p, ctypes.c_int64, c_void_p]),
     "met2_last_error": (ctypes.c_char_p, []),
     "met2_version": (ctypes.c_int, []),
     "met2_echo_rank": (ctypes.c_int, [ctypes.c_int]),

@@ -21,8 +21,11 @@ REG_METHOD_CODE = {"NNLS": 0, "T2SPARC": 1, "X2": 2, "L_curve": 3, "GCV": 4, "Ba
 
 ST_SKIPPED, ST_NONFINITE, ST_ITMAX, ST_SSE_ZERO, ST_NOT_PD = 1, 2, 4, 8, 16
 ST_AT_BOUND = 64
+ST_MM_CAP, ST_BAD_SIGMA = 128, 256    # met2_rician_fit
 # Levenberg-Marquardt settings of the three-pool parametric fit (csrc/met2_param.cu)
 PARAM_DEFAULTS = dict(mu0=1e-3, mu_max=1e16, ftol=1e-12, xtol=1e-10, max_iter=2000)
+# majorize-minimize settings of the Rician-likelihood fit (csrc/met2_rician.cu)
+RICIAN_DEFAULTS = dict(max_iter=200, tol=1e-9)
 REG_IS_LAMBDA, NO_NORMALISE, COLD_START, GCV_EVAL, FULL_START, GCV_GRID, ECHO_SPACE = 1, 2, 4, 8, 16, 32, 64   # MET2_T2_FLAG_*
 # Largest residual of the reduction (max_j |d_j - U C_j| / max_j |d_j| over the flip angles, measured by
 # met2_echo_basis) for which a rank of the reduced echo space is used.  24 (MET2_ECHO_RANK): the rounding of the
@@ -616,6 +619,58 @@ class Met2Plan:
                 _ptr(self.logT2), _ptr(self.comp), _ptr(out["fsol"]), _ptr(out["est_signal"]), _ptr(out["maps"]),
                 _stream()), "met2_spatial_finish")
         out["x"] = x
+        return out
+
+    # ------------------------------------------------------------------ Rician-likelihood fit
+    def rician_fit(self, sig, fa_index, lam, sigma, fsol, status, **cfg):
+        """Rician-likelihood spectra (definition in csrc/met2_rician.cu): majorize-minimize iterations of warm-started
+        Tikhonov NNLS solves with modified data, started from a point fit of this plan.  sig[V, nTE] is the signal the
+        point fit used, fa_index[V] its flip-angle indices, lam[V] its lambda (`t2_fit(..., flags=REG_IS_LAMBDA)["reg"]`),
+        fsol[V, nT2] its spectra and status[V] its status; sigma is the noise SD in the signal's units, a number or
+        one value per voxel.  cfg overrides RICIAN_DEFAULTS.  The solves run in the Gram domain, whichever kernels the
+        point fit ran.  Returns CUDA tensors fsol[V, nT2], est_signal[V, nTE] (the noiseless model D x sig[0]),
+        maps[V, 6], iters[V] (int32, MM solves run), status[V] (the point fit's plus MET2_ST_MM_CAP, MET2_ST_ITMAX and
+        MET2_ST_BAD_SIGMA | MET2_ST_SKIPPED) and x[V, nT2] (normalised spectra).  All work is enqueued on the current
+        stream."""
+        unknown = set(cfg) - set(RICIAN_DEFAULTS)
+        if unknown:
+            raise ValueError("unknown rician_fit settings %s" % sorted(unknown))
+        o = {**RICIAN_DEFAULTS, **cfg}
+        sig = self._signals(sig)
+        V = sig.shape[0]
+        dev = self.dev
+        fa_index = torch.as_tensor(fa_index).to(device=dev, dtype=torch.int32).contiguous()
+        lam = torch.as_tensor(lam).to(device=dev, dtype=torch.float64).contiguous()
+        sigma = torch.as_tensor(sigma, dtype=torch.float64).to(dev).reshape(-1)
+        if sigma.numel() == 1:
+            sigma = sigma.expand(V)
+        sigma = sigma.contiguous()
+        fsol = torch.as_tensor(fsol).to(device=dev, dtype=torch.float64)
+        status = torch.as_tensor(status).to(device=dev, dtype=torch.int32).contiguous()
+        if (fa_index.shape != (V,) or lam.shape != (V,) or sigma.shape != (V,) or tuple(fsol.shape) != (V, self.npc)
+                or status.shape != (V,)):
+            raise ValueError("rician_fit: sig[V, nTE], fa_index[V], lam[V], sigma (a number or [V]), fsol[V, nT2] and "
+                             "status[V] expected")
+        out = dict(fsol=torch.empty((V, self.npc), dtype=torch.float64, device=dev),
+                   est_signal=torch.empty((V, self.nTE), dtype=torch.float64, device=dev),
+                   maps=torch.empty((V, 6), dtype=torch.float64, device=dev),
+                   iters=torch.empty(V, dtype=torch.int32, device=dev),
+                   status=torch.empty(V, dtype=torch.int32, device=dev),
+                   x=torch.empty((V, self.npc), dtype=torch.float64, device=dev))
+        if V == 0:
+            return out
+        hr = self.dict_hr
+        with torch.cuda.device(dev):
+            fitted = (status & ST_SKIPPED) == 0
+            x0 = torch.where(fitted[:, None], fsol / sig[:, :1], 0.0).contiguous()
+            _lib.check(self.lib.met2_rician_fit(
+                _ptr(sig), _ptr(fa_index), _ptr(lam), _ptr(sigma), _ptr(x0), _ptr(status), V, self.nTE, self.npc,
+                hr.nA, _ptr(hr.G), _ptr(hr.dicT), _ptr(self.kband), int(o["max_iter"]), float(o["tol"]), _ptr(out["x"]),
+                _ptr(out["iters"]), _ptr(out["status"]), _stream()), "met2_rician_fit")
+            _lib.check(self.lib.met2_spatial_finish(
+                _ptr(sig), _ptr(fa_index), _ptr(out["status"]), _ptr(out["x"]), V, self.nTE, self.npc, hr.nA,
+                _ptr(hr.dicT), _ptr(self.logT2), _ptr(self.comp), _ptr(out["fsol"]), _ptr(out["est_signal"]),
+                _ptr(out["maps"]), _stream()), "met2_spatial_finish")
         return out
 
     # ------------------------------------------------------------------ three-pool parametric fit

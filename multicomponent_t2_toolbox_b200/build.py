@@ -9,7 +9,7 @@ LIB_PATH = os.path.join(PKG_DIR, "libmet2.so")
 SOURCES = ["met2_api.cu", "met2_epg.cu", "met2_basis.cu", "met2_smooth.cu", "met2_aux.cu", "met2_fa.cu", "met2_t2.cu", "met2_t2_m_nnls.cu", "met2_t2_m_t2sparc.cu",
            "met2_t2_m_x2.cu", "met2_t2_m_lcurve.cu", "met2_t2_m_bayesreg.cu", "met2_t2_m_gcv.cu", "met2_t2_echo_r16.cu", "met2_t2_echo_r24.cu",
            "met2_t2_echo_reg_r16.cu", "met2_t2_echo_reg_r24.cu", "met2_tv.cu", "met2_mppca.cu", "met2_degibbs.cu", "met2_boot.cu",
-           "met2_spatial.cu", "met2_param.cu"]
+           "met2_spatial.cu", "met2_param.cu", "met2_rician.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     # no implicit FMA contraction: Brent / corner-selection comparisons must round like the reference's separate

@@ -73,7 +73,7 @@ def degibbs_step1(data, mask):
 
 def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR, reg_method, reg_matrix, denoise,
                      FA_method, FA_smooth, myelin_T2, num_cores, n_bootstrap=0, bootstrap_seed=0, spatial_mu=0.0,
-                     spatial_sweeps=10, parametric=False, degibbs=False):
+                     spatial_sweeps=10, parametric=False, degibbs=False, rician_sigma=None):
     """Same arguments as the reference.  `num_cores` selects the number of GPUs (-1 = all visible; see
     n_gpus_from_num_cores): the masked voxels of the volume are spread over them by pipeline.MultiGpuFit.
 
@@ -95,7 +95,17 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
 
     degibbs=True (not in the reference, reached from Python only): after Step 1 (denoising first, as MRtrix advises:
     unringing correlates the noise), every axial slice of every echo is unrung on the GPU (degibbs_step1, the local
-    subvoxel-shift method of MRtrix3's mrdegibbs), then masked again with negatives clipped to 0.  No file is added."""
+    subvoxel-shift method of MRtrix3's mrdegibbs), then masked again with negatives clipped to 0.  No file is added.
+
+    rician_sigma (not in the reference, reached from Python only): also the Rician-likelihood fit started from each
+    voxel's point fit (pipeline.recon_arrays), with the noise SD rician_sigma in the data's units: a number, an
+    [nx, ny, nz] array, or 'MPPCA' for the sigma map of batched.mppca_denoise on the masked data (the denoised data are
+    discarded; the map is written as MPPCA_sigma.nii.gz).  Written as MWF_rician, IEWF_rician, FWF_rician, T2_M_rician,
+    T2_IE_rician, TWC_rician, fsol_4D_rician, Est_Signal_rician and rician_iters (.nii.gz) beside the unchanged ten
+    outputs.  The likelihood describes raw magnitude data, so it needs denoise='None' and degibbs=False."""
+    if rician_sigma is not None and (denoise != 'None' or degibbs):
+        raise ValueError("rician_sigma describes the noise of the raw magnitude data: it needs denoise='None' and "
+                         "degibbs=False")
     n_gpus = n_gpus_from_num_cores(num_cores)
     warm = threading.Thread(target=_warm_gpus, args=(n_gpus,), daemon=True)   # CUDA contexts + libmet2.so while the files load
     warm.start()
@@ -127,6 +137,12 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
         print('Step #1: Denoising using MP-PCA:')
         den, mppca_sigma, _ = batched.mppca_denoise(data, mask)
         data, mppca_sigma = den.cpu().numpy(), mppca_sigma.cpu().numpy()
+    if isinstance(rician_sigma, str):
+        if rician_sigma != 'MPPCA':
+            raise ValueError("rician_sigma must be a number, an array or 'MPPCA'")
+        print('Noise map for the Rician fit: MP-PCA')
+        _, mppca_sigma, _ = batched.mppca_denoise(data, mask)
+        rician_sigma = mppca_sigma = mppca_sigma.cpu().numpy()
     if degibbs:
         print('Step #1b: Gibbs-ringing removal:')
         data = degibbs_step1(data, mask)
@@ -139,12 +155,14 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
     vol = pipeline.recon_arrays(data, mask, np.asarray(TE_array, dtype=np.float64), TR, reg_method, reg_matrix,
                                 FA_method, myelin_T2=myelin_T2, data_fa=data_fa, diagnostics=True, premasked=True,
                                 n_gpus=n_gpus, n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed,
-                                spatial_mu=spatial_mu, spatial_sweeps=spatial_sweeps, parametric=parametric)
+                                spatial_mu=spatial_mu, spatial_sweeps=spatial_sweeps, parametric=parametric,
+                                rician_sigma=rician_sigma)
     print('Step #4: Estimation of quantitative metrics')
     # the ten volumes (motor...:474-503) are written concurrently, largest first: every writer deflates with all cores
     # (nifti_io), but the eight 3-D maps are too small to keep them busy one at a time (2.2 s -> 1.2 s on 8 cores)
     names = OUTPUTS + (BOOTSTRAP_OUTPUTS if n_bootstrap > 0 else ()) + \
-        (tuple(pipeline.PARAM_VOLUMES) if parametric else ())
+        (tuple(pipeline.PARAM_VOLUMES) if parametric else ()) + \
+        (tuple(pipeline.RICIAN_VOLUMES) if rician_sigma is not None else ())
     order = sorted(names, key=lambda name: -vol[name].size)
     with ThreadPoolExecutor(max_workers=4) as pool:
         list(pool.map(lambda name: nifti_io.save(vol[name], join(name + '.nii.gz'), affine=img.affine), order))

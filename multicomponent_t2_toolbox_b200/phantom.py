@@ -102,7 +102,8 @@ def _epg_signal_batch_gpu(n_echoes, tau, T1, T2, alpha_deg):
 
 def make_phantom(shape=(16, 16, 4), n_echoes=32, tau=10.0, TR=1000.0, T1=1000.0, seed=1, fa_mode="uniform",
                  snr_range=(50.0, 150.0), Km=1000.0, mask_mode="full", backend="numpy"):
-    """Return dict(data[nx,ny,nz,nTE], mask[nx,ny,nz], truth={...}).
+    """Return dict(data[nx,ny,nz,nTE], mask[nx,ny,nz], truth={...}); truth["sigma"] is the SD of the Rician noise in
+    the data's units.
 
     fa_mode: "uniform" -> FA ~ U(100, 180) per voxel (config 1); "b1" -> smooth B1 field (configs 2, 3, 5).
     mask_mode: "full" -> all ones; "ellipsoid" -> ~52 % fill, exercises the gather/scatter of masked voxels.
@@ -146,7 +147,7 @@ def make_phantom(shape=(16, 16, 4), n_echoes=32, tau=10.0, TR=1000.0, T1=1000.0,
         raise ValueError(mask_mode)
     data = noisy.reshape(nx, ny, nz, n_echoes) * mask[..., None]
     truth = dict(mwf=mwf.reshape(shape), fwf=fwf.reshape(shape), iewf=iewf.reshape(shape), t2m=t2m.reshape(shape),
-                 t2ie=t2ie.reshape(shape), fa=fa.reshape(shape), snr=snr.reshape(shape))
+                 t2ie=t2ie.reshape(shape), fa=fa.reshape(shape), snr=snr.reshape(shape), sigma=sigma.reshape(shape))
     return dict(data=data, mask=mask, truth=truth, TE_array=tau * np.arange(1, n_echoes + 1), TR=TR)
 
 

@@ -95,7 +95,8 @@ def spatial_neighbours(flat, shape, fitted):
 
 
 # The per-voxel outputs of the stages: name, trailing shape (ints and Met2Plan attributes), dtype, and the stage that
-# produces it.  "fa" always runs, "t2" unless fa_only, "bootstrap" when n_bootstrap > 0, "parametric" when parametric.
+# produces it.  "fa" always runs, "t2" unless fa_only, "bootstrap" when n_bootstrap > 0, "parametric" when parametric,
+# "rician" when a noise sigma is given.
 VOXEL_OUTPUTS = (
     ("fa_index", (), torch.int32, "fa"), ("fa_deg", (), torch.float64, "fa"), ("km", (), torch.float64, "fa"),
     ("fa_status", (), torch.int32, "fa"),
@@ -104,13 +105,21 @@ VOXEL_OUTPUTS = (
     ("boot_stats", (6, 4), torch.float64, "bootstrap"), ("boot_n_valid", (), torch.int32, "bootstrap"),
     ("param_params", (7,), torch.float64, "parametric"), ("param_maps", (6,), torch.float64, "parametric"),
     ("param_est_signal", ("nTE",), torch.float64, "parametric"), ("param_sse", (), torch.float64, "parametric"),
-    ("param_iters", (), torch.int32, "parametric"), ("param_status", (), torch.int32, "parametric"))
+    ("param_iters", (), torch.int32, "parametric"), ("param_status", (), torch.int32, "parametric"),
+    ("rician_fsol", ("npc",), torch.float64, "rician"), ("rician_est_signal", ("nTE",), torch.float64, "rician"),
+    ("rician_maps", (6,), torch.float64, "rician"), ("rician_iters", (), torch.int32, "rician"),
+    ("rician_status", (), torch.int32, "rician"))
 
 # the volumes of the three-pool parametric fit: name -> (output, column)
 PARAM_VOLUMES = {"MWF_3pool": ("param_maps", 0), "IEWF_3pool": ("param_maps", 1), "FWF_3pool": ("param_maps", 2),
                  "T2_M_3pool": ("param_maps", 3), "T2_IE_3pool": ("param_maps", 4), "T2_FW_3pool": ("param_params", 5),
                  "FA_3pool": ("param_params", 6), "TWC_3pool": ("param_maps", 5), "SSE_3pool": ("param_sse", None),
                  "Est_Signal_3pool": ("param_est_signal", None)}
+
+# the volumes of the Rician-likelihood fit: name -> (output, column)
+RICIAN_VOLUMES = {**{name + "_rician": ("rician_maps", i) for i, name in enumerate(MAP_NAMES)},
+                  "fsol_4D_rician": ("rician_fsol", None), "Est_Signal_rician": ("rician_est_signal", None),
+                  "rician_iters": ("rician_iters", None)}
 
 # The volumes of `recon_arrays`: name, per-voxel output, column (None: all of it) and dtype.  A volume is returned when
 # its per-voxel output was computed.
@@ -120,7 +129,9 @@ VOLUMES = (("FA", "fa_deg", None, np.float64), ("FA_index", "fa_index", None, np
            ("Est_Signal", "est_signal", None, np.float64), ("status", "status", None, np.int32),
            *((name + "_bootstrap", "boot_stats", i, np.float64) for i, name in enumerate(MAP_NAMES)),
            ("bootstrap_n_valid", "boot_n_valid", None, np.int32),
-           *((name, key, col, np.float64) for name, (key, col) in PARAM_VOLUMES.items()))
+           *((name, key, col, np.float64) for name, (key, col) in PARAM_VOLUMES.items()),
+           *((name, key, col, np.int32 if key == "rician_iters" else np.float64)
+             for name, (key, col) in RICIAN_VOLUMES.items()))
 
 
 def _fa_stage(plan, s):
@@ -159,11 +170,19 @@ def _param_stage(plan, s):
     return {"param_" + k: v for k, v in pf.items()}
 
 
-def _stages(fa_only=False, n_bootstrap=0, bootstrap_seed=0, parametric=False):
+def _rician_stage(plan, s):
+    """`Met2Plan.rician_fit` started from the point fit, with lambda from a second `t2_fit` under REG_IS_LAMBDA (the
+    point fit's reg is k_est for X2) and the per-voxel noise sigma s["sigma"]."""
+    lam = plan.t2_fit(s["sig"], s["fa"]["fa_index"], flags=batched.REG_IS_LAMBDA)["reg"]
+    rf = plan.rician_fit(s["sig"], s["fa"]["fa_index"], lam, s["sigma"], s["t2"]["fsol"], s["t2"]["status"])
+    return {"rician_" + k: rf[k] for k in ("fsol", "est_signal", "maps", "iters", "status")}
+
+
+def _stages(fa_only=False, n_bootstrap=0, bootstrap_seed=0, parametric=False, rician=False):
     """The per-voxel stages in order, as (name, stage).  A stage takes (plan, s), s: the device state of one set of
-    voxels (sig, sig_fa, ranges: their (lo, hi) in the whole voxel list, and the fa / t2 results, reused as `out=`), and
-    returns its VOXEL_OUTPUTS as CUDA tensors, enqueued on the current stream.  Bootstrap and the parametric fit start
-    from the point fit."""
+    voxels (sig, sig_fa, sigma for the Rician fit, ranges: their (lo, hi) in the whole voxel list, and the fa / t2
+    results, reused as `out=`), and returns its VOXEL_OUTPUTS as CUDA tensors, enqueued on the current stream.
+    Bootstrap, the parametric and the Rician fit start from the point fit."""
     stages = [("fa", _fa_stage)]
     if not fa_only:
         stages.append(("t2", _t2_stage))
@@ -171,6 +190,8 @@ def _stages(fa_only=False, n_bootstrap=0, bootstrap_seed=0, parametric=False):
             stages.append(("bootstrap", lambda plan, s: _bootstrap_stage(plan, s, n_bootstrap, bootstrap_seed)))
         if parametric:
             stages.append(("parametric", _param_stage))
+        if rician:
+            stages.append(("rician", _rician_stage))
     return stages
 
 
@@ -180,13 +201,15 @@ def _outputs(stages):
     return [o for o in VOXEL_OUTPUTS if o[3] in ran]
 
 
-def host_buffers(plan, V, pinned=True, n_bootstrap=0, parametric=False):
+def host_buffers(plan, V, pinned=True, n_bootstrap=0, parametric=False, rician=False):
     """Host (pinned) arrays for the outputs of `fit_voxels` / `MultiGpuFit.fit` of V voxels: the per-voxel outputs of
-    the point fit, plus those of the bootstrap (n_bootstrap > 0) and of the parametric fit, and fsol_sum[npc]."""
+    the point fit, plus those of the bootstrap (n_bootstrap > 0), of the parametric fit and of the Rician fit, and
+    fsol_sum[npc]."""
     pin = pinned and torch.cuda.is_available()
     bufs = {name: torch.empty((V,) + tuple(getattr(plan, n) if isinstance(n, str) else n for n in shape), dtype=dtype,
                               pin_memory=pin)
-            for name, shape, dtype, _ in _outputs(_stages(n_bootstrap=n_bootstrap, parametric=parametric))}
+            for name, shape, dtype, _ in _outputs(_stages(n_bootstrap=n_bootstrap, parametric=parametric,
+                                                            rician=rician))}
     bufs["fsol_sum"] = torch.empty(plan.npc, dtype=torch.float64, pin_memory=pin)
     return bufs
 
@@ -243,12 +266,13 @@ class MultiGpuFit:
                                 range(n)))
         return cls(plans, chunks_per_device)
 
-    def fit(self, sig, sig_fa=None, out=None, n_bootstrap=0, bootstrap_seed=0, parametric=False):
+    def fit(self, sig, sig_fa=None, out=None, n_bootstrap=0, bootstrap_seed=0, parametric=False, sigma=None):
         """sig[V, nTE] (+ sig_fa for the FA stage): host tensors / arrays, pinned for full-speed DMA.  `out`: dict of
         host tensors as from `host_buffers` (what it lacks is allocated).  Returns dict of numpy views of `out`.
         n_bootstrap > 0: also the per-voxel bootstrap of the maps (keys boot_*), each device over its own chunks with
         voxel_offset = the chunk's start, so the result does not depend on the device count.  parametric: also the
-        three-pool parametric fit (keys param_*).
+        three-pool parametric fit (keys param_*).  sigma[V] (host, raw signal units): also the Rician-likelihood fit
+        (keys rician_*); each device copies its chunks of it beside sig.
 
         Everything is ENQUEUED from this one thread, phase by phase over the devices (copies in, then each stage of
         `_stages`, then copies out: ~0.1 ms of host time per device and phase, all asynchronous), then the streams are
@@ -258,11 +282,15 @@ class MultiGpuFit:
         sig = torch.as_tensor(sig)
         if sig_fa is not None:
             sig_fa = torch.as_tensor(sig_fa)
+        rician = sigma is not None
+        if rician:
+            sigma = torch.as_tensor(sigma, dtype=torch.float64)
         V = sig.shape[0]
-        stages = _stages(False, n_bootstrap, bootstrap_seed, parametric)
+        stages = _stages(False, n_bootstrap, bootstrap_seed, parametric, rician)
         names = [name for name, *_ in _outputs(stages)]
         if out is None or not all(k in out for k in names):
-            out = {**host_buffers(self.plans[0], V, n_bootstrap=n_bootstrap, parametric=parametric), **(out or {})}
+            out = {**host_buffers(self.plans[0], V, n_bootstrap=n_bootstrap, parametric=parametric, rician=rician),
+                   **(out or {})}
         nd = len(self.plans)
         parts = chunk_deal(V, nd, self.chunks_per_device)
         trace = [dict() for _ in self.plans] if os.environ.get("MET2_MULTI_TRACE") else None
@@ -276,12 +304,13 @@ class MultiGpuFit:
         for d in live:                                   # ---- phase 1: host -> device
             plan = self.plans[d]
             Vd = sum(hi - lo for lo, hi in parts[d])
-            key = (d, Vd, sig_fa is not None)
+            key = (d, Vd, sig_fa is not None, rician)
             b = self._bufs.get(key)
             with torch.cuda.device(plan.dev), torch.cuda.stream(self.streams[d]):
                 if b is None:
                     d_sig = torch.empty((Vd, plan.nTE), dtype=torch.float64, device=plan.dev)
-                    b = dict(sig=d_sig, sig_fa=d_sig if sig_fa is None else torch.empty_like(d_sig), fa=None, t2=None)
+                    b = dict(sig=d_sig, sig_fa=d_sig if sig_fa is None else torch.empty_like(d_sig), fa=None, t2=None,
+                             sigma=torch.empty(Vd, dtype=torch.float64, device=plan.dev) if rician else None)
                     self._bufs = {k: v for k, v in self._bufs.items() if k[0] != d}
                     self._bufs[key] = b
                 b["ranges"] = parts[d]
@@ -290,6 +319,8 @@ class MultiGpuFit:
                     b["sig"][o:o + hi - lo].copy_(sig[lo:hi], non_blocking=True)
                     if sig_fa is not None:
                         b["sig_fa"][o:o + hi - lo].copy_(sig_fa[lo:hi], non_blocking=True)
+                    if rician:
+                        b["sigma"][o:o + hi - lo].copy_(sigma[lo:hi], non_blocking=True)
                     o += hi - lo
             bufs[d] = b
             mark(d, "h2d_enqueued")
@@ -319,7 +350,7 @@ class MultiGpuFit:
 
 
 def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, fa_only=False, n_bootstrap=0,
-               bootstrap_seed=0, voxel_offset=0, spatial=None, parametric=False):
+               bootstrap_seed=0, voxel_offset=0, spatial=None, parametric=False, sigma=None):
     """Steps 2-4 on a list of voxels given as host array sig[V, nTE]; returns host arrays (dict).
     in_mask[V] (optional): also return the mean-spectrum diagnostics of motor...:375-403 over the voxels with
     in_mask == 1 (key "diagnostics").  roi = (labels[V], values) (optional): also the ROI-based estimates of
@@ -327,8 +358,9 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
     with that many replicates (keys boot_*); voxel_offset: the position of sig[0] in the whole voxel list (a torchrun
     rank's slab start).  spatial = (flat, shape, mu, n_sweeps) (optional): the voxels are the masked voxels flat[V] of
     a volume of `shape`, and fsol / est_signal / maps / status are those of the spatially regularised fit with coupling
-    weight mu.  parametric: also the three-pool parametric fit started from the point fit (keys param_*).  fa_only:
-    only the FA stage's outputs."""
+    weight mu.  parametric: also the three-pool parametric fit started from the point fit (keys param_*).  sigma[V]
+    (raw signal units): also the Rician-likelihood fit started from the point fit (keys rician_*).  fa_only: only the
+    FA stage's outputs."""
     dev = plan.dev
     V = sig.shape[0]
     with torch.cuda.device(dev):
@@ -339,8 +371,9 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
             d_sig_fa = sig_fa.to(dev)
         else:
             d_sig_fa = torch.as_tensor(sig_fa).to(dev, non_blocking=True)
-        s = dict(sig=d_sig, sig_fa=d_sig_fa, ranges=[(voxel_offset, voxel_offset + V)], fa=None, t2=None)
-        stages = _stages(fa_only, n_bootstrap, bootstrap_seed, parametric)
+        d_sigma = None if sigma is None else torch.as_tensor(sigma, dtype=torch.float64).to(dev, non_blocking=True)
+        s = dict(sig=d_sig, sig_fa=d_sig_fa, sigma=d_sigma, ranges=[(voxel_offset, voxel_offset + V)], fa=None, t2=None)
+        stages = _stages(fa_only, n_bootstrap, bootstrap_seed, parametric, sigma is not None)
         out = {}
         for _, stage in stages:
             out.update(stage(plan, s))
@@ -367,7 +400,7 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
 def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, myelin_T2=40.0, data_fa=None, plan=None,
                  npc=None, n_alphas=None, device=None, rank=0, world_size=1, diagnostics=False, rois=None,
                  premasked=False, fa_only=False, n_gpus=1, n_bootstrap=0, bootstrap_seed=0, spatial_mu=0.0,
-                 spatial_sweeps=10, parametric=False):
+                 spatial_sweeps=10, parametric=False, rician_sigma=None):
     """Steps 2-4 of motor_recon_met2 on in-memory arrays.  Returns the ten output volumes (plus FA_index) as numpy.
 
     n_bootstrap > 0: also the per-voxel bootstrap uncertainty of the six maps with that many replicates per voxel
@@ -389,6 +422,13 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
     unchanged.  Per voxel, so it runs on every GPU and rank like the point fit; it cannot be combined with spatial_mu,
     since either spectrum could then start it.
 
+    rician_sigma (a number or an [nx, ny, nz] array, the noise SD in the data's units): also the Rician-likelihood fit
+    (`batched.Met2Plan.rician_fit`, definition in csrc/met2_rician.cu) started from each voxel's point fit, with the
+    lambda that fit selected: volumes MWF_rician, IEWF_rician, FWF_rician, T2_M_rician, T2_IE_rician, TWC_rician,
+    fsol_4D_rician, Est_Signal_rician and rician_iters (int32, MM solves run); zero outside the mask and where the
+    point fit skipped the voxel or sigma is not finite and >= 0.  The ten standard volumes are unchanged.  Per voxel,
+    so it runs on every GPU and rank like the point fit; it cannot be combined with spatial_mu.
+
     n_gpus != 1 (None / -1 = all visible GPUs): the voxel list of this ONE volume is spread over the GPUs of the node by
     `MultiGpuFit` (host in -> host out, no collective).  With world_size > 1 (one process per GPU under torchrun) only
     this rank's slab of the masked voxels is fitted and the other voxels are left zero; the caller combines the ranks
@@ -405,6 +445,9 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
     if spatial_mu > 0 and parametric:
         raise ValueError("spatial_mu > 0 cannot be combined with parametric: it is ambiguous which spectrum starts the "
                          "parametric fit")
+    if rician_sigma is not None and spatial_mu > 0:
+        raise ValueError("spatial_mu > 0 cannot be combined with rician_sigma: it is ambiguous which spectrum starts the "
+                         "Rician fit")
     data = np.asarray(data, dtype=np.float64)
     nx, ny, nz, nt = data.shape
     TE_array = np.asarray(TE_array, dtype=np.float64)
@@ -421,6 +464,9 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
             plan = batched.Met2Plan(*plan_args, device=device, **plan_kw)
     flat, sig = masked_voxel_list(data, mask, premasked)
     lo, hi = slab_bounds(len(flat), rank, world_size)
+    sigma = None
+    if rician_sigma is not None and not fa_only:
+        sigma = np.broadcast_to(np.asarray(rician_sigma, dtype=np.float64), (nx, ny, nz)).reshape(-1)[flat[lo:hi]]
     sig_fa = None
     if data_fa is not None:
         if isinstance(data_fa, torch.Tensor):
@@ -451,7 +497,12 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
         if sig_fa is not None:
             pin_fa = torch.empty((V, nt), dtype=torch.float64).pin_memory()
             pin_fa.copy_(sig_fa if isinstance(sig_fa, torch.Tensor) else torch.as_tensor(sig_fa))
-        res = multi.fit(pin, pin_fa, n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed, parametric=parametric)
+        pin_sigma = None
+        if sigma is not None:
+            pin_sigma = torch.empty(V, dtype=torch.float64).pin_memory()
+            pin_sigma.numpy()[:] = sigma
+        res = multi.fit(pin, pin_fa, n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed, parametric=parametric,
+                        sigma=pin_sigma)
         if V > 0 and (in_mask is not None or roi is not None or spatial is not None):
             # these couple the voxels of every device's chunks: on the first device, from the gathered point fit
             with torch.cuda.device(plan.dev):
@@ -463,7 +514,7 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
     else:
         res = fit_voxels(plan, sig[lo:hi], sig_fa, in_mask=in_mask, roi=roi, fa_only=fa_only,
                          n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed, voxel_offset=lo, spatial=spatial,
-                         parametric=parametric)
+                         parametric=parametric, sigma=sigma)
     sel = flat[lo:hi]
     vol = {}
     for name, key, col, dtype in VOLUMES:
