@@ -37,6 +37,7 @@ extern "C" {
 #define MET2_MAX_NT2 128 /* T2 bins (reference: 60, or 96 for T2SPARC; config 4 uses 100) */
 #define MET2_MAX_NTE 64  /* echoes (reference data: 32; config 4 uses 48) */
 #define MET2_MAX_KNOTS 32
+#define MET2_MAX_PROFILE 512 /* positions of a slice profile (met2_epg_dictionary_profile) */
 #define MET2_MAX_LAMBDAS 64
 #define MET2_ECHO_RANK 24       /* rows of the reduced echo space (met2_echo_basis, met2_t2_fit_echo): exact to the rounding
                                    of the dictionary's own entries for every protocol met so far */
@@ -126,6 +127,25 @@ int met2_epg_dictionary(const double* alphas_deg, int nA, const double* T2s, con
  * Same kernel as the dictionary; used by the synthetic phantom generator (epg/epg.py:64 epg_signal). */
 int met2_epg_signals(const double* alphas_deg, const double* T2s, const double* T1s, int64_t N, int nTE, double tau_ms,
                      double* sig, void* stream);
+
+/* Slice-profile-integrated EPG dictionary for 2-D multi-slice data (no counterpart in the reference; definition in
+ * csrc/met2_epg.cu, DESIGN §10g).  A slice profile is K positions with excitation scale x[k], refocusing scale r[k]
+ * and weight w[k] (HOST arrays [K], checked before anything is enqueued; the caller normalises sum w = 1):
+ *   dic[a][e][j] = (1 - exp(-TR/T1_j)) * sum_{k = 0..K-1 in order} w[k] * EPG_e(T2_j, T1_j, refocusing alpha_a r[k],
+ *                                                                              excitation (alpha_a / 2) x[k])
+ * with EPG_e the recurrence of met2_epg_dictionary; alpha_a stays the nominal angle at the slice centre.  Layouts and
+ * size limits of met2_epg_dictionary; K = 1 with x = r = w = 1 gives its output bit for bit.  1 <= K <=
+ * MET2_MAX_PROFILE and every x, r, w finite and >= 0, else MET2_ERR_ARG before anything is enqueued. */
+int met2_epg_dictionary_profile(const double* alphas_deg, int nA, const double* T2s, const double* T1s, int nT2,
+                                int nTE, double tau_ms, double TR_ms, const double* x, const double* r, const double* w,
+                                int K, double* dic, double* dicT, void* stream);
+
+/* Profile-integrated curves for arbitrary (alpha, T2, T1) triples: sig[N][nTE] without the (1-exp(-TR/T1)) factor,
+ * like met2_epg_signals (the synthetic phantom generator).  Same profile arguments as met2_epg_dictionary_profile;
+ * N < 2^31. */
+int met2_epg_signals_profile(const double* alphas_deg, const double* T2s, const double* T1s, int64_t N, int nTE,
+                             double tau_ms, const double* x, const double* r, const double* w, int K, double* sig,
+                             void* stream);
 
 /* Gram tables of the dictionary, G[a] = D_a^T D_a  ([nA][nT2][nT2]), and the 5-band form of K = L^T L
  * (kband[10][nT2]: rows 0..4 kband[d][c] = K[c+d-2][c], rows 5..9 the row-band form of L itself, kband[5+d][r] = L[r][r+d-2]) for the Tikhonov term of algorithms.py:262-269 (A = [D; sqrt(lambda) L]).

@@ -39,6 +39,12 @@ SIGNATURES = {
                                            ctypes.c_double, ctypes.c_double, c_void_p, c_void_p, c_void_p]),
     "met2_epg_signals": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_double,
                                         c_void_p, c_void_p]),
+    "met2_epg_dictionary_profile": (ctypes.c_int, [c_void_p, ctypes.c_int, c_void_p, c_void_p, ctypes.c_int,
+                                                   ctypes.c_int, ctypes.c_double, ctypes.c_double, c_void_p, c_void_p,
+                                                   c_void_p, ctypes.c_int, c_void_p, c_void_p, c_void_p]),
+    "met2_epg_signals_profile": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, ctypes.c_int64, ctypes.c_int,
+                                                ctypes.c_double, c_void_p, c_void_p, c_void_p, ctypes.c_int, c_void_p,
+                                                c_void_p]),
     "met2_gram_tables": (ctypes.c_int, [c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_int, c_void_p, c_void_p, c_void_p,
                                         c_void_p, c_void_p]),
     "met2_fa_workspace_bytes": (ctypes.c_int64, [ctypes.c_int64, ctypes.POINTER(FaCfg)]),

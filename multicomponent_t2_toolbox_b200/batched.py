@@ -243,10 +243,13 @@ def segment_means(sig, fa_index, labels, n_seg, dictionary):
 
 
 class Dictionary:
-    """Device EPG dictionary of one angle grid: dic [nA][nTE][nT2], dicT [nA][nT2][nTE], G [nA][nT2][nT2]."""
+    """Device EPG dictionary of one angle grid: dic [nA][nTE][nT2], dicT [nA][nT2][nTE], G [nA][nT2][nT2].
+    profile = (x, r, w) (`grids.slice_profile` or the caller's own): the slice-profile-integrated dictionary of 2-D
+    multi-slice data (met2_epg_dictionary_profile, DESIGN §10g) instead of the single-angle one; w is normalised here."""
 
-    def __init__(self, alphas, T2s, T1s, n_echoes, tau, TR, dev):
+    def __init__(self, alphas, T2s, T1s, n_echoes, tau, TR, dev, profile=None):
         lib = _lib.load()
+        self.profile = None if profile is None else grids.as_slice_profile(profile)
         self.alphas_host = np.ascontiguousarray(alphas, dtype=np.float64)
         self.nA, self.nT2, self.nTE = len(self.alphas_host), len(T2s), int(n_echoes)
         self.alphas = _dev_f64(self.alphas_host, dev)
@@ -256,9 +259,15 @@ class Dictionary:
         self.dicT = torch.empty((self.nA, self.nT2, self.nTE), dtype=torch.float64, device=dev)
         self.G = torch.empty((self.nA, self.nT2, self.nT2), dtype=torch.float64, device=dev)
         with torch.cuda.device(dev):
-            _lib.check(lib.met2_epg_dictionary(_ptr(self.alphas), self.nA, _ptr(t2), _ptr(t1), self.nT2, self.nTE,
-                                               float(tau), float(TR), _ptr(self.dic), _ptr(self.dicT), _stream()),
-                       "met2_epg_dictionary")
+            if self.profile is None:
+                _lib.check(lib.met2_epg_dictionary(_ptr(self.alphas), self.nA, _ptr(t2), _ptr(t1), self.nT2, self.nTE,
+                                                   float(tau), float(TR), _ptr(self.dic), _ptr(self.dicT), _stream()),
+                           "met2_epg_dictionary")
+            else:
+                x, r, w = (a.ctypes.data_as(ctypes.c_void_p) for a in self.profile)    # host arrays
+                _lib.check(lib.met2_epg_dictionary_profile(
+                    _ptr(self.alphas), self.nA, _ptr(t2), _ptr(t1), self.nT2, self.nTE, float(tau), float(TR), x, r, w,
+                    len(self.profile[2]), _ptr(self.dic), _ptr(self.dicT), _stream()), "met2_epg_dictionary_profile")
             _lib.check(lib.met2_gram_tables(_ptr(self.dic), self.nA, self.nTE, self.nT2, None, _ptr(self.G), None, None,
                                             _stream()), "met2_gram_tables")
 
@@ -337,10 +346,13 @@ class Met2Plan:
     def __init__(self, n_echoes, tau, TR, reg_method="X2", reg_matrix="I", FA_method="spline", myelin_T2=40.0,
                  npc=None, n_alphas=None, T1=1000.0, device=None, lambda_reg=None, Laplac=None, Dic_3D=None,
                  Dic_3D_LR=None, alpha_values=None, alpha_values_spline=None, T2s=None, t2_flags=0, echo_space=True,
-                 echo_ranks=None):
+                 echo_ranks=None, slice_profile=None):
         """Tables for one reconstruction set-up.  By default everything is built like motor...:204-277 (EPG dictionary
         on the GPU); `Dic_3D` (+ `Dic_3D_LR`, `alpha_values`, `alpha_values_spline`, `T2s`, `Laplac`) lets a caller bring
-        its own dictionary in the reference layout [nTE, nT2, nA] — used by the drop-in row workers and per-voxel API."""
+        its own dictionary in the reference layout [nTE, nT2, nA] — used by the drop-in row workers and per-voxel API.
+        slice_profile = (x, r, w) (`grids.slice_profile`): both the fine and the coarse (spline-knot) dictionaries are
+        the slice-profile-integrated ones of 2-D multi-slice data (`Dictionary(profile=...)`, DESIGN §10g); the angle
+        grids keep their meaning (the nominal angle at the slice centre).  The parametric fit does not take a profile."""
         if reg_method not in REG_METHOD_CODE:
             raise ValueError("unknown reg_method %r" % (reg_method,))
         if FA_method not in FA_METHOD_CODE:
@@ -356,6 +368,9 @@ class Met2Plan:
         # ECHO_TAIL_MAX; (24,) pins the rank that is exact to the rounding of the dictionary's entries)
         self.echo_ranks = None if echo_ranks is None else tuple(int(r) for r in echo_ranks)
         self.nTE, self.tau, self.TR = int(n_echoes), float(tau), float(TR)
+        if slice_profile is not None and Dic_3D is not None:
+            raise ValueError("slice_profile builds the dictionary: it cannot be combined with Dic_3D")
+        self.slice_profile = None if slice_profile is None else grids.as_slice_profile(slice_profile)
         if Dic_3D is not None:
             Dic_3D = np.asarray(Dic_3D, dtype=np.float64)
             if Dic_3D.ndim == 2:
@@ -395,9 +410,11 @@ class Met2Plan:
                     self.dict_lr = Dictionary.from_reference_layout(Dic_3D_LR, self.alpha_spline, self.dev)
                     self.knots = _dev_f64(self.alpha_spline, self.dev)
             else:
-                self.dict_hr = Dictionary(self.alpha_values, self.T2s, self.T1s, self.nTE, tau, TR, self.dev)
+                self.dict_hr = Dictionary(self.alpha_values, self.T2s, self.T1s, self.nTE, tau, TR, self.dev,
+                                          self.slice_profile)
                 if FA_method == "spline":
-                    self.dict_lr = Dictionary(self.alpha_spline, self.T2s, self.T1s, self.nTE, tau, TR, self.dev)
+                    self.dict_lr = Dictionary(self.alpha_spline, self.T2s, self.T1s, self.nTE, tau, TR, self.dev,
+                                              self.slice_profile)
                     self.knots = _dev_f64(self.alpha_spline, self.dev)
             self.L_dev = _dev_f64(self.Laplac, self.dev)
             self.kband = torch.zeros((10, self.npc), dtype=torch.float64, device=self.dev)
@@ -697,6 +714,8 @@ class Met2Plan:
         PARAM_DEFAULTS.  Returns CUDA tensors params[V, 7] (amplitudes in signal units, T2_m, T2_ie, T2_fw in ms,
         flip angle in deg), maps[V, 6] (met2_t2_fit's columns), est_signal[V, nTE], sse[V], iters[V] (int32) and
         status[V] (int32).  Voxels the point fit skipped get zeros.  All work is enqueued on the current stream."""
+        if self.slice_profile is not None:
+            raise ValueError("the parametric fit models a single refocusing angle: it does not take a slice profile")
         c = self.param_cfg(**cfg)
         sig = self._signals(sig)
         V = sig.shape[0]

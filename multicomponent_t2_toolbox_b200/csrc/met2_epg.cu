@@ -8,11 +8,13 @@
 #include "met2_host.h"
 #include "met2_epg.cuh"
 
+#ifdef MET2_HOST_EMU
+#define __grid_constant__
+#endif
+
 namespace met2 {
 
-__device__ __forceinline__ void epg_decay(double alpha_deg, double T2, double T1, int n, double tau, double scale,
-                                          double* out, int out_stride) {
-    const EpgCoef<double> c = epg_coef(alpha_deg, T2, T1, tau);
+__device__ __forceinline__ void epg_train(const EpgCoef<double>& c, int n, double scale, double* out, int out_stride) {
     double Fp[MET2_MAX_NTE + 2], Fm[MET2_MAX_NTE + 2], Z[MET2_MAX_NTE + 2];
     for (int k = 0; k < n + 2; ++k) Fp[k] = Fm[k] = Z[k] = 0.0;
     double F0 = c.f0;
@@ -32,6 +34,11 @@ __device__ __forceinline__ void epg_decay(double alpha_deg, double T2, double T1
         }
         out[(size_t)echo * out_stride] = scale * F0;
     }
+}
+
+__device__ __forceinline__ void epg_decay(double alpha_deg, double T2, double T1, int n, double tau, double scale,
+                                          double* out, int out_stride) {
+    epg_train(epg_coef(alpha_deg, T2, T1, tau), n, scale, out, out_stride);
 }
 
 __global__ void epg_dictionary_kernel(const double* __restrict__ alphas, int nA, const double* __restrict__ T2s,
@@ -55,6 +62,71 @@ __global__ void epg_signals_kernel(const double* __restrict__ alphas, const doub
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= N) return;
     epg_decay(alphas[i], T2s[i], T1s[i], nTE, tau, 1.0, sig + i * nTE, 1);
+}
+
+// ---------------------------------------------------------------------------------------------------- slice profile
+// Profile-integrated echo trains for 2-D multi-slice CPMG (DESIGN §10g).  A slice profile is K positions with
+// excitation scale x[k], refocusing scale r[k] and weight w[k]; at nominal angle alpha the curve is
+//     S_e = sum_{k = 0..K-1, in this order}  w[k] * EPG_e(T2, T1, refocusing = alpha r[k], excitation = (alpha/2) x[k])
+// with EPG_e the recurrence above (epg_train).  One block per curve: the threads run the K trains C = blockDim.x at a
+// time into sT[e][C] (shared), then the owner of echo e (thread e mod C) adds the chunk's C terms to sA[e] one after the
+// other.  The sum order is therefore k = 0, 1, ..., K-1 whatever the block size or the scheduling of the threads, and
+// K = 1 with x = r = w = 1 gives 0 + 1 * F0 = the train of epg_decay bit for bit.
+// The profile is passed by value (12 KB of kernel parameters): it is checked on the host before any launch.
+struct ProfileTab {
+    double x[MET2_MAX_PROFILE], r[MET2_MAX_PROFILE], w[MET2_MAX_PROFILE];
+};
+
+__device__ __forceinline__ void profile_train(double alpha, double T2, double T1, int nTE, double tau,
+                                              const ProfileTab& p, int K, double* sT, double* sA) {
+    const int C = blockDim.x, t = threadIdx.x;
+    for (int e = t; e < nTE; e += C) sA[e] = 0.0;
+    for (int k0 = 0; k0 < K; k0 += C) {
+        const int k = k0 + t;
+        if (k < K) epg_train(epg_coef(alpha * p.r[k], (alpha / 2.0) * p.x[k], T2, T1, tau), nTE, 1.0, sT + t, C);
+        __syncthreads();
+        const int cnt = min(C, K - k0);
+        for (int e = t; e < nTE; e += C) {
+            double s = sA[e];
+            for (int i = 0; i < cnt; ++i) s = s + p.w[k0 + i] * sT[e * C + i];
+            sA[e] = s;
+        }
+        __syncthreads();
+    }
+}
+
+__global__ void epg_dictionary_profile_kernel(const double* __restrict__ alphas, const double* __restrict__ T2s,
+                                              const double* __restrict__ T1s, int nT2, int nTE, double tau, double TR,
+                                              const __grid_constant__ ProfileTab p, int K, double* __restrict__ dic,
+                                              double* __restrict__ dicT) {
+#ifdef MET2_HOST_EMU
+    double* sT = simt::g_shared.data;
+#else
+    extern __shared__ double sT[];
+#endif
+    double* sA = sT + (size_t)nTE * blockDim.x;
+    const int a = blockIdx.x / nT2, j = blockIdx.x - a * nT2;
+    profile_train(alphas[a], T2s[j], T1s[j], nTE, tau, p, K, sT, sA);
+    const double scale = 1.0 - exp(-TR / T1s[j]);   // epg.py:57
+    for (int e = threadIdx.x; e < nTE; e += blockDim.x) {
+        const double v = scale * sA[e];
+        if (dic) dic[((size_t)a * nTE + e) * nT2 + j] = v;
+        if (dicT) dicT[((size_t)a * nT2 + j) * nTE + e] = v;
+    }
+}
+
+__global__ void epg_signals_profile_kernel(const double* __restrict__ alphas, const double* __restrict__ T2s,
+                                           const double* __restrict__ T1s, int nTE, double tau,
+                                           const __grid_constant__ ProfileTab p, int K, double* __restrict__ sig) {
+#ifdef MET2_HOST_EMU
+    double* sT = simt::g_shared.data;
+#else
+    extern __shared__ double sT[];
+#endif
+    double* sA = sT + (size_t)nTE * blockDim.x;
+    const size_t i = blockIdx.x;
+    profile_train(alphas[i], T2s[i], T1s[i], nTE, tau, p, K, sT, sA);
+    for (int e = threadIdx.x; e < nTE; e += blockDim.x) sig[i * nTE + e] = sA[e];
 }
 
 // G[a] = D_a^T D_a, one block per angle; D_a staged in shared memory.
@@ -124,6 +196,62 @@ extern "C" int met2_epg_signals(const double* alphas_deg, const double* T2s, con
     MET2_LAUNCH((unsigned)((N + 127) / 128), 128, 0, st, epg_signals_kernel)(alphas_deg, T2s, T1s, (long long)N, nTE, tau_ms, sig);
     count_launch();
     return check_launch("epg_signals_kernel");
+}
+
+namespace {
+
+// K in 1..MET2_MAX_PROFILE and every x / r / w finite and >= 0 (host arrays) -> the kernels' table; else MET2_ERR_ARG.
+int profile_table(const char* what, const double* x, const double* r, const double* w, int K, ProfileTab* p) {
+    if (!x || !r || !w || K < 1 || K > MET2_MAX_PROFILE)
+        return set_error(MET2_ERR_ARG, "%s: bad slice profile (K=%d, 1..%d positions)", what, K, MET2_MAX_PROFILE);
+    for (int k = 0; k < K; ++k) {
+        const double v[3] = {x[k], r[k], w[k]};
+        for (double q : v)
+            if (!(q >= 0.0 && q <= 1.7976931348623157e308))   // false for NaN, negatives and +Inf
+                return set_error(MET2_ERR_ARG, "%s: slice profile entry %d is not finite and >= 0", what, k);
+        p->x[k] = x[k];
+        p->r[k] = r[k];
+        p->w[k] = w[k];
+    }
+    return MET2_OK;
+}
+
+// 32 threads for up to 32 positions, else 64 (one chunk of trains at the K = 64 of the default profile)
+int profile_threads(int K) { return K <= 32 ? 32 : 64; }
+
+}  // namespace
+
+extern "C" int met2_epg_dictionary_profile(const double* alphas_deg, int nA, const double* T2s, const double* T1s,
+                                           int nT2, int nTE, double tau_ms, double TR_ms, const double* x,
+                                           const double* r, const double* w, int K, double* dic, double* dicT,
+                                           void* stream) {
+    if (!alphas_deg || !T2s || !T1s || nA <= 0 || nT2 <= 0 || nT2 > MET2_MAX_NT2 || nTE <= 0 || nTE > MET2_MAX_NTE ||
+        (int64_t)nA * nT2 > INT32_MAX)
+        return set_error(MET2_ERR_ARG, "met2_epg_dictionary_profile: bad argument (nA=%d nT2=%d nTE=%d)", nA, nT2, nTE);
+    ProfileTab p;
+    int rc = profile_table("met2_epg_dictionary_profile", x, r, w, K, &p);
+    if (rc) return rc;
+    const int C = profile_threads(K);
+    MET2_LAUNCH(nA * nT2, C, sizeof(double) * (size_t)nTE * (C + 1), (cudaStream_t)stream,
+                epg_dictionary_profile_kernel)(alphas_deg, T2s, T1s, nT2, nTE, tau_ms, TR_ms, p, K, dic, dicT);
+    count_launch();
+    return check_launch("epg_dictionary_profile_kernel");
+}
+
+extern "C" int met2_epg_signals_profile(const double* alphas_deg, const double* T2s, const double* T1s, int64_t N,
+                                        int nTE, double tau_ms, const double* x, const double* r, const double* w,
+                                        int K, double* sig, void* stream) {
+    if (!alphas_deg || !T2s || !T1s || !sig || N < 0 || N > INT32_MAX || nTE <= 0 || nTE > MET2_MAX_NTE)
+        return set_error(MET2_ERR_ARG, "met2_epg_signals_profile: bad argument");
+    ProfileTab p;
+    int rc = profile_table("met2_epg_signals_profile", x, r, w, K, &p);
+    if (rc) return rc;
+    if (N == 0) return MET2_OK;
+    const int C = profile_threads(K);
+    MET2_LAUNCH((unsigned)N, C, sizeof(double) * (size_t)nTE * (C + 1), (cudaStream_t)stream,
+                epg_signals_profile_kernel)(alphas_deg, T2s, T1s, nTE, tau_ms, p, K, sig);
+    count_launch();
+    return check_launch("epg_signals_profile_kernel");
 }
 
 extern "C" int met2_gram_tables(const double* dic, int nA, int nTE, int nT2, const double* L, double* G, double* kband,

@@ -17,11 +17,13 @@ struct EpgCoef {
     S f0, fm1;   // initial state after the alpha/2 excitation: F0 and F-1
 };
 
+// Refocusing angle alpha_deg and a separate excitation angle exc_deg (the slice-profile dictionary of
+// met2_profile.cu evaluates the train at per-position angles; the reference's recurrence takes both angles).
 template <class S>
-__device__ __forceinline__ EpgCoef<S> epg_coef(S alpha_deg, S T2, double T1, double tau) {
+__device__ __forceinline__ EpgCoef<S> epg_coef(S alpha_deg, S exc_deg, S T2, double T1, double tau) {
     const double rad = 3.14159265358979323846 / 180.0;
     const S a = alpha_deg * rad;
-    const S a_exc = (alpha_deg / 2.0) * rad;   // epg.py:57: excitation = alpha/2
+    const S a_exc = exc_deg * rad;
     const double half = tau / 2.0;
     EpgCoef<S> c;
     c.e2 = exp(-half * (1.0 / T2));
@@ -34,6 +36,13 @@ __device__ __forceinline__ EpgCoef<S> epg_coef(S alpha_deg, S T2, double T1, dou
     c.f0 = sin(a_exc);    // epg.py:145
     c.fm1 = cos(a_exc);   // epg.py:147 (index 2 of the state vector is the F-1 slot)
     return c;
+}
+
+// The reference's coefficients: excitation = alpha/2 (epg.py:57).  Same operations as the two-angle form with
+// exc_deg = alpha_deg / 2, so the dictionary and the parametric fit are unchanged bit for bit.
+template <class S>
+__device__ __forceinline__ EpgCoef<S> epg_coef(S alpha_deg, S T2, double T1, double tau) {
+    return epg_coef(alpha_deg, alpha_deg / 2.0, T2, T1, tau);
 }
 
 // relaxation over tau/2 of one block (epg.py:82-85,133-141)

@@ -85,3 +85,69 @@ def reg_matrix(name, T2s):
         deltaT2[0] = deltaT2[1]
         return np.diag(1.0 / deltaT2)
     raise ValueError("Error: Wrong reg_matrix option!")
+
+
+def hann_sinc(tbw, n=512):
+    """Hann-windowed sinc of time-bandwidth product `tbw`, sampled at the midpoints of n steps over the pulse."""
+    t = (np.arange(n) + 0.5) / n - 0.5
+    return np.sinc(tbw * t) * (0.5 + 0.5 * np.cos(2.0 * np.pi * t))
+
+
+def pulse_rotation(waveform, flip_deg, freq):
+    """Rotation angle (deg) of an RF pulse at the off-resonance frequencies `freq` (cycles per pulse duration), by a
+    hard-pulse Cayley-Klein Bloch simulation: the waveform (any real samples, scaled so that their sum is flip_deg) is
+    applied as len(waveform) instantaneous rotations about (b_j, 0, 2 pi freq / n).  Returns 2 arcsin|beta| (evaluated
+    as 2 atan2(|beta|, |alpha|)); the phase of the result is dropped."""
+    b = np.asarray(waveform, dtype=np.float64)
+    b = b * (np.deg2rad(float(flip_deg)) / b.sum())
+    g = 2.0 * np.pi * np.asarray(freq, dtype=np.float64) / len(b)
+    a, bb = np.ones(g.shape, complex), np.zeros(g.shape, complex)
+    for bj in b:
+        phi = np.hypot(bj, g)
+        s = np.sin(phi / 2.0)
+        with np.errstate(invalid="ignore", divide="ignore"):
+            nx = np.where(phi > 0.0, bj / phi, 0.0)
+            nz = np.where(phi > 0.0, g / phi, 0.0)
+        al = np.cos(phi / 2.0) - 1j * nz * s
+        be = -1j * nx * s
+        a, bb = al * a - np.conj(be) * bb, be * a + np.conj(al) * bb
+    return np.rad2deg(2.0 * np.arctan2(np.abs(bb), np.abs(a)))   # 2 arcsin|beta|, well conditioned near 180
+
+
+def slice_profile(tbw=2.7, ratio=1.0, K=64, extent=1.5, waveform_exc=None, waveform_ref=None):
+    """Slice profile (x, r, w) of a 2-D multi-slice CPMG acquisition for the profile-integrated EPG dictionary
+    (`batched.Dictionary(profile=...)`, csrc/met2_epg.cu): K positions z evenly spaced over [-extent, extent] in units of
+    the excitation slice thickness, equal weights w = 1 / K, and the effective angles of the excitation (nominal 90)
+    and refocusing (nominal 180) pulses there as fractions of the nominal angle: x[k] = theta_exc(z_k) / 90,
+    r[k] = theta_ref(z_k) / 180.
+
+    Each pulse is simulated by `pulse_rotation` (hard-pulse Cayley-Klein Bloch).  The default pulse is a Hann-windowed
+    sinc of time-bandwidth product `tbw` (`hann_sinc`); waveform_exc / waveform_ref replace either by the caller's
+    samples (scaled to the nominal angle).  Position z lies at tbw * z cycles per pulse off resonance for the excitation
+    and at tbw * z / ratio for the refocusing pulse, whose slab is `ratio` times the excitation thickness.  The
+    excitation phase across the slice is ignored: only the rotation angle 2 arcsin|beta| enters the model, as in the
+    single-angle dictionary.  A caller with its own pulse simulation passes its own (x, r, w) instead."""
+    K = int(K)
+    if not 1 <= K <= 512:
+        raise ValueError("K must be in 1..512")
+    if not (tbw > 0 and ratio > 0 and extent >= 0):
+        raise ValueError("tbw and ratio must be > 0 and extent >= 0")
+    z = np.linspace(-extent, extent, K) if K > 1 else np.zeros(1)
+    exc = hann_sinc(tbw) if waveform_exc is None else waveform_exc
+    ref = hann_sinc(tbw) if waveform_ref is None else waveform_ref
+    x = pulse_rotation(exc, 90.0, tbw * z) / 90.0
+    r = pulse_rotation(ref, 180.0, tbw * z / ratio) / 180.0
+    return x, r, np.full(K, 1.0 / K)
+
+
+def as_slice_profile(profile):
+    """(x, r, w) as three float64 arrays of one length K in 1..512, all finite and >= 0, with w normalised to sum 1."""
+    try:
+        x, r, w = (np.ascontiguousarray(np.asarray(a, dtype=np.float64).reshape(-1)) for a in profile)
+    except (TypeError, ValueError):
+        raise ValueError("a slice profile is a tuple (x, r, w) of three arrays")
+    if not (len(x) == len(r) == len(w) and 1 <= len(x) <= 512):
+        raise ValueError("a slice profile needs x, r, w of one length K in 1..512")
+    if not all(np.all(np.isfinite(a)) and np.all(a >= 0.0) for a in (x, r, w)) or not w.sum() > 0.0:
+        raise ValueError("slice profile entries must be finite and >= 0, with a positive sum of weights")
+    return x, r, np.ascontiguousarray(w / w.sum())

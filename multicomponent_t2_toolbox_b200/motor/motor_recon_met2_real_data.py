@@ -73,7 +73,7 @@ def degibbs_step1(data, mask):
 
 def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR, reg_method, reg_matrix, denoise,
                      FA_method, FA_smooth, myelin_T2, num_cores, n_bootstrap=0, bootstrap_seed=0, spatial_mu=0.0,
-                     spatial_sweeps=10, parametric=False, degibbs=False, rician_sigma=None):
+                     spatial_sweeps=10, parametric=False, degibbs=False, rician_sigma=None, slice_profile=None):
     """Same arguments as the reference.  `num_cores` selects the number of GPUs (-1 = all visible; see
     n_gpus_from_num_cores): the masked voxels of the volume are spread over them by pipeline.MultiGpuFit.
 
@@ -102,7 +102,15 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
     [nx, ny, nz] array, or 'MPPCA' for the sigma map of batched.mppca_denoise on the masked data (the denoised data are
     discarded; the map is written as MPPCA_sigma.nii.gz).  Written as MWF_rician, IEWF_rician, FWF_rician, T2_M_rician,
     T2_IE_rician, TWC_rician, fsol_4D_rician, Est_Signal_rician and rician_iters (.nii.gz) beside the unchanged ten
-    outputs.  The likelihood describes raw magnitude data, so it needs denoise='None' and degibbs=False."""
+    outputs.  The likelihood describes raw magnitude data, so it needs denoise='None' and degibbs=False.
+
+    slice_profile = (x, r, w) (not in the reference, reached from Python only; grids.slice_profile): for 2-D
+    multi-slice data, every fit runs on the slice-profile-integrated EPG dictionary (pipeline.recon_arrays) instead of
+    the single-angle one.  The same files are written; FA is the nominal angle at the slice centre.  It cannot be
+    combined with parametric=True."""
+    if slice_profile is not None and parametric:
+        raise ValueError("the parametric fit models a single refocusing angle: it cannot be combined with "
+                         "slice_profile")
     if rician_sigma is not None and (denoise != 'None' or degibbs):
         raise ValueError("rician_sigma describes the noise of the raw magnitude data: it needs denoise='None' and "
                          "degibbs=False")
@@ -156,7 +164,7 @@ def motor_recon_met2(TE_array, path_to_data, path_to_mask, path_to_save_data, TR
                                 FA_method, myelin_T2=myelin_T2, data_fa=data_fa, diagnostics=True, premasked=True,
                                 n_gpus=n_gpus, n_bootstrap=n_bootstrap, bootstrap_seed=bootstrap_seed,
                                 spatial_mu=spatial_mu, spatial_sweeps=spatial_sweeps, parametric=parametric,
-                                rician_sigma=rician_sigma)
+                                rician_sigma=rician_sigma, slice_profile=slice_profile)
     print('Step #4: Estimation of quantitative metrics')
     # the ten volumes (motor...:474-503) are written concurrently, largest first: every writer deflates with all cores
     # (nifti_io), but the eight 3-D maps are too small to keep them busy one at a time (2.2 s -> 1.2 s on 8 cores)

@@ -16,7 +16,10 @@ from .motor_recon_met2_real_data import degibbs_step1, tv_denoise
 
 
 def motor_recon_met2_ROIs(TE_array, path_to_data, path_to_mask, path_to_ROIs, path_to_save_data, TR, reg_matrix, denoise,
-                          FA_method, FA_smooth, myelin_T2, num_cores, degibbs=False):
+                          FA_method, FA_smooth, myelin_T2, num_cores, degibbs=False, slice_profile=None):
+    """Same arguments as the reference.  slice_profile = (x, r, w) (not in the reference; grids.slice_profile): the
+    flip-angle search and the ROI fits run on the slice-profile-integrated EPG dictionary of 2-D multi-slice data
+    (pipeline.recon_arrays)."""
     img = nifti_io.load(path_to_data)
     data = img.get_fdata().astype(np.float64, copy=False)
     mask = nifti_io.load(path_to_mask).get_fdata().astype(np.int64, copy=False)
@@ -38,7 +41,8 @@ def motor_recon_met2_ROIs(TE_array, path_to_data, path_to_mask, path_to_ROIs, pa
     data_fa = batched.gaussian_smooth(data, sigma=2.0) if FA_smooth == 'yes' else None
     vol = pipeline.recon_arrays(data, mask, np.asarray(TE_array, dtype=np.float64), TR, "X2", reg_matrix, FA_method,
                                 myelin_T2=myelin_T2, data_fa=data_fa, diagnostics=True, rois=ROIs, premasked=True,
-                                fa_only=True)   # the ROI estimator never fits voxel spectra (reference :349-445)
+                                fa_only=True,   # the ROI estimator never fits voxel spectra (reference :349-445)
+                                slice_profile=slice_profile)
     roi = vol["roi"]
     join = (lambda name: path_to_save_data + name) if path_to_save_data.endswith('/') else \
         (lambda name: os.path.join(path_to_save_data, name))

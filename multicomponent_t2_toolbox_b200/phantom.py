@@ -10,23 +10,25 @@ same operator sequence as epg/epg.py:64-153 (shift, relax tau/2, RF, shift, rela
 import numpy as np
 
 
-def epg_signal_batch(n_echoes, tau, T1, T2, alpha_deg, chunk=65536):
+def epg_signal_batch(n_echoes, tau, T1, T2, alpha_deg, chunk=65536, exc_deg=None):
     """EPG multi-echo decay for arrays of (T1, T2, alpha) — one decay curve per element.
 
     State layout follows epg/epg.py:97-147: index 0 is F0, block k=1..n holds (F+k, F-k, Zk).  The excitation is
-    alpha/2 and the start state is x[0]=sin(a_exc), F-1 slot = cos(a_exc) (epg/epg.py:57,143-147).
-    Returns [N, n_echoes] (no (1-exp(-TR/T1)) factor).
+    alpha/2 (or exc_deg, an array like alpha_deg) and the start state is x[0]=sin(a_exc), F-1 slot = cos(a_exc)
+    (epg/epg.py:57,143-147).  Returns [N, n_echoes] (no (1-exp(-TR/T1)) factor).
     """
     T1 = np.asarray(T1, dtype=np.float64).ravel()
     T2 = np.asarray(T2, dtype=np.float64).ravel()
     alpha_deg = np.asarray(alpha_deg, dtype=np.float64).ravel()
+    if exc_deg is not None:
+        exc_deg = np.broadcast_to(np.asarray(exc_deg, dtype=np.float64).ravel(), alpha_deg.shape)
     N = T2.shape[0]
     out = np.empty((N, n_echoes))
     n = n_echoes
     for s in range(0, N, chunk):
         e = min(N, s + chunk)
         a = alpha_deg[s:e] * (np.pi / 180.0)
-        a_exc = (alpha_deg[s:e] / 2.0) * (np.pi / 180.0)
+        a_exc = (alpha_deg[s:e] / 2.0 if exc_deg is None else exc_deg[s:e]) * (np.pi / 180.0)
         e2 = np.exp(-(tau / 2.0) / T2[s:e])
         e1 = np.exp(-(tau / 2.0) / T1[s:e])
         c2 = np.cos(a / 2.0) ** 2
@@ -80,8 +82,20 @@ def b1_field(shape, rng, jitter=3.0):
     return np.clip(fa, 95.0, 180.0)
 
 
-def _epg_signal_batch_gpu(n_echoes, tau, T1, T2, alpha_deg):
-    """Same curves as epg_signal_batch, computed by libmet2's EPG kernel (met2_epg_signals)."""
+def epg_profile_signal_batch(n_echoes, tau, T1, T2, alpha_deg, profile):
+    """Slice-profile-integrated curves of met2_epg_signals_profile on the host: sum over the positions k, in order, of
+    w[k] * epg_signal_batch at refocusing alpha r[k] and excitation (alpha / 2) x[k]."""
+    x, r, w = profile
+    alpha_deg = np.asarray(alpha_deg, dtype=np.float64).ravel()
+    acc = np.zeros((alpha_deg.shape[0], n_echoes))
+    for k in range(len(w)):
+        acc = acc + w[k] * epg_signal_batch(n_echoes, tau, T1, T2, alpha_deg * r[k], exc_deg=alpha_deg / 2.0 * x[k])
+    return acc
+
+
+def _epg_signal_batch_gpu(n_echoes, tau, T1, T2, alpha_deg, profile=None):
+    """Same curves as epg_signal_batch (epg_profile_signal_batch with a profile), computed by libmet2's EPG kernels
+    (met2_epg_signals, met2_epg_signals_profile)."""
     import ctypes
 
     import torch
@@ -93,6 +107,14 @@ def _epg_signal_batch_gpu(n_echoes, tau, T1, T2, alpha_deg):
     t2 = torch.as_tensor(np.ascontiguousarray(T2, dtype=np.float64)).to(dev)
     t1 = torch.as_tensor(np.ascontiguousarray(T1, dtype=np.float64)).to(dev)
     out = torch.empty((a.numel(), n_echoes), dtype=torch.float64, device=dev)
+    if profile is not None:
+        x, r, w = (ctypes.c_void_p(q.ctypes.data) for q in profile)    # host arrays
+        _lib.check(lib.met2_epg_signals_profile(ctypes.c_void_p(a.data_ptr()), ctypes.c_void_p(t2.data_ptr()),
+                                                ctypes.c_void_p(t1.data_ptr()), a.numel(), n_echoes, float(tau), x, r,
+                                                w, len(profile[2]), ctypes.c_void_p(out.data_ptr()),
+                                                ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)),
+                   "met2_epg_signals_profile")
+        return out.cpu().numpy()
     _lib.check(lib.met2_epg_signals(ctypes.c_void_p(a.data_ptr()), ctypes.c_void_p(t2.data_ptr()),
                                     ctypes.c_void_p(t1.data_ptr()), a.numel(), n_echoes, float(tau),
                                     ctypes.c_void_p(out.data_ptr()),
@@ -101,7 +123,7 @@ def _epg_signal_batch_gpu(n_echoes, tau, T1, T2, alpha_deg):
 
 
 def make_phantom(shape=(16, 16, 4), n_echoes=32, tau=10.0, TR=1000.0, T1=1000.0, seed=1, fa_mode="uniform",
-                 snr_range=(50.0, 150.0), Km=1000.0, mask_mode="full", backend="numpy"):
+                 snr_range=(50.0, 150.0), Km=1000.0, mask_mode="full", backend="numpy", slice_profile=None):
     """Return dict(data[nx,ny,nz,nTE], mask[nx,ny,nz], truth={...}); truth["sigma"] is the SD of the Rician noise in
     the data's units.
 
@@ -109,6 +131,9 @@ def make_phantom(shape=(16, 16, 4), n_echoes=32, tau=10.0, TR=1000.0, T1=1000.0,
     mask_mode: "full" -> all ones; "ellipsoid" -> ~52 % fill, exercises the gather/scatter of masked voxels.
     backend: "numpy" (host recurrence) or "gpu" (libmet2's EPG kernel; for the half-million-voxel bench volumes).
     The two backends agree to ~1e-15 relative; the random draws are identical.
+    slice_profile = (x, r, w) (`grids.slice_profile`): the curves are integrated over that slice profile, as 2-D
+    multi-slice data are (met2_epg_signals_profile; truth["fa"] is the nominal angle at the slice centre).  The random
+    draws are those of the same call without a profile.
     """
     rng = np.random.default_rng(seed)
     nx, ny, nz = shape
@@ -128,6 +153,11 @@ def make_phantom(shape=(16, 16, 4), n_echoes=32, tau=10.0, TR=1000.0, T1=1000.0,
     snr = rng.uniform(snr_range[0], snr_range[1], V)
     T1v = np.full(V, float(T1))
     epg = _epg_signal_batch_gpu if backend == "gpu" else epg_signal_batch
+    if slice_profile is not None:
+        from .grids import as_slice_profile
+        prof = as_slice_profile(slice_profile)
+        epg = (lambda *a: _epg_signal_batch_gpu(*a, profile=prof)) if backend == "gpu" else \
+            (lambda *a: epg_profile_signal_batch(*a, prof))
     sig = mwf[:, None] * epg(n_echoes, tau, T1v, t2m, fa)
     sig += iewf[:, None] * epg(n_echoes, tau, T1v, t2ie, fa)
     sig += fwf[:, None] * epg(n_echoes, tau, T1v, t2fw, fa)

@@ -400,8 +400,13 @@ def fit_voxels(plan, sig, sig_fa=None, pinned_out=None, in_mask=None, roi=None, 
 def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, myelin_T2=40.0, data_fa=None, plan=None,
                  npc=None, n_alphas=None, device=None, rank=0, world_size=1, diagnostics=False, rois=None,
                  premasked=False, fa_only=False, n_gpus=1, n_bootstrap=0, bootstrap_seed=0, spatial_mu=0.0,
-                 spatial_sweeps=10, parametric=False, rician_sigma=None):
+                 spatial_sweeps=10, parametric=False, rician_sigma=None, slice_profile=None):
     """Steps 2-4 of motor_recon_met2 on in-memory arrays.  Returns the ten output volumes (plus FA_index) as numpy.
+
+    slice_profile = (x, r, w) (`grids.slice_profile`, for 2-D multi-slice data): the plan's dictionaries (fine and
+    spline-knot) are the slice-profile-integrated ones (`batched.Met2Plan(slice_profile=...)`, DESIGN §10g); every
+    device of a multi-GPU run builds the same.  FA stays the nominal angle at the slice centre.  Used when `plan` is
+    None (a given plan brings its own dictionaries); it cannot be combined with parametric.
 
     n_bootstrap > 0: also the per-voxel bootstrap uncertainty of the six maps with that many replicates per voxel
     (`batched.Met2Plan.bootstrap`): volumes "<MAP>_bootstrap" [nx, ny, nz, 4] (mean, sd, p2.5, p97.5) and
@@ -448,6 +453,9 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
     if rician_sigma is not None and spatial_mu > 0:
         raise ValueError("spatial_mu > 0 cannot be combined with rician_sigma: it is ambiguous which spectrum starts the "
                          "Rician fit")
+    if slice_profile is not None and parametric:
+        raise ValueError("the parametric fit models a single refocusing angle: it cannot be combined with "
+                         "slice_profile")
     data = np.asarray(data, dtype=np.float64)
     nx, ny, nz, nt = data.shape
     TE_array = np.asarray(TE_array, dtype=np.float64)
@@ -455,7 +463,7 @@ def recon_arrays(data, mask, TE_array, TR, reg_method, reg_matrix, FA_method, my
     if plan is None:
         plan_args = (TE_array.shape[0], TE_array[1] - TE_array[0], TR)
         plan_kw = dict(reg_method=reg_method, reg_matrix=reg_matrix, FA_method=FA_method, myelin_T2=myelin_T2, npc=npc,
-                       n_alphas=n_alphas)
+                       n_alphas=n_alphas, slice_profile=slice_profile)
         want = torch.cuda.device_count() if (n_gpus is None or n_gpus < 1) else min(int(n_gpus), torch.cuda.device_count())
         if world_size == 1 and want > 1 and device is None and not fa_only:
             multi = MultiGpuFit.create(want, *plan_args, **plan_kw)
